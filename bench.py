@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference [...]                 # the reference's CPU path (oracle port) on host cores
+    python bench.py [...] --dump-outputs DIR               # + the detections of the last timed step as DIR/<name>.npy
 
 One step = one pass of the whole detector (backbone + support-guided head) over one batch of
 synthetic 640x640 ore-shaped query images, 1-way 25-shot, random-init (synthetic) weights.
@@ -260,6 +261,22 @@ def fsodrcnn_record(dev, steps):
             "detections": int(sum(len(o["instances"]) for o in out))}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each host tensor as out_dir/<name>.npy, float32 kept and integers widened to float64 (exact), so that two
+    builds can be compared output for output on the same seeded inputs."""
+    import numpy as np
+    arrays = {n: v.numpy() if v.dtype == torch.float32 else v.numpy().astype(np.float64) for n, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of detections exceed {DUMP_LIMIT_BYTES}; use a smaller --batch")
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
+
+
 def run_gpu_arm(args):
     import torch.distributed as dist
     from faster_orefsdet_b200 import ops
@@ -329,6 +346,10 @@ def run_gpu_arm(args):
         barrier()
         clk = clocks.stop() if rank == 0 else None
         ms = ev0.elapsed_time(ev1)
+        # what the caller of the timed path received from its last step, copied out before a later replay can reuse
+        # the graph's output buffers
+        last = dict(zip(("boxes", "scores", "classes", "counts"), (v.cpu() for v in out))) \
+            if args.dump_outputs and rank == 0 else None
         # Per-kernel durations: the timed region replays one CUDA graph per step, inside which events cannot be read,
         # so the same K steps are re-run eagerly right here (same inputs, same kernels, same launch parameters) with
         # CUDA events around every C-ABI call on torch's current stream.
@@ -592,6 +613,8 @@ def run_gpu_arm(args):
         line["cpu_baseline"] = {"value": cpu_rate, "unit": UNIT, "cores": cpu_threads, "kind": "port",
                                 "sample": f"{args.cpu_images} images 640x640 after 2 warm-up, batch-1 loop, oracle head + "
                                           f"PyTorch-CPU VoVNet/FPN, {cpu_dt:.1f} s"}
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -608,7 +631,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C3 / C4 sub-records")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling (global batch 256) sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the padded detections of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

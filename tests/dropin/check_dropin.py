@@ -1,4 +1,4 @@
-"""Subprocess body of tests/test_dropin_cpu.py (build container only: needs /root/reference).
+"""Subprocess body of tests/test_dropin_cpu.py (needs FOD_REFERENCE_DIR, see tests/golden/refshim.py).
 
 Plays `fsod_train_net.py --eval-only` / `demo.py` up to the model construction with the UNMODIFIED reference imported
 the way those scripts import it, then installs this package over the reference's registry names and builds the model
@@ -51,11 +51,11 @@ out["override_replaces"] = (META_ARCH_REGISTRY.get("CenterNet2Detector") is ours
                             and ref_roi.ROI_HEADS_REGISTRY.get("CustomCascadeROIHeads") is ours.CustomCascadeROIHeads)
 
 cfg = get_cfg()                                                   # the REFERENCE's config object and defaults
-cfg.merge_from_file("/root/reference/configs/fsod/finetune_vovnet.yaml")
+cfg.merge_from_file(os.path.join(refshim.REFERENCE, "configs/fsod/finetune_vovnet.yaml"))
 cfg.merge_from_list(["MODEL.DEVICE", "cuda"])
 moved = []
 _to = torch.nn.Module.to
-torch.nn.Module.to = lambda self, *a, **k: (moved.append(a), self)[1]     # no GPU in the build container
+torch.nn.Module.to = lambda self, *a, **k: (moved.append(a), self)[1]     # the test needs no GPU
 try:
     model = build_model(cfg)                                      # fsod_train_net.py:95 -> Trainer.build_model -> this
 finally:
@@ -71,7 +71,7 @@ out["submodules"] = {"proposal_generator": type(model.proposal_generator).__modu
 import runpy  # noqa: E402
 
 try:
-    ns = runpy.run_path("/root/reference/fsod_train_net.py", run_name="fsod_train_net_not_main")
+    ns = runpy.run_path(os.path.join(refshim.REFERENCE, "fsod_train_net.py"), run_name="fsod_train_net_not_main")
     torch.nn.Module.to = lambda self, *a, **k: self
     try:
         m2 = ns["Trainer"].build_model(cfg)

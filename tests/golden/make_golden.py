@@ -2,7 +2,7 @@
 
     python tests/golden/make_golden.py            # writes tests/golden/*.npz
 
-Needs /root/reference (read-only) - it never runs on the GPU box; the tests only
+Needs FOD_REFERENCE_DIR (a read-only checkout of the reference); the tests only
 read the committed ``.npz`` files.  The reference modules are imported from
 where they lie through ``refshim`` (stand-ins for the missing third-party
 packages only; see its docstring).  Harness-level substitutions, none of which
@@ -50,7 +50,7 @@ from detectron2.modeling.postprocessing import detector_postprocess  # noqa: E40
 from fewx.modeling.fsod.fsod_fast_rcnn import fsod_fast_rcnn_inference_single_image  # noqa: E402
 from fewx.modeling.fsod.fsod_cen import SM_Block  # noqa: E402
 
-YAML = "/root/reference/configs/fsod/finetune_vovnet.yaml"
+YAML = os.path.join(refshim.REFERENCE, "configs/fsod/finetune_vovnet.yaml")
 
 
 class StubBackbone(torch.nn.Module):
@@ -233,6 +233,8 @@ def run_ops(model, cfg):
     x = synth.tensor((3, 16, 16, 128), 81, -1.0, 1.0)
     with torch.no_grad():
         rec["sm_p4"] = np_(model.vip_p4(x))
+    # the pooled maps in a file of their own keep every fixture under 1 MB
+    np.savez_compressed(os.path.join(HERE, "roi_pool.npz"), **{k: rec.pop(k) for k in ("pool_out8", "pool_out4")})
     np.savez_compressed(os.path.join(HERE, "ops.npz"), **rec)
     print("ops:", {k: v.shape for k, v in rec.items()})
 

@@ -40,7 +40,7 @@ import fewx.modeling  # noqa: E402,F401
 import fewx.modeling.fsod.fsod_rcnn as ref_rcnn  # noqa: E402
 
 ref_rcnn.Have_a_Look = lambda *a, **k: None
-YAML = "/root/reference/configs/fsod/Base-FSOD-C4.yaml"
+YAML = os.path.join(refshim.REFERENCE, "configs/fsod/Base-FSOD-C4.yaml")
 
 
 def fsodrcnn_support(class_ids, seed):

@@ -1,7 +1,7 @@
 """Make the UNMODIFIED reference importable in the build container.
 
 Used only by ``tests/golden/make_golden.py`` (golden-vector generation; runs in
-the build container where /root/reference exists, never on the GPU box).
+a machine where FOD_REFERENCE_DIR points at a checkout of the reference project).
 
 The reference (fewx/ + CenterNet2/ + the vendored detectron2 inside
 detectron2.7z) needs third-party packages that are not installed here
@@ -16,7 +16,7 @@ stand-ins:
     actually executes: ``Registry``, ``CfgNode`` and ``weight_init``.
 
 The reference sources themselves are imported from where they lie
-(/root/reference, and the archive unpacked to a temp dir); nothing is copied
+(FOD_REFERENCE_DIR, and the archive unpacked to a temp dir); nothing is copied
 into the repository.
 """
 from __future__ import annotations
@@ -31,7 +31,7 @@ import struct
 import sys
 import types
 
-REFERENCE = "/root/reference"
+REFERENCE = os.environ.get("FOD_REFERENCE_DIR", "")     # checkout of the reference project (fewx/, configs/, detectron2.7z)
 
 MISSING = {
     "fvcore", "iopath", "yacs", "termcolor", "pycocotools", "omegaconf", "matplotlib", "black", "nis",

@@ -355,7 +355,7 @@ def test_roi_align_matches_reference_and_oracle():
         pooled, lv = ops.roi_align([f.to(DEV) for f in fl], (8, 16, 32), bx.to(DEV), None, 1, res, want_levels=True)
         assert np.array_equal(lv.cpu().numpy(), want_lv.numpy())
         got = pooled.cpu().reshape(2 * 96, res, res, 128).permute(0, 3, 1, 2)
-        assert_close(got[:, ::8], t(g[f"pool_out{res}"]), what=f"roi_align{res} vs reference")
+        assert_close(got[:, ::8], t(golden("roi_pool")[f"pool_out{res}"]), what=f"roi_align{res} vs reference")
         assert_close(got, O.roi_pool(fl, [bx[0], bx[1]], res), what=f"roi_align{res} vs oracle")
 
 

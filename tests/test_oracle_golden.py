@@ -72,7 +72,7 @@ def test_roi_pool_matches_reference():
     fl, bx = _pool_inputs(g)
     for res in (8, 4):
         out = O.roi_pool(fl, [bx[0], bx[1]], res)
-        assert_close(out[:, ::8], t(g[f"pool_out{res}"]), what=f"roi_pool{res}")
+        assert_close(out[:, ::8], t(golden("roi_pool")[f"pool_out{res}"]), what=f"roi_pool{res}")
 
 
 def test_relation_head_matches_reference():
