@@ -61,6 +61,7 @@ _PROTOTYPES = {
     "fod_group_norm_workspace_bytes": ([_i, _i], ctypes.c_size_t),
     "fod_group_norm_nhwc": ([_vp, _i, ctypes.c_long, _i, _i, _vp, _vp, _f, _i, _vp, _vp, _i, _vp, _vp], _i),
     "fod_absmax": ([_vp, ctypes.c_size_t, _vp, _vp], _i),
+    "fod_absmax_rows": ([_vp, _i, ctypes.c_size_t, _vp, _vp], _i),
     "fod_stem_patches": ([_vp, _i, _i, _i, _vp, _vp], _i),
     "fod_stem_patches_u8": ([_vp, _i, _i, _i, ctypes.POINTER(_f), ctypes.POINTER(_f), _vp, _vp], _i),
     "fod_stem1_u8_tc": ([_vp, _i, _i, _i, ctypes.POINTER(_f), ctypes.POINTER(_f), _vp, _vp, _vp, ctypes.c_long, _vp, _i, _vp], _i),

@@ -756,8 +756,11 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
   if (warp == kWarpAlloc) tmem_dealloc<2>(tmem_base, kTmemCols);
 }
 
-// max |x| of a dense fp32 array into *out (non-negative floats order like their bit patterns); *out must start at 0
+// max |x| of a dense fp32 array into *out (non-negative floats order like their bit patterns); *out must start at 0.
+// blockIdx.y selects one of several arrays of n floats laid end to end, and out[blockIdx.y] receives its maximum.
 __global__ void absmax_kernel(const float* __restrict__ x, size_t n, float* __restrict__ out) {
+  x += (size_t)blockIdx.y * n;
+  out += blockIdx.y;
   float m = 0.f;
   const size_t n4 = n >> 2;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
@@ -889,12 +892,19 @@ extern "C" int fod_ese_gate(const float* colsum, int n, int tiles_per_img, int c
 }
 
 extern "C" int fod_absmax(const float* x, size_t n, float* out, fod_stream_t stream) {
+  return fod_absmax_rows(x, 1, n, out, stream);
+}
+
+extern "C" int fod_absmax_rows(const float* x, int rows, size_t row_len, float* out, fod_stream_t stream) {
   FOD_REQUIRE(x && out, "fod_absmax: null pointer");
   FOD_REQUIRE(((uintptr_t)x & 15) == 0, "fod_absmax: input must be 16-byte aligned");
-  FOD_CUDA_CALL(cudaMemsetAsync(out, 0, sizeof(float), as_stream(stream)));
-  if (n == 0) return FOD_OK;
-  const size_t blocks = (n / 4 + 255) / 256;
-  cvt::absmax_kernel<<<(unsigned)(blocks < 148 * 8 ? (blocks ? blocks : 1) : 148 * 8), 256, 0, as_stream(stream)>>>(x, n, out);
+  FOD_REQUIRE(rows >= 1 && rows <= 65535 && (rows == 1 || row_len % 4 == 0), "fod_absmax_rows: 1..65535 rows of a multiple of 4 floats");
+  FOD_CUDA_CALL(cudaMemsetAsync(out, 0, sizeof(float) * rows, as_stream(stream)));
+  if (row_len == 0) return FOD_OK;
+  const size_t per_row = (148 * 8 + rows - 1) / rows;                  // about 148 * 8 CTAs in all
+  const size_t blocks = (row_len / 4 + 255) / 256;
+  const dim3 grid((unsigned)(blocks < per_row ? (blocks ? blocks : 1) : per_row), (unsigned)rows);
+  cvt::absmax_kernel<<<grid, 256, 0, as_stream(stream)>>>(x, row_len, out);
   FOD_CUDA_LAUNCH_CHECK("fod_absmax");
   return FOD_OK;
 }

@@ -58,8 +58,8 @@ class FsodFastRCNNOutputLayers(nn.Module):
         self.test_topk_per_image = cfg.TEST.DETECTIONS_PER_IMAGE
 
     def _conv1(self, x):
-        if tcconv.supported(self.conv_1, x):
-            return tcconv.conv(x, self.conv_1, relu=True)
+        if tcconv.supported(self.conv_1, x):      # one operand bound per ROI row (see resnet.ConvNorm)
+            return tcconv.conv(x, self.conv_1, relu=True, x_amax=ops.absmax(x, per_image=True).reshape(1, -1))
         return F.relu(self.conv_1(x))
 
     def embed_support(self, x_support: torch.Tensor) -> Dict[str, torch.Tensor]:

@@ -64,13 +64,27 @@ class ParallelPolarizedSelfAttention(nn.Module):
         """softmax over the 14x14 positions of ch_wq(support): [1, 196, 1] (depends on the support only)."""
         return F.softmax(self._conv1x1(self.ch_wq, q).reshape(q.shape[0], -1, 1), dim=1)
 
-    def forward(self, x: torch.Tensor, q: torch.Tensor, wq: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, q: torch.Tensor) -> torch.Tensor:
         b, c, _, _ = x.shape
         wv = self._conv1x1(self.ch_wv, x)                                        # [b, c/2, h*w]
-        wq = self.support_query(q) if wq is None else wq
-        wz = torch.matmul(wv, wq)                                                # [b, c/2, 1]
+        wz = torch.matmul(wv, self.support_query(q))                             # [b, c/2, 1]
         z = self._conv1x1(self.ch_wz, wz)                                        # [b, c, 1]
         return torch.sigmoid(self.ln(z.permute(0, 2, 1))).permute(0, 2, 1).reshape(b, c, 1, 1)
+
+    def gates(self, x: torch.Tensor, wq: torch.Tensor, k: torch.Tensor) -> torch.Tensor:
+        """forward for all classes at once, plus the depthwise kernel of each class: x [B, c, 14, 14] (avgpool14 of the
+        query), wq [h*w, C] (support_query of every class), k [C, c] -> gates [C, B, c].  One image at a time, so that
+        every matrix product has the same shape whatever the batch: cuBLAS may pick another algorithm (another
+        summation order) for another shape, and an image's gates must not depend on its batch mates."""
+        x = x.contiguous()
+        cv, cz = self.ch_wv, self.ch_wz
+        wv_w, wz_w = cv.weight.reshape(cv.out_channels, -1), cz.weight.reshape(cz.out_channels, -1)
+        out = []
+        for b in range(x.shape[0]):
+            wv = torch.addmm(cv.bias[:, None], wv_w, x[b].reshape(x.shape[1], -1))         # [c/2, h*w]
+            z = torch.addmm(cz.bias[:, None], wz_w, wv @ wq)                               # [c, C]
+            out.append(torch.sigmoid(self.ln(z.t())) + k)                                 # [C, c]
+        return torch.stack(out, 1)
 
 
 @register(META_ARCH_REGISTRY)
@@ -123,9 +137,9 @@ class FsodRCNN(nn.Module):
         for c in class_ids:
             r4 = support_dict["res4_avg"][c].to(dev, torch.float32)
             k.append(r4.mean((2, 3)).reshape(1, -1))                                      # depthwise 1x1 kernel, :487
-            wq.append(self.channel_attention.support_query(r4))
+            wq.append(self.channel_attention.support_query(r4).reshape(-1, 1))
             emb.append(self.roi_heads.box_predictor.embed_support(support_dict["res5_avg"][c].to(dev, torch.float32)))
-        self._episode = {"class_ids": class_ids, "k": torch.cat(k, 0), "wq": wq, "emb": emb,
+        self._episode = {"class_ids": class_ids, "k": torch.cat(k, 0), "wq": torch.cat(wq, 1), "emb": emb,
                          "weights": tuple((p.data_ptr(), p._version) for p in self.parameters())}
         self._episode_src = support_dict
         self._episode_key = ("memory", id(support_dict))
@@ -231,17 +245,16 @@ class FsodRCNN(nn.Module):
         if res4.is_cuda:
             res4 = ops.nhwc(res4, "res4")
         B, C = res4.shape[0], len(ep["class_ids"])
-        pooled = self.agp(res4)                                                     # shared by all classes (:480)
-        amax = ops.absmax(res4)
+        gates = self.channel_attention.gates(self.agp(res4), ep["wq"], ep["k"])      # [C, B, 1024]: (:480-488)
+        amax = ops.absmax(res4, per_image=True)                                     # per image: no batch-mate coupling
         trace = {"gate": [], "proposals": []}
         cap = self.proposal_generator.post_nms_topk
         props = torch.zeros((B, C, cap, 4), dtype=torch.float32, device=res4.device)
         counts = torch.zeros((B, C), dtype=torch.int32, device=res4.device)
         fake_images = type("Sizes", (), {"image_sizes": image_sizes})()
         for ci in range(C):
-            weight = self.channel_attention(pooled, None, ep["wq"][ci])             # [B, 1024, 1, 1]
-            gate = (weight.reshape(B, -1) + ep["k"][ci:ci + 1]).contiguous()        # channel_att + spatial_att = gate (.) res4
-            bound = (amax * gate.abs().max()).reshape(1)
+            gate = gates[ci]                                                        # channel_att + spatial_att = gate (.) res4
+            bound = (amax * gate.abs().amax(1)).reshape(1, B)
             plist, _ = self.proposal_generator(fake_images, {self.proposal_generator.in_features[0]: res4}, None,
                                                gates=[gate], bounds=[bound])
             trace["gate"].append(gate)

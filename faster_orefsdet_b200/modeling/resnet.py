@@ -13,6 +13,7 @@ import torch
 import torch.nn.functional as F
 from torch import nn
 
+from .. import ops
 from ..compat import BACKBONE_REGISTRY, Backbone, ShapeSpec, register
 from . import tcconv
 from .backbone import FrozenBatchNorm2d
@@ -27,16 +28,17 @@ class ConvNorm(nn.Conv2d):
         nn.init.kaiming_normal_(self.weight, mode="fan_out", nonlinearity="relu")    # c2_msra_fill
 
     def forward(self, x, relu: bool = False, residual: Optional[torch.Tensor] = None):
+        """On CUDA every image (every ROI row in res5) is scaled by its own operand bound, so that its result depends
+        neither on the other images of the batch nor on rows nobody wrote (the padding rows of a ragged ROI batch)."""
         if x.is_cuda:       # the kernels read NHWC memory; ATen ops (stem, pooling) may hand over NCHW
             x = x.contiguous(memory_format=torch.channels_last)
         if tcconv.supported(self, x) and not self.training:
-            return tcconv.conv(x, self, self.norm, relu=relu, residual=residual)
+            return tcconv.conv(x, self, self.norm, relu=relu, residual=residual, x_amax=ops.absmax(x, per_image=True).reshape(1, -1))
         if x.is_cuda and self.kernel_size == (1, 1) and self.stride == (2, 2) and self.in_channels % 4 == 0 and not self.training:
             # a strided 1x1 convolution = the 1x1 convolution of the subsampled map
             xs = x[:, :, ::2, ::2].contiguous(memory_format=torch.channels_last)
             pk, b, cout = tcconv.packed(self, self.norm)
-            from .. import ops
-            return ops.conv2d_nhwc(xs, pk, b, cout, 1, relu, residual=residual)
+            return ops.conv2d_nhwc(xs, pk, b, cout, 1, relu, residual=residual, x_amax=ops.absmax(xs, per_image=True).reshape(1, -1))
         with torch.backends.cudnn.flags(allow_tf32=False):
             y = self.norm(F.conv2d(x, self.weight, None, self.stride, self.padding))
         if residual is not None:

@@ -48,14 +48,18 @@ class StandardRPNHead(nn.Module):
     def forward(self, features: List[torch.Tensor], gates: Optional[List[torch.Tensor]] = None,
                 bounds: Optional[List[torch.Tensor]] = None):
         """``gates[l]`` [N, C]: per-(image, channel) factors multiplied into features[l] first (the support correlation
-        of FsodRCNN); ``bounds[l]``: device scalar >= max|features[l] * gate|."""
+        of FsodRCNN); ``bounds[l]``: device floats [1, N], bound of max|features[l] * gate| per image.  Each image is
+        scaled by its own bound in both convolutions: its outputs do not depend on its batch mates."""
         logits, deltas = [], []
         A = self.objectness_logits.out_channels
         for l, x in enumerate(features):
             g = gates[l] if gates is not None else None
             if tcconv.supported(self.conv, x) and (g is None or x.shape[1] % 32 == 0):
-                t = tcconv.conv(x, self.conv, relu=True, a_gate=g, x_amax=bounds[l] if bounds is not None else None)
-                y = tcconv.conv(t, self.objectness_logits, extra=self.anchor_deltas)       # [N, A + 4A (+pad), H, W]
+                x_amax = bounds[l] if bounds is not None else ops.absmax(ops.nhwc(x), per_image=True).reshape(1, -1)
+                t_amax = ops.new_amax(x.device, x.shape[0])
+                t = tcconv.conv(x, self.conv, relu=True, a_gate=g, x_amax=x_amax, y_amax=t_amax)
+                y = tcconv.conv(t, self.objectness_logits, extra=self.anchor_deltas,       # [N, A + 4A (+pad), H, W]
+                                x_amax=t_amax.reshape(1, -1))
                 logits.append(y[:, :A])
                 deltas.append(y[:, A:A + self.anchor_deltas.out_channels])
             else:                                                                          # CPU tensors

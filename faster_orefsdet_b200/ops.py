@@ -460,13 +460,16 @@ def conv2d_pack(weight: Tensor) -> Tensor:
     return packed
 
 
-def absmax(x: Tensor) -> Tensor:
-    """max |x| of a dense fp32 tensor as a device float[1] (no host sync): the operand bound conv2d_nhwc needs."""
+def absmax(x: Tensor, per_image: bool = False) -> Tensor:
+    """max |x| of a dense fp32 tensor as a device float[1] (no host sync): the operand bound conv2d_nhwc needs.
+    ``per_image``: one maximum per index of dim 0 instead, as device floats [N] (x_amax.reshape(1, N) of conv2d_nhwc)."""
     _chk(x, torch.float32, "x")
     if not (x.is_contiguous() or x.is_contiguous(memory_format=torch.channels_last)):
         raise _lib.FodError("absmax: dense tensor expected")
-    out = torch.empty((1,), dtype=torch.float32, device=x.device)
-    _lib.check(_lib.lib().fod_absmax(_ptr(x), x.numel(), _ptr(out), _stream()), "fod_absmax")
+    rows = x.shape[0] if per_image else 1
+    out = torch.empty((rows,), dtype=torch.float32, device=x.device)
+    if rows:
+        _lib.check(_lib.lib().fod_absmax_rows(_ptr(x), rows, x.numel() // rows, _ptr(out), _stream()), "fod_absmax_rows")
     return out
 
 

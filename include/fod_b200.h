@@ -344,6 +344,10 @@ int fod_ese_gate(const float* colsum, int n, int tiles_per_img, int channels, lo
                  const float* fc_bias, float* gate, fod_stream_t stream);
 /* max |x| of a dense fp32 array -> *out (device float; zeroed inside) */
 int fod_absmax(const float* x, size_t n, float* out, fod_stream_t stream);
+/* max |x| of each of `rows` arrays of row_len floats laid end to end (one per image of a batch) -> out[rows] (device
+ * floats; zeroed inside): the per-image operand bounds of fod_conv2d_nhwc (amax_per_image bit 0).  row_len a multiple of 4
+ * when rows > 1. */
+int fod_absmax_rows(const float* x, int rows, size_t row_len, float* out, fod_stream_t stream);
 
 /* ---------------------------------------------------------------------------
  * H0  GroupNorm (+ ReLU) over NHWC maps: the normalisation of CenterNetHead's tower

@@ -158,7 +158,20 @@ def test_roi_relation_final_stay_inside_their_buffers(monkeypatch):
     assert int(status.item()) == 0
 
 
-@pytest.mark.parametrize("sizes,B,C", [(((25, 42), (13, 21), (7, 11)), 2, 3), (((8, 16),), 1, 1), (((1, 1), (5, 3)), 1, 7)])
+def test_roi_align_14_wide_stays_inside_its_buffers(monkeypatch):
+    """Resolution 14 over 1024-channel stride-16 maps (the ROI pooling of the FsodRCNN path), ragged counts, boxes of
+    every kind including sampling grids beyond the tap tables."""
+    from tests.test_ops_gpu import roi14_case
+    f, bx, counts = roi14_case(1024, 13, 17, 2, 950)
+    fd, bd, cd = f.to(DEV), bx.to(DEV), counts.to(DEV)
+
+    def valid(pooled):
+        return [pooled[p, :int(counts[p])] for p in range(bx.shape[0])]
+
+    run_guarded(monkeypatch, lambda: ops.roi_align([fd], [16], bd, cd, 2, 14), valid)
+
+
+@pytest.mark.parametrize("sizes,B,C",[(((25, 42), (13, 21), (7, 11)), 2, 3), (((8, 16),), 1, 1), (((1, 1), (5, 3)), 1, 7)])
 def test_correlate_levels_stays_inside_its_buffers(monkeypatch, sizes, B, C):
     sd = head_state_dict()
     qs = [synth.tensor((B, 128, h, w), 150 + h + 3 * i, -1.5, 1.5).to(DEV) for i, (h, w) in enumerate(sizes)]

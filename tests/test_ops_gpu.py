@@ -428,6 +428,60 @@ def test_roi_align_tile_stationary_is_bit_identical_to_per_roi(height, width, C)
                     assert_close(got[p, :n].reshape(n, 8, 8, 128).permute(0, 3, 1, 2)[ok], ref, what=f"problem {p} vs oracle")
 
 
+def roi14_case(ch, h, w, ppi, seed):
+    """B = 2 stride-16 maps [2, ch, h, w] and [2 * ppi, 100, 4] boxes of every kind _roi_stress_boxes makes, a few of
+    them wider than 7 * 14 * 16 = 1568 px (sampling grid beyond the tap tables), with counts 100, 37, 0, 1 (repeated)."""
+    B, cap = 2, 100
+    P = B * ppi
+    f = synth.tensor((B, ch, h, w), seed, -3.0, 3.0)
+    bx = _roi_stress_boxes(P * cap, seed + 1, 16 * h, 16 * w).reshape(P, cap, 4)
+    wide = synth.tensor((P, 6, 4), seed + 2, 0.0, 1.0)
+    bx[:, 2:8] = torch.stack((-400.0 * wide[..., 0], 16 * h * wide[..., 1], 1700.0 + 2000.0 * wide[..., 2],
+                              16 * h * wide[..., 1] + 8.0 + 300.0 * wide[..., 3]), -1)
+    counts = torch.tensor(([100, 37, 0, 1] * 2)[:P], dtype=torch.int32)
+    return f, bx, counts
+
+
+@pytest.mark.parametrize("ch,hw,ppi", [(128, (6, 8), 1), (256, (13, 17), 2), (1024, (50, 84), 3), (1024, (6, 8), 2),
+                                       (128, (50, 84), 3), (256, (6, 8), 3), (1024, (13, 17), 1)])
+def test_roi_align_14_wide_maps_matches_torchvision_float64(ch, hw, ppi):
+    """fod_roi_align_wide at resolution 14 (roi_align_kernel<14>, ch / 128 channel blocks in blockIdx.z, both the tap-table
+    and the sample-by-sample path) on one stride-16 level against torchvision's ROIAlign in float64 (aligned=True,
+    adaptive sampling): within 1e-5 of the map maximum; the problem -> image index is p // problems_per_image; rows at
+    and beyond each count keep the sentinel the output was filled with.  An inverted box has an empty sampling grid
+    (torchvision rejects it): its row must be exactly zero.
+    On the 50 x 84 maps fp32 itself misses 1e-5: a sample coordinate near x = 60 carries a rounding error of a few
+    1e-6 map pixels (one ulp is 3.8e-6), and between two pixels of this random map the value changes by up to 6.  torchvision's own
+    fp32 ROIAlign (the operator of the reference) is off by 3.7e-5 of max|f| = 3 there.  So every element must be within
+    1e-5 of max|f| of the float64 result plus the error of torchvision's fp32 result at that element, and within 1e-5
+    of max|f| of that fp32 result (measured on a B200: 3.2e-5 from float64 where fp32 torchvision is 3.7e-5 off)."""
+    from torchvision.ops import roi_align as tv_roi_align
+    h, w = hw
+    f, bx, counts = roi14_case(ch, h, w, ppi, 900 + ch + h)
+    P, cap = bx.shape[:2]
+    assert bool(((bx[:, :8, 2] - bx[:, :8, 0]) > 1568.0).any())
+    out = torch.full((P, cap, 196, ch), -7.0, device=DEV)
+    ops.roi_align([f.to(DEV)], [16], bx.to(DEV), counts.to(DEV), ppi, 14, out=out)
+    got = out.cpu()
+    tol = 1e-5 * float(f.abs().max())
+    for p in range(P):
+        n = int(counts[p])
+        assert bool((got[p, n:] == -7.0).all()), f"problem {p}: rows beyond the count were written"
+        if n == 0:
+            continue
+        ok = (bx[p, :n, 2] >= bx[p, :n, 0]) & (bx[p, :n, 3] >= bx[p, :n, 1])
+        rois = torch.cat((torch.full((n, 1), float(p // ppi)), bx[p, :n]), 1).double()
+        ref = torch.zeros((n, ch, 14, 14), dtype=torch.float64)
+        ref[ok] = tv_roi_align(f.double(), rois[ok], 14, 1.0 / 16, sampling_ratio=0, aligned=True)
+        ref32 = torch.zeros((n, ch, 14, 14), dtype=torch.float64)
+        ref32[ok] = tv_roi_align(f, rois[ok].float(), 14, 1.0 / 16, sampling_ratio=0, aligned=True).double()
+        g = got[p, :n].reshape(n, 14, 14, ch).permute(0, 3, 1, 2).double()
+        err = (g - ref).abs() - (ref32 - ref).abs()
+        assert float(err.max()) <= tol, f"problem {p}: {float(err.max()):.3e} beyond fp32 torchvision's error (> {tol:.3e})"
+        err32 = (g - ref32).abs()
+        assert float(err32.max()) <= tol, f"problem {p}: max err vs fp32 torchvision {float(err32.max()):.3e} > {tol:.3e}"
+
+
 def test_roi_align_tile_stationary_resumes_after_a_full_task_list():
     """300 small boxes crowded into one corner: every ROI's eight bin rows start inside the same 8 x 8-pixel tile, more
     tasks than one pass of the tile-stationary kernel holds (it stops at the first ROI that does not fit and resumes)."""
