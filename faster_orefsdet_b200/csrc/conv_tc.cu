@@ -65,7 +65,6 @@ constexpr uint32_t kOffBias = kOffSum + 4 * kSlabBytes;
 constexpr uint32_t kOffBars = kOffBias + 128 * 4;
 constexpr uint32_t kNumBars = 2 * kQStages + 3 * kStages + 2 * kAccStages;
 constexpr uint32_t kOffTmemPtr = kOffBars + kNumBars * 8;
-constexpr uint32_t kOffFlag = kOffTmemPtr + 8;
 constexpr uint32_t kSmemBytes = kOffTmemPtr + 16;
 constexpr uint32_t kSmemAlloc = kSmemBytes + 1024;
 
@@ -148,9 +147,29 @@ struct Params {
   int x_presplit_from;     // single-tap path: input channels >= this are pre-split, each slice at the scale of ITS x_amax row
   int slice_ch[8];         // first channel of the slice that x_amax row k bounds
   uint32_t q_stage_bytes, q_stage_stride;
+  // shared-memory A operand (conv_tc_kernel<true>): an A stage is three TMA boxes of a_box_bytes; the weights of one tap
+  // row (3 taps x hi / lo) form a B stage of b_stage_bytes at off_b, b_stages deep; the output staging starts at off_sum
+  uint32_t a_box_bytes, b_stage_bytes, off_b, off_sum;
+  int b_stages;
 };
 
-__global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_constant__ Params P) {
+// Shared-memory A variant (kSmemA), for 3x3 layers whose input arrives pre-split at one scale: the stored fp16 halves
+// are what the MMA multiplies, so the tensor core reads them straight from the TMA-staged tile instead of from tensor
+// memory, and there are no converter warps.  A K-major SW128 descriptor has one stride between 8-row groups, so the
+// 18-pixel-wide halo cannot serve as the operand; per 32-channel chunk three dx-shifted boxes of 16 x 10 pixels are
+// staged instead, and the operand of tap (dy, dx) is box dx from pixel row dy on (start + dy * 2048 bytes, 1024-aligned).
+// Stride 2: the three taps of a tap row are three 8 x 16 boxes with element strides 2, one A stage per tap row.  In a
+// 128-byte row the split format is [16 hi | 16 lo | 16 hi | 16 lo]: step ks of the K = 16 MMAs reads hi at +64 ks bytes
+// and lo at +64 ks + 32, the K advance inside a swizzle atom.  MMAs, their order and the part boundaries are those of
+// the tensor-memory path, so the result is bit-identical to it.
+constexpr int kAStagesS = 2;
+constexpr int kEpiWarpsS = 8;                // two per TMEM quadrant, splitting its 32-column slabs
+constexpr int kThreadsS = (kWarpEpi0 + kEpiWarpsS) * 32;   // TMA A, MMA, watcher, TMA B, epilogue
+constexpr uint32_t kRowBytesS1 = 16 * 128;   // one pixel row of a stride-1 box
+constexpr uint32_t kMaxDynSmem = 232448;     // opt-in dynamic shared memory per block (sm_100)
+
+template <bool kSmemA>
+__global__ void __launch_bounds__(kSmemA ? kThreadsS : kThreads, 1) conv_tc_kernel(const __grid_constant__ Params P) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const uint32_t sbase = smem_u32(smem);
@@ -161,7 +180,12 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
 #ifdef FOD_DBG
   long long* const dbg_buf = (pair == 0 && rank == 0) ? g_dbg : nullptr;
 #endif
-  const uint32_t bar0 = sbase + kOffBars;
+  const uint32_t off_sum = kSmemA ? P.off_sum : kOffSum;
+  const uint32_t off_bias = kSmemA ? P.off_sum + (uint32_t)P.ncol32 * kSlabBytes : kOffBias;
+  const uint32_t off_bars = kSmemA ? off_bias + 128 * 4 : kOffBars;
+  const uint32_t off_tmem_ptr = off_bars + kNumBars * 8, off_flag = off_tmem_ptr + 8;
+  const uint32_t bar0 = sbase + off_bars;
+  constexpr int epi_warps = kSmemA ? kEpiWarpsS : 4;
   auto q_full = [&](int s) { return bar0 + 8u * s; };                                  // TMA -> converters
   auto q_empty = [&](int s) { return bar0 + 8u * (kQStages + s); };                    // converters -> TMA
   auto b_full = [&](int s) { return bar0 + 8u * (2 * kQStages + s); };                 // TMA of both CTAs -> MMA (leader)
@@ -183,25 +207,27 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
   };
   image_scale(0);
 
+  // kSmemA: q_full / q_empty are the A stages (TMA bytes of both CTAs -> MMA, MMA commit -> TMA), b_full / st_free the
+  // weight stages of one tap row; `ready` is unused
   if (tid == 0) {
     for (int s = 0; s < kQStages; ++s) {
       mbar_init(q_full(s), 1);
-      mbar_init(q_empty(s), kConvWarps);
+      mbar_init(q_empty(s), kSmemA ? 1 : kConvWarps);
     }
     for (int s = 0; s < kStages; ++s) {
-      mbar_init(b_full(s), 1);              // unused (the weight bytes complete `ready`)
+      mbar_init(b_full(s), 1);              // unused without kSmemA (the weight bytes complete `ready`)
       mbar_init(ready(s), kConvWarps + 1);  // one set of 8 warps per CTA, both CTAs, + the weight producer's expect_tx
       mbar_init(st_free(s), 1);
     }
     for (int s = 0; s < kAccStages; ++s) {
       mbar_init(acc_full(s), 1);
-      mbar_init(acc_empty(s), 8);  // 4 epilogue warps x 2 CTAs
+      mbar_init(acc_empty(s), 2 * epi_warps);  // epilogue warps x 2 CTAs
     }
-    *reinterpret_cast<volatile uint32_t*>(smem + kOffFlag) = 0;
+    *reinterpret_cast<volatile uint32_t*>(smem + off_flag) = 0;
     fence_barrier_init();
   }
   if (warp == kWarpAlloc) {
-    tmem_alloc<2>(sbase + kOffTmemPtr, kTmemCols);
+    tmem_alloc<2>(sbase + off_tmem_ptr, kTmemCols);
     tmem_relinquish<2>();
   }
   if (warp == kWarpTma && lane == 0) {
@@ -213,7 +239,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
   tc_fence_before();
   cluster_sync();
   tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr);
+  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(smem + off_tmem_ptr);
 
   // Static schedule: iteration i of pair k owns pair-unit pu = i * num_pairs + k = (tile pair tp, channel group grp),
   // grp innermost so that the pairs working on the same input tile run at the same time (L2 reuse of the halo).
@@ -222,7 +248,158 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
   auto unit_grp = [&](int i) { return (i * P.num_pairs + pair) % P.n_groups; };
   const int chunks = P.chunks, taps = P.taps, cin_chunks = P.cin_chunks;
 
-  if (warp == kWarpTma) {
+  // kSmemA: the unit of synchronisation is the tap row (cc, dy): one weight stage, and a new A stage at dy == 0 (stride 1)
+  // or at every tap row (stride 2)
+  const bool per_row_a = P.per_tap != 0;
+  const uint32_t a_stage_bytes = 3 * P.a_box_bytes;
+  if (kSmemA && warp == kWarpTma) {
+    // ------------------------------------------------------------------ TMA producer: A stages (three boxes each)
+    if (lane == 0) {
+      const uint32_t a_full_leader = map_to_cta(q_full(0), 0);
+      uint32_t ga = 0;
+      for (int i = 0; in_range(i); ++i) {
+        const int t = min(unit_tile(i), P.tiles_total - 1);
+        const int n = t / P.tiles_per_img, tt = t - n * P.tiles_per_img;
+        const int ty = tt / P.tiles_x, tx = tt - ty * P.tiles_x;
+        const int x0 = tx * kTileW * P.stride - 1, y0 = ty * kTileH * P.stride - 1;
+        for (int cc = 0; cc < cin_chunks; ++cc)
+          for (int dy = 0; dy < 3; dy += per_row_a ? 1 : 3, ++ga) {
+            const int s = (int)(ga % kAStagesS);
+            mbar_wait(q_empty(s), ((ga / kAStagesS) & 1) ^ 1);
+            if (rank == 0) mbar_arrive_expect_tx(q_full(s), 2 * a_stage_bytes);
+            for (int dx = 0; dx < 3; ++dx)
+              tma_load_4d_2sm(sbase + kOffQ + s * a_stage_bytes + dx * P.a_box_bytes, &P.in_map, a_full_leader + 8u * s,
+                              cc * kChunk, x0 + dx, y0 + dy, n);
+          }
+      }
+    }
+  } else if (kSmemA && warp == kWarpTmaB) {
+    // ------------------------------------------------------------------ TMA producer: weights of a tap row
+    if (lane == 0) {
+      const uint32_t b_full_leader = map_to_cta(b_full(0), 0);
+      const uint32_t plane = (uint32_t)P.nhalf * 64u;
+      uint32_t g = 0;
+      for (int i = 0; in_range(i); ++i) {
+        const int row0 = unit_grp(i) * P.n_group + (int)rank * P.nhalf;
+        for (int cc = 0; cc < cin_chunks; ++cc)
+          for (int dy = 0; dy < 3; ++dy, ++g) {
+            const int s = (int)(g % P.b_stages);
+            mbar_wait(st_free(s), ((g / P.b_stages) & 1) ^ 1);
+            if (rank == 0) mbar_arrive_expect_tx(b_full(s), 12 * plane);   // 3 taps x hi / lo x 2 CTAs
+            for (int dx = 0; dx < 3; ++dx) {
+              const int k0 = ((dy * 3 + dx) * cin_chunks + cc) * kChunk;
+              const uint32_t dst = sbase + P.off_b + s * P.b_stage_bytes + dx * 2 * plane;
+              tma_load_2d_2sm(dst, &P.whi_map, b_full_leader + 8u * s, k0, row0);
+              tma_load_2d_2sm(dst + plane, &P.wlo_map, b_full_leader + 8u * s, k0, row0);
+            }
+          }
+      }
+    }
+  } else if (kSmemA && warp == kWarpMma) {
+    // ------------------------------------------------------------------ MMA issuer (leader CTA), A from shared memory
+    if (rank == 0) {
+      const uint32_t idesc = idesc_f16(256, P.n_group);
+      const uint32_t plane16 = ((uint32_t)P.nhalf * 64u) >> 4, tap16 = 2 * plane16, bstep16 = P.b_stage_bytes >> 4;
+      const uint32_t box16 = P.a_box_bytes >> 4, astep16 = a_stage_bytes >> 4, row16 = per_row_a ? 0u : kRowBytesS1 >> 4;
+      const uint32_t flag = sbase + off_flag;
+      const int cpp = P.chunks_per_part, b_stages = P.b_stages;
+      const uint64_t a_desc0 = smem_desc_k_sw128(sbase + kOffQ), b_desc0 = smem_desc_k_sw64(sbase + P.off_b);
+      const uint32_t d0 = tmem_base + kColAcc;
+      uint64_t a_desc = a_desc0, b_desc = b_desc0;
+      uint32_t d = d0, af = acc_full(0), sf = st_free(0), qf = q_empty(0);
+      uint32_t upto = 0, g = 0;
+      int sb = 0, sa = 0, pc = 0, as_ = 0;
+      for (int i = 0; in_range(i); ++i) {
+        int lc = 0;
+        for (int cc = 0; cc < cin_chunks; ++cc)
+          for (int dy = 0; dy < 3; ++dy, ++g) {
+            while (upto <= g) {
+              uint32_t v;
+              asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"(flag) : "memory");
+              upto = __shfl_sync(0xffffffffu, v, 0);
+            }
+            tc_fence_after();
+            const uint64_t a_row = a_desc + (uint64_t)(dy * row16);
+#pragma unroll 1
+            for (int dx = 0; dx < 3; ++dx, ++lc) {
+              const bool last = (pc == cpp - 1) || (lc == chunks - 1);
+              if (elect_one()) {
+                const uint64_t a = a_row + dx * box16, bhi = b_desc + dx * tap16, blo = bhi + plane16;
+#pragma unroll
+                for (int ks = 0; ks < 2; ++ks) {   // A: [16 hi | 16 lo] per 64 bytes of the row; B: 32 bytes per step
+                  const uint64_t ah = a + (uint64_t)(ks * 4), al = ah + 2u, boff = (uint64_t)(ks * 2);
+                  mma_f16_ss<2>(d, ah, bhi + boff, idesc, (pc | ks) ? 1u : 0u);
+                  mma_f16_ss<2>(d, al, bhi + boff, idesc, 1u);
+                  mma_f16_ss<2>(d, ah, blo + boff, idesc, 1u);
+                }
+                if (last) mma_commit_pair(af, 3);
+              }
+              __syncwarp();
+              if (last) {
+                pc = 0;
+                as_ ^= 1;
+                d = d0 + (uint32_t)as_ * 128u;
+                af = acc_full(as_);
+              } else {
+                ++pc;
+              }
+            }
+            const bool a_done = per_row_a || dy == 2;
+            if (elect_one()) {
+              mma_commit_pair(sf, 3);
+              if (a_done) mma_commit_pair(qf, 3);
+            }
+            __syncwarp();
+            if (++sb == b_stages) {
+              sb = 0;
+              b_desc = b_desc0;
+              sf = st_free(0);
+            } else {
+              b_desc += bstep16;
+              sf += 8;
+            }
+            if (a_done) {
+              if (++sa == kAStagesS) {
+                sa = 0;
+                a_desc = a_desc0;
+                qf = q_empty(0);
+              } else {
+                a_desc += astep16;
+                qf += 8;
+              }
+            }
+          }
+      }
+    }
+  } else if (kSmemA && warp == kWarpAlloc) {
+    // ------------------------------------------------------------------ barrier watcher of the MMA warp, per tap row
+    if (rank == 0 && lane == 0) {
+      const uint32_t flag = sbase + off_flag;
+      uint32_t g = 0, ga = 0, gp = 0;
+      const int cpp = P.chunks_per_part;
+      for (int i = 0; in_range(i); ++i) {
+        int pc = 0, lc = 0;
+        for (int cc = 0; cc < cin_chunks; ++cc)
+          for (int dy = 0; dy < 3; ++dy, ++g) {
+            for (int dx = 0; dx < 3; ++dx, ++lc) {   // a part that starts in this row needs its accumulator drained
+              if (pc == 0) mbar_wait(acc_empty(gp % kAccStages), ((gp / kAccStages) & 1) ^ 1);
+              if (pc == cpp - 1 || lc == chunks - 1) {
+                ++gp;
+                pc = 0;
+              } else {
+                ++pc;
+              }
+            }
+            if (per_row_a || dy == 0) {
+              mbar_wait(q_full(ga % kAStagesS), (ga / kAStagesS) & 1);
+              ++ga;
+            }
+            mbar_wait(b_full(g % P.b_stages), (g / P.b_stages) & 1);
+            asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(flag), "r"(g + 1) : "memory");
+          }
+      }
+    }
+  } else if (!kSmemA && warp == kWarpTma) {
     // ------------------------------------------------------------------ TMA producer: input tile + halo, per 32 channels
     if (lane == 0) {
       uint32_t g = 0;
@@ -244,7 +421,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
           }
       }
     }
-  } else if (warp == kWarpTmaB) {
+  } else if (!kSmemA && warp == kWarpTmaB) {
     // ------------------------------------------------------------------ TMA producer: weight chunk (hi + lo planes)
     if (lane == 0) {
       const uint32_t b_full_leader = map_to_cta(ready(0), 0);   // the weight bytes complete the `ready` barrier
@@ -266,7 +443,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
           }
       }
     }
-  } else if (warp == kWarpMma) {
+  } else if (!kSmemA && warp == kWarpMma) {
     // ------------------------------------------------------------------ MMA issuer (leader CTA)
     // The whole warp runs the loop converged and one elected lane issues: every operand of tcgen05.mma is then a
     // warp-uniform value that ptxas keeps in uniform registers.  (Inside an `if (lane == 0)` region the same code
@@ -274,7 +451,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
     if (rank == 0) {
       const uint32_t idesc = idesc_f16(256, P.n_group);
       const uint32_t plane16 = ((uint32_t)P.nhalf * 64u) >> 4, bstep16 = b_stage >> 4;
-      const uint32_t flag = sbase + kOffFlag;
+      const uint32_t flag = sbase + off_flag;
       const int cpp = P.chunks_per_part;
       // Everything a chunk's MMAs need is carried in (uniform) registers and advanced AFTER the chunk has been issued,
       // so nothing but the flag test sits between the last MMA of one chunk and the first MMA of the next: the
@@ -332,13 +509,13 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         }
       }
     }
-  } else if (warp == kWarpAlloc) {
+  } else if (!kSmemA && warp == kWarpAlloc) {
     // ------------------------------------------------------------------ barrier watcher of the MMA warp (leader)
     // An mbarrier wait costs ~200 cycles even when the phase completed long ago, and this thread is the only one that
     // waits per chunk: the weight bytes of both CTAs and the converter warps of both CTAs therefore complete ONE
     // barrier per stage (ready: 16 warp arrivals + the producer's expect_tx arrival + the TMA bytes).
     if (rank == 0 && lane == 0) {
-      const uint32_t flag = sbase + kOffFlag;
+      const uint32_t flag = sbase + off_flag;
       uint32_t g = 0, gp = 0;
       const int cpp = P.chunks_per_part;
       for (int i = 0; in_range(i); ++i) {
@@ -361,14 +538,16 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         }
       }
     }
-  } else if (warp >= kWarpEpi0 && warp < kWarpEpi0 + 4) {
+  } else if (warp >= kWarpEpi0 && warp < kWarpEpi0 + epi_warps) {
     // ------------------------------------------------------------------ epilogue: one output pixel per lane
-    const int qd = warp & 3;
+    // warp = (TMEM quadrant qd, slab phase sp): the warp handles the 32-column slabs j = sp, sp + epi_warps / 4, ...
+    const int qd = warp & 3, sp = (warp - kWarpEpi0) >> 2;
+    constexpr int sstep = epi_warps / 4;
     const int m = qd * 32 + lane;
     const uint32_t acc_empty_leader = map_to_cta(acc_empty(0), 0);
     const bool issuer = (warp == kWarpEpi0 && lane == 0);
-    const uint32_t row_s = sbase + kOffSum + (uint32_t)((m >> 3) * 1024 + (m & 7) * 128);
-    const uint32_t bias_s = sbase + kOffBias;
+    const uint32_t row_s = sbase + off_sum + (uint32_t)((m >> 3) * 1024 + (m & 7) * 128);
+    const uint32_t bias_s = sbase + off_bias;
     const int ncol32 = P.ncol32, parts = P.parts;
     const float w_inv = __ldg(P.w_inv);
     float rescale = xs_inv * w_inv;   // undoes the two power-of-two operand scales (exact)
@@ -403,12 +582,12 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
       if (P.res && px_valid)
         res_px = P.res + (((size_t)n * P.res_h + (oy >> P.res_shift)) * P.res_w + (ox >> P.res_shift)) * P.cout;
       if (issuer) tma_store_wait_read<0>();  // the previous tile has left the staging slabs
-      named_bar_sync(1, 128);
+      named_bar_sync(1, 32 * epi_warps);
       {
         const int ch = ch0 + m;
-        reinterpret_cast<float*>(smem + kOffBias)[m] = (P.bias && ch < P.cout) ? __ldg(P.bias + ch) : 0.f;
+        if (sp == 0) reinterpret_cast<float*>(smem + off_bias)[m] = (P.bias && ch < P.cout) ? __ldg(P.bias + ch) : 0.f;
       }
-      named_bar_sync(1, 128);
+      named_bar_sync(1, 32 * epi_warps);
 #pragma unroll 1
       for (int part = 0; part < parts; ++part, ++gp) {
         const int as_ = gp % kAccStages;
@@ -418,12 +597,16 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         const uint32_t trow = tmem_base + ((uint32_t)(qd * 32) << 16) + col_acc + as_ * acc_w;
         const int part_chunks = min(P.chunks_per_part, P.chunks - part * P.chunks_per_part);
         const float comp = 1.f + P.rz_kappa * 0.5f * (float)(part_chunks * mma_per_chunk);
+        if (sp >= ncol32) {   // a group narrower than the epilogue's slab phases: nothing to read
+          __syncwarp();
+          if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * as_);
+        }
 #pragma unroll 1
-        for (int j = 0; j < ncol32; ++j) {
+        for (int j = sp; j < ncol32; j += sstep) {
           uint32_t v[32];
           tmem_ld32(trow + j * 32, v);
           tmem_wait_ld();
-          if (j == ncol32 - 1) {  // accumulator fully read: hand it back to the MMA warp
+          if (j + sstep >= ncol32) {  // this warp's columns of the accumulator are read: hand them back to the MMA warp
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * as_);
@@ -510,19 +693,19 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         vmax = 0.f;
       }
       fence_proxy_async_smem();
-      named_bar_sync(1, 128);
+      named_bar_sync(1, 32 * epi_warps);
       if (issuer && do_store) {
         for (int j = 0; j < ncol32 && ch0 + j * 32 < P.cout; ++j)
-          tma_store_4d(&P.out_map, sbase + kOffSum + j * kSlabBytes, ch0 + j * 32, tx * kTileW, ty * kTileH, n);
+          tma_store_4d(&P.out_map, sbase + off_sum + j * kSlabBytes, ch0 + j * 32, tx * kTileW, ty * kTileH, n);
         tma_store_commit();
       }
-      if (P.colsum && do_store && qd < ncol32) {
+      if (P.colsum && do_store && sp == 0 && qd < ncol32) {
         // Channel sums over the tile's pixels that lie inside the image, in a fixed order (deterministic, independent of
         // the batch).  Warp = 32-channel slab; lane = (row offset 0..3, 4-channel group): a warp reads four consecutive
         // 128-byte rows per step (conflict-free), 32 steps cover the tile; the four row offsets meet in two shuffles.
         const int vy = min(kTileH, P.ho - ty * kTileH), vx = min(kTileW, P.wo - tx * kTileW);
         const uint32_t c4 = (uint32_t)(lane & 7), ro = (uint32_t)(lane >> 3);
-        const uint32_t sb = sbase + kOffSum + (uint32_t)qd * kSlabBytes;
+        const uint32_t sb = sbase + off_sum + (uint32_t)qd * kSlabBytes;
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f), acq = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll 4
         for (uint32_t r0 = 0; r0 < 128; r0 += 4) {
@@ -554,7 +737,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
       const uint32_t wmax = __reduce_max_sync(0xffffffffu, __float_as_uint(vmax));
       if (lane == 0 && wmax) atomicMax(reinterpret_cast<unsigned int*>(P.y_amax), wmax);
     }
-  } else if (warp >= kWarpConv0) {
+  } else if (!kSmemA && warp >= kWarpConv0) {
     // ------------------------------------------------------------------ converters
     // Phase A, once per staged tile (i.e. once per 32 input channels, not once per tap): all 16 warps convert the tile
     // IN PLACE from fp32 to scaled fp16 hi / lo: a 128-byte pixel row of 32 floats becomes [32 x hi | 32 x lo], the
@@ -1022,7 +1205,26 @@ static int conv2d_nhwc_impl(const float* x, int n, int h, int w, int cin, long x
   FOD_REQUIRE(tiles * prm.n_groups < (1L << 30), "fod_conv2d_nhwc: too many tiles");
   prm.tiles_total = (int)tiles;
   prm.pair_units = (int)((tiles + 1) / 2) * prm.n_groups;
-  int rc = cvt::make_nhwc_map_strided(&prm.in_map, x, n, h, w, cin, x_pixel_stride, cvt::kChunk, halo_w, halo_h, stride);
+  // The shared-memory A kernel serves 3x3 layers whose input is pre-split at one scale (stride 1, or stride 2 with a single
+  // bound, where the stored halves are brought to the common scale by exactly 1), for the channel groups whose A stages,
+  // weight stages and output staging fit the shared memory; everything else converts through tensor memory.
+  bool smem_a = (prm.x_presplit || (stride == 2 && x_presplit_from == 0 && n_amax == 1)) &&
+                (prm.n_group <= 96 || (stride == 2 && prm.n_group == 128));
+  uint32_t smem_alloc = cvt::kSmemAlloc;
+  if (smem_a) {
+    prm.a_box_bytes = (uint32_t)(cvt::kTileW * (per_tap ? cvt::kTileH : cvt::kTileH + 2) * 128);
+    prm.b_stage_bytes = (uint32_t)(6 * prm.nhalf * 64 + 1023) / 1024 * 1024;
+    prm.off_b = cvt::kOffQ + cvt::kAStagesS * 3 * prm.a_box_bytes;
+    const uint32_t tail = (uint32_t)prm.ncol32 * cvt::kSlabBytes + 128 * 4 + cvt::kNumBars * 8 + 16;
+    const long room = (long)cvt::kMaxDynSmem - 1024 - prm.off_b - tail;
+    prm.b_stages = (int)(room / (long)prm.b_stage_bytes < cvt::kStages ? room / (long)prm.b_stage_bytes : cvt::kStages);
+    prm.off_sum = prm.off_b + (uint32_t)prm.b_stages * prm.b_stage_bytes;
+    smem_alloc = prm.off_sum + tail + 1024;
+    smem_a = prm.b_stages >= 2;
+  }
+  int rc = smem_a && !per_tap
+               ? cvt::make_nhwc_map_strided(&prm.in_map, x, n, h, w, cin, x_pixel_stride, cvt::kChunk, cvt::kTileW, cvt::kTileH + 2, 1)
+               : cvt::make_nhwc_map_strided(&prm.in_map, x, n, h, w, cin, x_pixel_stride, cvt::kChunk, halo_w, halo_h, stride);
   if (rc != FOD_OK) return rc;
   rc = cvt::make_nhwc_map_strided(&prm.out_map, y, n, ho, wo, cout, y_pixel_stride, cvt::kChunk, cvt::kTileW, cvt::kTileH, 1);
   if (rc != FOD_OK) return rc;
@@ -1038,11 +1240,12 @@ static int conv2d_nhwc_impl(const float* x, int n, int h, int w, int cin, long x
   FOD_CUDA_CALL(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const int max_pairs = sms / 2 > 0 ? sms / 2 : 1;
   prm.num_pairs = prm.pair_units < max_pairs ? prm.pair_units : max_pairs;
-  FOD_CUDA_CALL(cudaFuncSetAttribute(cvt::conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cvt::kSmemAlloc));
+  auto kernel = smem_a ? cvt::conv_tc_kernel<true> : cvt::conv_tc_kernel<false>;
+  FOD_CUDA_CALL(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_alloc));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(2 * prm.num_pairs);
-  cfg.blockDim = dim3(cvt::kThreads);
-  cfg.dynamicSmemBytes = cvt::kSmemAlloc;
+  cfg.blockDim = dim3(smem_a ? cvt::kThreadsS : cvt::kThreads);
+  cfg.dynamicSmemBytes = smem_alloc;
   cfg.stream = as_stream(stream);
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
@@ -1051,7 +1254,7 @@ static int conv2d_nhwc_impl(const float* x, int n, int h, int w, int cin, long x
   at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, cvt::conv_tc_kernel, prm);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, prm);
   if (e != cudaSuccess) {
     set_error("fod_conv2d_nhwc: launch failed: %s", cudaGetErrorString(e));
     return FOD_ERR_CUDA;

@@ -17,6 +17,20 @@ shapes = [  # name, H, W, Cin, Cout, k (a name ending in "_s2": stride 2)
     ("fpn_out3", 80, 80, 128, 128, 3), ("fpn_lat3", 80, 80, 256, 128, 1), ("tower4", 40, 40, 128, 128, 3),
 ]
 only = sys.argv[2].split(",") if len(sys.argv) > 2 else None
+# the 3x3 layers whose input the model hands over pre-split (split hand-off): also timed with such an input, which the
+# shared-memory A kernel serves (OSA5, N = 112, stays on the tensor-memory path)
+PRESPLIT = {"stem3_s2", "stem2", "osa2_0", "osa2_1", "osa3_0", "osa3_1", "osa4_0", "osa4_1", "osa5_0"}
+
+
+def presplit(x, amax):
+    """fp32 NHWC view -> [16 x fp16 hi | 16 x fp16 lo] of x * 2^e per 16 channels (2^e from amax), as an fp32 NHWC view"""
+    n, c, h, w = x.shape
+    _, ex = torch.frexp(amax.reshape(-1)[:1])
+    xs = x.permute(0, 2, 3, 1) * ((141 - ex.to(torch.int32)) << 23).view(torch.float32)
+    hi = xs.half()
+    lo = (xs - hi.float()).half()
+    packed = torch.cat([hi.reshape(n, h, w, c // 16, 16), lo.reshape(n, h, w, c // 16, 16)], dim=-1)
+    return packed.contiguous().view(torch.float32).reshape(n, h, w, c).permute(0, 3, 1, 2)
 
 
 def timeit(fn, iters=5, warm=2):
@@ -47,11 +61,22 @@ for name, H, W, cin, cout, k in shapes:
     ref = F.relu(F.conv2d(x, wc, b, padding=k // 2, stride=st))
     err = float((y - ref).abs().max()) / float(ref.abs().max())
     t_a = timeit(lambda: ops.conv2d_nhwc(x, packed, b, cout, k, True, out=y, x_amax=ax, stride=st))
-    t_b = timeit(lambda: F.relu_(F.conv2d(x, wc, b, padding=k // 2, stride=st)))
     fl = 2.0 * B * (H // st) * (W // st) * cin * cout * k * k
+    t_b = timeit(lambda: F.relu_(F.conv2d(x, wc, b, padding=k // 2, stride=st)))
+    split = ""
+    if name in PRESPLIT:
+        xp = presplit(x, ax)
+        if st == 1:
+            fn = lambda: ops.conv2d_nhwc(xp, packed, b, cout, k, True, out=y, x_amax=ax, x_presplit=True)
+        else:
+            fn = lambda: ops.conv2d_nhwc_split(xp, packed, b, cout, k, y, ax, x_presplit_from=0, slice_ch=[0], stride=2)
+        t_s = timeit(fn)
+        same = torch.equal(fn(), ops.conv2d_nhwc(x, packed, b, cout, k, True, x_amax=ax, stride=st))
+        split = f"   pre-split {t_s:7.3f} ms ({fl/t_s/1e9:6.1f}){'' if same else '  DIFFERS from the fp32 input'}"
+        del xp
     tot_a += t_a
     tot_b += t_b
     print(f"{name:9s} {H}x{W} {cin}->{cout} k{k}: tc {t_a:7.3f} ms ({fl/t_a/1e9:6.1f} TFLOP/s fp32-equiv)   cudnn {t_b:7.3f} ms "
-          f"({fl/t_b/1e9:5.1f})   rel err {err:.1e}", flush=True)
+          f"({fl/t_b/1e9:5.1f})   rel err {err:.1e}{split}", flush=True)
     del x, y, ref
 print(f"total: tc {tot_a:.2f} ms, cudnn {tot_b:.2f} ms")

@@ -1,11 +1,16 @@
 // Probe for the fp16-split variant of the tensor-core GEMM: tcgen05.mma kind::f16 with A in tensor memory (packed
 // half2 per 32-bit column), B in shared memory (fp16, K-major, 64-byte swizzle, loaded by TMA).  x = hi + lo with
 // hi = fp16(x * 2^e), lo = fp16(x * 2^e - hi): three products hi.hi + lo.hi + hi.lo, fp32 accumulation.
-// Development tool:  f16_probe [N]
+// `ss` mode: the same products with A in shared memory instead (K-major, 128-byte swizzle, per 128-byte row
+// [16 hi | 16 lo | 16 hi | 16 lo] as the split hand-off stores it, the layout the shared-memory A convolution reads):
+// D must equal the tensor-memory result bit for bit at A start offsets of 0, 2048 and 4096 bytes (a tap row of the
+// convolution's stride-1 boxes), and both paths are timed.
+// Development tool:  f16_probe [N] [ss]   (nvcc -gencode arch=compute_100a,code=sm_100a tools/f16_probe.cu csrc/tmap.cu csrc/api.cu)
 #include <cuda_fp16.h>
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
+#include <string.h>
 #include <vector>
 
 #include "../faster_orefsdet_b200/csrc/common.cuh"
@@ -18,27 +23,11 @@ using namespace fod::tc;
 
 constexpr int K = 32;
 
-__host__ __device__ constexpr uint32_t idesc_f16(int M, int N) {
-  return (1u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ uint64_t smem_desc_k_sw64(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(512 >> 4) << 32;   // 8 rows x 64 B
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)4 << 61;            // SWIZZLE_64B
-  return d;
-}
-__device__ __forceinline__ void mma_f16_ts(uint32_t d, uint32_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-               ::"r"(d), "r"(a), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-
 struct P { CUtensorMap bhi, blo; };
 
+// ss: A from shared memory, rows starting `dy` * 16 rows (dy * 2048 bytes) into a 160-row swizzled buffer
 __global__ void __launch_bounds__(128, 1) probe(const __grid_constant__ P p, const float* __restrict__ X, float xs, float* __restrict__ out,
-                                                int N, int repeat) {
+                                                int N, int repeat, int ss, int dy) {
   extern __shared__ __align__(1024) uint8_t raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) & ~uintptr_t(1023));
   __shared__ uint64_t bar, bar2;
@@ -66,6 +55,15 @@ __global__ void __launch_bounds__(128, 1) probe(const __grid_constant__ P p, con
   }
   const uint32_t ta = t0 + ((uint32_t)(warp * 32) << 16);
   tmem_st16(ta, vh); tmem_st16(ta + 16, vl); tmem_wait_st();
+  const uint32_t sa = sb + (2 * plane + 1023) / 1024 * 1024;   // A buffer (ss)
+  {
+    const uint32_t r = (uint32_t)(tid + 16 * dy), row = sa + r * 128;
+    const uint32_t* src[8] = {vh, vh + 4, vl, vl + 4, vh + 8, vh + 12, vl + 8, vl + 12};   // 16-byte chunks of the row
+    for (uint32_t c = 0; c < 8; ++c)
+      asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(row + ((c ^ (r & 7)) << 4)), "r"(src[c][0]), "r"(src[c][1]),
+                   "r"(src[c][2]), "r"(src[c][3]) : "memory");
+    fence_proxy_async_smem();
+  }
   tc_fence_before(); __syncthreads(); tc_fence_after();
   mbar_wait(smem_u32(&bar2), 0);
   long long t_start = clock64();
@@ -74,12 +72,23 @@ __global__ void __launch_bounds__(128, 1) probe(const __grid_constant__ P p, con
     const uint64_t bh = smem_desc_k_sw64(sb), bl = smem_desc_k_sw64(sb + plane);
     for (int rep = 0; rep < repeat; ++rep) {
       if (elect_one()) {
+        if (ss) {
+          const uint64_t a = smem_desc_k_sw128(sa + (uint32_t)dy * 2048);
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks) {
-          const uint64_t bo = (uint64_t)((ks * 32) >> 4);
-          mma_f16_ts(d, t0 + ks * 8, bh + bo, idesc, (rep | ks) ? 1u : 0u);
-          mma_f16_ts(d, t0 + 16 + ks * 8, bh + bo, idesc, 1u);
-          mma_f16_ts(d, t0 + ks * 8, bl + bo, idesc, 1u);
+          for (int ks = 0; ks < 2; ++ks) {   // hi at +64 ks bytes, lo at +64 ks + 32
+            const uint64_t bo = (uint64_t)((ks * 32) >> 4), ah = a + (uint64_t)(ks * 4), al = ah + 2;
+            mma_f16_ss<1>(d, ah, bh + bo, idesc, (rep | ks) ? 1u : 0u);
+            mma_f16_ss<1>(d, al, bh + bo, idesc, 1u);
+            mma_f16_ss<1>(d, ah, bl + bo, idesc, 1u);
+          }
+        } else {
+#pragma unroll
+          for (int ks = 0; ks < 2; ++ks) {
+            const uint64_t bo = (uint64_t)((ks * 32) >> 4);
+            mma_f16_ts<1>(d, t0 + ks * 8, bh + bo, idesc, (rep | ks) ? 1u : 0u);
+            mma_f16_ts<1>(d, t0 + 16 + ks * 8, bh + bo, idesc, 1u);
+            mma_f16_ts<1>(d, t0 + ks * 8, bl + bo, idesc, 1u);
+          }
         }
       }
       __syncwarp();
@@ -89,7 +98,7 @@ __global__ void __launch_bounds__(128, 1) probe(const __grid_constant__ P p, con
   mbar_wait(smem_u32(&bar), 0);
   tc_fence_after();
   if (tid == 0 && repeat > 1)
-    printf("  %d MMAs (M=128 N=%d K=16 f16) in %lld cycles = %.1f cycles/MMA\n", repeat * 6, N, clock64() - t_start,
+    printf("  %s: %d MMAs (M=128 N=%d K=16 f16) in %lld cycles = %.1f cycles/MMA\n", ss ? "SS" : "TS", repeat * 6, N, clock64() - t_start,
            double(clock64() - t_start) / (repeat * 6));
   for (int c0 = 0; c0 < N; c0 += 32) {
     uint32_t v[32];
@@ -103,6 +112,7 @@ __global__ void __launch_bounds__(128, 1) probe(const __grid_constant__ P p, con
 
 int main(int argc, char** argv) {
   const int N = argc > 1 ? atoi(argv[1]) : 128;
+  const bool ss = argc > 2 && !strcmp(argv[2], "ss");
   std::vector<float> X(128 * K), W(N * K);
   srand(1);
   for (auto& v : X) v = (rand() / (float)RAND_MAX - 0.3f) * 37.f;
@@ -134,9 +144,40 @@ int main(int argc, char** argv) {
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { printf("encode failed %d\n", (int)r); return 2; }
   }
-  CK(cudaFuncSetAttribute(probe, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * N * 64 + 2048));
+  const int smem = (2 * N * 64 + 1023) / 1024 * 1024 + 160 * 128 + 2048;
+  CK(cudaFuncSetAttribute(probe, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  if (ss) {   // D of the SS path at each A start offset against the TS path, bit for bit; then both timed
+    std::vector<float> Ots(128 * N), Oss(128 * N);
+    probe<<<1, 128, smem>>>(p, dX, xs, dO, N, 1, 0, 0);
+    CK(cudaDeviceSynchronize());
+    CK(cudaMemcpy(Ots.data(), dO, Ots.size() * 4, cudaMemcpyDeviceToHost));
+    for (int dy = 0; dy < 3; ++dy) {
+      probe<<<1, 128, smem>>>(p, dX, xs, dO, N, 1, 1, dy);
+      CK(cudaDeviceSynchronize());
+      CK(cudaMemcpy(Oss.data(), dO, Oss.size() * 4, cudaMemcpyDeviceToHost));
+      int ndiff = 0, cmin = N, cmax = -1;
+      double dmax = 0, ref = 0;
+      for (int i = 0; i < 128 * N; ++i) {
+        ref = fmax(ref, fabs(Ots[i]));
+        if (memcmp(&Oss[i], &Ots[i], 4)) {
+          ++ndiff;
+          cmin = i % N < cmin ? i % N : cmin;
+          cmax = i % N > cmax ? i % N : cmax;
+          dmax = fmax(dmax, fabs((double)Oss[i] - Ots[i]));
+        }
+      }
+      if (!ndiff) printf("N=%d SS, A at +%d bytes: D equals the TS result bitwise\n", N, dy * 2048);
+      else printf("N=%d SS, A at +%d bytes: D differs from the TS result in %d of %d elements (columns %d..%d), by up to %.3e "
+                  "of max|D| %.3e\n", N, dy * 2048, ndiff, 128 * N, cmin, cmax, dmax / ref, ref);
+    }
+    for (int mode = 0; mode < 2; ++mode) {
+      probe<<<1, 128, smem>>>(p, dX, xs, dO, N, 2000, mode, 0);
+      CK(cudaDeviceSynchronize());
+    }
+    return 0;
+  }
   for (int repeat : {1, 2000}) {
-    probe<<<1, 128, 2 * N * 64 + 2048>>>(p, dX, xs, dO, N, repeat);
+    probe<<<1, 128, smem>>>(p, dX, xs, dO, N, repeat, 0, 0);
     CK(cudaDeviceSynchronize());
     if (repeat > 1) break;
     std::vector<float> O(128 * N);
