@@ -36,7 +36,6 @@ _PROTOTYPES = {
     "fod_version": ([], _i),
     "fod_last_error": ([ctypes.c_char_p, ctypes.c_size_t], _i),
     "fod_support_taps": ([_vp, _i, _i, _i, _vp, _vp], _i),
-    "fod_correlate": ([_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp], _i),
     "fod_correlate_levels": ([ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.POINTER(fod_level_t), _i, _vp, _vp,
                               ctypes.POINTER(_vp), ctypes.POINTER(_vp), _i, _i, _vp], _i),
     "fod_decode_topk": ([ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.POINTER(fod_level_t), _i, _i, _i, _i,
@@ -55,7 +54,6 @@ _PROTOTYPES = {
                                _vp, _vp], _i),
     "fod_relation_head": ([_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, ctypes.POINTER(_f), _vp, _vp, _vp, _vp,
                            _vp], _i),
-    "fod_split_tf32": ([_vp, _vp, ctypes.c_size_t, _vp], _i),
     "fod_final_detect": ([_vp, _vp, _vp, _i, _i, _i, _f, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
     "fod_batched_nms": ([_vp, _vp, _vp, _i, _d, _vp, _vp, _vp], _i),
     "fod_group_norm_workspace_bytes": ([_i, _i], ctypes.c_size_t),

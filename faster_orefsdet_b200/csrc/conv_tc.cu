@@ -37,9 +37,9 @@
 //     border and at Cout by the tensor map, so the output may be a channel slice of a wider NHWC buffer: concatenation
 //     is free).
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
+#include "split_format.cuh"
 #include "tc05.cuh"
 
 namespace fod {
@@ -52,7 +52,6 @@ constexpr int kTileH = 8, kTileW = 16;
 constexpr int kChunk = 32;
 constexpr int kQStages = 3, kStages = 6, kAccStages = 2;
 constexpr int kPartChunks = 16;
-constexpr float kRzKappa = 0.f;  // a scalar compensation of the truncation bias (8.8e-8 per MMA for same-sign sums, tools/rz_calib.py) over-corrects real, mixed-sign layers: off
 constexpr uint32_t kQStageStrideS1 = ((kTileH + 2) * (kTileW + 2) * 128 + 1023) / 1024 * 1024;   // 23552
 constexpr uint32_t kBPlaneMax = 64 * 64;                                    // 64 rows (half of a 128 group) x 32 fp16
 constexpr uint32_t kBStageBytes = 2 * kBPlaneMax;                           // hi + lo
@@ -77,18 +76,6 @@ constexpr uint32_t kAStageCols = 32;                // [hi: 16 columns of packed
 constexpr uint32_t kColA = 0;                       // 6 stages x 32
 constexpr uint32_t kColAcc = kStages * kAStageCols; // 2 stages x 128
 
-// 2^e with amax * 2^e in [2^13, 2^14) (and its inverse); 1 for zero / denormal-range / non-finite bounds
-__device__ __forceinline__ void pow2_scale(float amax, float& scale, float& inv) {
-  const int E = (int)((__float_as_uint(amax) >> 23) & 0xFF);
-  if (E < 32 || E > 240) {
-    scale = 1.f;
-    inv = 1.f;
-  } else {
-    scale = __uint_as_float((uint32_t)(267 - E) << 23);  // 2^(13 - (E - 127))
-    inv = __uint_as_float((uint32_t)(E - 13) << 23);
-  }
-}
-
 #ifdef FOD_DBG
 __device__ long long* g_dbg = nullptr;   // [role][g][4] clock64 stamps of pair 0 / rank 0, chunks kDbg0 .. kDbg0 + kDbgN
 constexpr uint32_t kDbg0 = 400, kDbgN = 64;
@@ -101,15 +88,6 @@ constexpr uint32_t kDbg0 = 400, kDbgN = 64;
 #define DBG_STAMP(role, g, slot)
 #endif
 
-// (a, b) -> packed fp16 pair of the rounded values (a in the low half) and of the exact remainders
-__device__ __forceinline__ void split_f16x2(float a, float b, uint32_t& hi, uint32_t& lo) {
-  const __half2 h = __floats2half2_rn(a, b);
-  const float2 hf = __half22float2(h);
-  const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-  hi = *reinterpret_cast<const uint32_t*>(&h);
-  lo = *reinterpret_cast<const uint32_t*>(&l);
-}
-
 struct Params {
   CUtensorMap in_map;   // [N][H][W][Cin] (pixel stride may exceed Cin), box 32 x halo_w x halo_h
   CUtensorMap out_map;  // [N][Ho][Wo][Cout], box 32 x 16 x 8
@@ -119,7 +97,6 @@ struct Params {
   const float* x_amax;  // [n_amax] upper bounds of max|x| (their maximum is used)
   const float* w_inv;   // 1 / weight scale (tail of the packed buffer)
   float* y_amax;        // null or: atomically raised to max|y|
-  float rz_kappa;       // first-order compensation of the accumulator's round-toward-zero bias, per MMA of a part
   const float* a_gate;  // null or: [N][Cin] factors multiplied into the input (the eSE gate of the producing stage, or the
                         // per-(image, channel) scale of a normalisation)
   const float* a_shift; // null or: [N][Cin] added after the factor, followed by ReLU if a_relu: x' = act(x * a_gate + a_shift)
@@ -551,10 +528,6 @@ __global__ void __launch_bounds__(kSmemA ? kThreadsS : kThreads, 1) conv_tc_kern
     const int ncol32 = P.ncol32, parts = P.parts;
     const float w_inv = __ldg(P.w_inv);
     float rescale = xs_inv * w_inv;   // undoes the two power-of-two operand scales (exact)
-    // The tensor core truncates its fp32 accumulator toward zero after every MMA: a part that accumulated n MMAs
-    // comes out smaller by ~kappa * n / 2 of its value in expectation (calibrated on the hardware, tools/rz_calib.py).
-    // Each part is scaled back by that factor before it is added; what remains is the unbiased part of the rounding.
-    const int mma_per_chunk = 6;
     float vmax = 0.f;                                // max |y| over the valid outputs this lane produced
     uint32_t gp = 0;
     for (int i = 0; in_range(i); ++i) {
@@ -595,8 +568,6 @@ __global__ void __launch_bounds__(kSmemA ? kThreadsS : kThreads, 1) conv_tc_kern
         mbar_wait(acc_full(as_), aph);
         tc_fence_after();
         const uint32_t trow = tmem_base + ((uint32_t)(qd * 32) << 16) + col_acc + as_ * acc_w;
-        const int part_chunks = min(P.chunks_per_part, P.chunks - part * P.chunks_per_part);
-        const float comp = 1.f + P.rz_kappa * 0.5f * (float)(part_chunks * mma_per_chunk);
         if (sp >= ncol32) {   // a group narrower than the epilogue's slab phases: nothing to read
           __syncwarp();
           if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * as_);
@@ -619,8 +590,8 @@ __global__ void __launch_bounds__(kSmemA ? kThreadsS : kThreads, 1) conv_tc_kern
 #pragma unroll
             for (int c4 = 0; c4 < 8; ++c4) {
               const uint32_t sa = slab + (uint32_t)((c4 ^ (m & 7)) << 4);
-              float4 x = make_float4(__uint_as_float(v[c4 * 4 + 0]) * comp, __uint_as_float(v[c4 * 4 + 1]) * comp,
-                                     __uint_as_float(v[c4 * 4 + 2]) * comp, __uint_as_float(v[c4 * 4 + 3]) * comp);
+              float4 x = make_float4(__uint_as_float(v[c4 * 4 + 0]), __uint_as_float(v[c4 * 4 + 1]), __uint_as_float(v[c4 * 4 + 2]),
+                                     __uint_as_float(v[c4 * 4 + 3]));
               if (part > 0) {
                 const float4 r = lds4s(sa);
                 x.x += r.x; x.y += r.y; x.z += r.z; x.w += r.w;
@@ -658,8 +629,8 @@ __global__ void __launch_bounds__(kSmemA ? kThreadsS : kThreads, 1) conv_tc_kern
 #pragma unroll
           for (int c4 = 0; c4 < 8; ++c4) {
             const uint32_t sa = slab + (uint32_t)((c4 ^ (m & 7)) << 4);
-            float4 x = make_float4(__uint_as_float(v[c4 * 4 + 0]) * comp, __uint_as_float(v[c4 * 4 + 1]) * comp,
-                                   __uint_as_float(v[c4 * 4 + 2]) * comp, __uint_as_float(v[c4 * 4 + 3]) * comp);
+            float4 x = make_float4(__uint_as_float(v[c4 * 4 + 0]), __uint_as_float(v[c4 * 4 + 1]), __uint_as_float(v[c4 * 4 + 2]),
+                                   __uint_as_float(v[c4 * 4 + 3]));
             if (part > 0) {
               const float4 r = lds4s(sa);
               x.x += r.x; x.y += r.y; x.z += r.z; x.w += r.w;
@@ -1021,25 +992,6 @@ __global__ void pack_weights_kernel(const float* __restrict__ w, int cout, int c
   }
 }
 
-int make_nhwc_map_strided(CUtensorMap* out, const float* base, int N, int H, int W, int C, long pixel_stride, int bc, int bw,
-                          int bh, int estride) {
-  PFN_encodeTiled enc = get_encode_tiled();
-  if (!enc) return FOD_ERR_CUDA;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)pixel_stride * 4, (cuuint64_t)W * pixel_stride * 4, (cuuint64_t)H * W * pixel_stride * 4};
-  cuuint32_t box[4] = {(cuuint32_t)bc, (cuuint32_t)bw, (cuuint32_t)bh, 1};
-  cuuint32_t estr[4] = {1, (cuuint32_t)estride, (cuuint32_t)estride, 1};
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed (%d) for map [%d,%d,%d,%d] pixel stride %ld box [%d,%d,%d]", (int)r, N, H, W, C,
-              pixel_stride, bc, bw, bh);
-    return FOD_ERR_CUDA;
-  }
-  return FOD_OK;
-}
-
 }  // namespace cvt
 }  // namespace fod
 
@@ -1148,13 +1100,7 @@ static int conv2d_nhwc_impl(const float* x, int n, int h, int w, int cin, long x
   prm.stride = stride;
   prm.cin_chunks = cin_pad / 32;
   prm.chunks = prm.taps * prm.cin_chunks;
-  // development knobs (tools/rz_calib.py): chunks per partial sum and the bias compensation per MMA
-  int part_chunks = cvt::kPartChunks;
-  float kappa = cvt::kRzKappa;
-  if (const char* e = getenv("FOD_CONV_PART_CHUNKS")) part_chunks = atoi(e) > 0 ? atoi(e) : part_chunks;
-  if (const char* e = getenv("FOD_CONV_RZ_KAPPA")) kappa = (float)atof(e);
-  prm.rz_kappa = kappa;
-  prm.parts = (prm.chunks + part_chunks - 1) / part_chunks;
+  prm.parts = (prm.chunks + cvt::kPartChunks - 1) / cvt::kPartChunks;
   prm.chunks_per_part = (prm.chunks + prm.parts - 1) / prm.parts;
   prm.parts = (prm.chunks + prm.chunks_per_part - 1) / prm.chunks_per_part;
   const int n16 = (cout + 15) / 16 * 16;
@@ -1223,10 +1169,13 @@ static int conv2d_nhwc_impl(const float* x, int n, int h, int w, int cin, long x
     smem_a = prm.b_stages >= 2;
   }
   int rc = smem_a && !per_tap
-               ? cvt::make_nhwc_map_strided(&prm.in_map, x, n, h, w, cin, x_pixel_stride, cvt::kChunk, cvt::kTileW, cvt::kTileH + 2, 1)
-               : cvt::make_nhwc_map_strided(&prm.in_map, x, n, h, w, cin, x_pixel_stride, cvt::kChunk, halo_w, halo_h, stride);
+               ? make_nhwc_map(&prm.in_map, x, n, h, w, cin, x_pixel_stride, cvt::kChunk, cvt::kTileW, cvt::kTileH + 2, 1,
+                               CU_TENSOR_MAP_SWIZZLE_128B)
+               : make_nhwc_map(&prm.in_map, x, n, h, w, cin, x_pixel_stride, cvt::kChunk, halo_w, halo_h, stride,
+                               CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc != FOD_OK) return rc;
-  rc = cvt::make_nhwc_map_strided(&prm.out_map, y, n, ho, wo, cout, y_pixel_stride, cvt::kChunk, cvt::kTileW, cvt::kTileH, 1);
+  rc = make_nhwc_map(&prm.out_map, y, n, ho, wo, cout, y_pixel_stride, cvt::kChunk, cvt::kTileW, cvt::kTileH, 1,
+                     CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc != FOD_OK) return rc;
   const long ktot = (long)prm.taps * cin_pad;
   const __half* whi = reinterpret_cast<const __half*>(packed);

@@ -50,13 +50,3 @@ extern "C" int fod_support_taps(const float* proto, int num_classes, int h, int 
   FOD_CUDA_LAUNCH_CHECK("fod_support_taps");
   return FOD_OK;
 }
-
-extern "C" int fod_correlate(const float* q, const float* taps, const float* w3, const float* b3, float* attn, int batch,
-                             int num_classes, int height, int width, fod_stream_t stream) {
-  // one level of fod_correlate_levels (correlate_tc.cu)
-  fod_level_t lv;
-  lv.height = height;
-  lv.width = width;
-  lv.stride = 0;
-  return fod_correlate_levels(&q, &taps, &lv, 1, w3, b3, &attn, nullptr, batch, num_classes, stream);
-}

@@ -530,9 +530,11 @@ extern "C" int fod_correlate_levels(const float* const* q, const float* const* t
     prm.attn_amax[l] = attn_amax ? attn_amax[l] : nullptr;
     FOD_REQUIRE((((uintptr_t)q[l] | (uintptr_t)attn[l]) & 15) == 0,
                 "fod_correlate_levels: level %d pointers must be 16-byte aligned", l);
-    int rc = make_nhwc_map(&prm.in_map[l], q[l], batch, H, W, kC, ctc::kChunk, ctc::kHaloW, ctc::kHaloH);
+    int rc = make_nhwc_map(&prm.in_map[l], q[l], batch, H, W, kC, kC, ctc::kChunk, ctc::kHaloW, ctc::kHaloH, 1,
+                           CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc != FOD_OK) return rc;
-    rc = make_nhwc_map(&prm.out_map[l], attn[l], batch * num_classes, H, W, kC, ctc::kChunk, ctc::kTileW, ctc::kTileH);
+    rc = make_nhwc_map(&prm.out_map[l], attn[l], batch * num_classes, H, W, kC, kC, ctc::kChunk, ctc::kTileW, ctc::kTileH, 1,
+                       CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc != FOD_OK) return rc;
   }
   prm.w3 = w3;

@@ -7,8 +7,8 @@
 //                          vovnet.py eSEModule; the gate is >= 0, so it commutes with the max), written straight into a
 //                          channel slice of the next stage's concat buffer.
 // One float4 (4 channels) per thread, coalesced 128-bit accesses; the 9-fold window overlap is served by L1/L2.
-#include <cuda_fp16.h>
 #include "common.cuh"
+#include "split_format.cuh"
 
 namespace fod {
 namespace glue {
@@ -387,17 +387,14 @@ __global__ void __launch_bounds__(kThreads) maxpool_kernel(const float* __restri
   }
   float* out = y + ((n * Ho + oy) * (size_t)Wo + ox) * ys;
   if (y_bound) {
-    // split hand-off format of the convolutions that read this map (conv_tc.cu): per 16 channels 64 bytes =
-    // [16 x fp16 hi | 16 x fp16 lo] of y * 2^e, 2^e = pow2_scale(y_bound[n]) - the consumer derives the same scale
-    const uint32_t E = (__float_as_uint(__ldg(y_bound + n)) >> 23) & 0xFFu;
-    const float sc = (E < 32u || E > 240u) ? 1.f : __uint_as_float((267u - E) << 23);
-    const __half2 h0 = __floats2half2_rn(m.x * sc, m.y * sc), h1 = __floats2half2_rn(m.z * sc, m.w * sc);
-    const float2 f0 = __half22float2(h0), f1 = __half22float2(h1);
-    const __half2 l0 = __floats2half2_rn(m.x * sc - f0.x, m.y * sc - f0.y), l1 = __floats2half2_rn(m.z * sc - f1.x, m.w * sc - f1.y);
-    const int ch = c4 * 4, grp = ch >> 4, q = ch & 15;       // 4 channels = 8 bytes of hi and 8 bytes of lo inside the group
+    // the split operand format of the convolutions that read this map (split_format.cuh), 2^e = pow2_scale(y_bound[n]):
+    // the consumer derives the same scale
+    float sc, unused;
+    pow2_scale(__ldg(y_bound + n), sc, unused);
     uint2 hv, lv;
-    hv.x = *reinterpret_cast<const uint32_t*>(&h0); hv.y = *reinterpret_cast<const uint32_t*>(&h1);
-    lv.x = *reinterpret_cast<const uint32_t*>(&l0); lv.y = *reinterpret_cast<const uint32_t*>(&l1);
+    split_f16x2(m.x * sc, m.y * sc, hv.x, lv.x);
+    split_f16x2(m.z * sc, m.w * sc, hv.y, lv.y);
+    const int ch = c4 * 4, grp = ch >> 4, q = ch & 15;       // 4 channels = 8 bytes of hi and 8 bytes of lo inside the group
     uint8_t* gb = reinterpret_cast<uint8_t*>(out) + grp * 64;
     *reinterpret_cast<uint2*>(gb + q * 2) = hv;
     *reinterpret_cast<uint2*>(gb + 32 + q * 2) = lv;

@@ -19,6 +19,7 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "split_format.cuh"
 #include "tc05.cuh"
 
 namespace fod {
@@ -100,15 +101,6 @@ struct Params {
   int num_problems, classes, roi_cap, tiles_per_problem, total_slots, num_pairs;
 };
 
-// (a, b) -> packed fp16 pair of the rounded values (a in the low half) and of the exact remainders
-__device__ __forceinline__ void split_f16x2(float a, float b, uint32_t& hi, uint32_t& lo) {
-  const __half2 h = __floats2half2_rn(a, b);
-  const float2 hf = __half22float2(h);
-  const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-  hi = *reinterpret_cast<const uint32_t*>(&h);
-  lo = *reinterpret_cast<const uint32_t*>(&l);
-}
-
 struct Slot {
   int p, r0, rows;  // rows = valid ROI rows in this unit (0 = padding unit of the last pair)
 };
@@ -147,13 +139,7 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
     const float* col = P.x_amax + (P.amax_stride ? img : 0);
     const int step = P.amax_stride ? P.amax_stride : 1;
     for (int i = 0; i < P.n_amax; ++i) amax = fmaxf(amax, __ldg(col + (size_t)i * step));
-    const int E = (int)((__float_as_uint(amax) >> 23) & 0xFF);
-    xs = 1.f;
-    xs_inv = 1.f;
-    if (E >= 32 && E <= 240) {     // amax * 2^e in [2^13, 2^14); 1 for zero / denormal-range / non-finite bounds
-      xs = __uint_as_float((uint32_t)(267 - E) << 23);
-      xs_inv = __uint_as_float((uint32_t)(E - 13) << 23);
-    }
+    pow2_scale(amax, xs, xs_inv);
   };
   image_scale(0);
 
@@ -467,30 +453,10 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
   if (warp == kWarpAlloc) tmem_dealloc<2>(tmem_base, kTmemCols);
 }
 
-// x -> (tf32-rounded hi, exact remainder lo): the B operand planes of the 3xTF32 scheme
-__global__ void split_tf32_kernel(const float* __restrict__ src, float* __restrict__ hi, float* __restrict__ lo, size_t n) {
-  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) {
-    float x = src[i];
-    uint32_t h;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(x));
-    hi[i] = __uint_as_float(h);
-    lo[i] = x - __uint_as_float(h);
-  }
-}
-
 }  // namespace rtc
 }  // namespace fod
 
 using namespace fod;
-
-extern "C" int fod_split_tf32(const float* src, float* hi_lo, size_t n, fod_stream_t stream) {
-  FOD_REQUIRE(src && hi_lo, "fod_split_tf32: null pointer");
-  if (n == 0) return FOD_OK;
-  rtc::split_tf32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, as_stream(stream)>>>(src, hi_lo, hi_lo + n, n);
-  FOD_CUDA_LAUNCH_CHECK("fod_split_tf32");
-  return FOD_OK;
-}
 
 extern "C" int fod_relation_head(const float* pooled, const float* x_amax, int n_amax, int amax_per_image,
                                  const float* w_fold_packed,

@@ -751,7 +751,8 @@ static int roi_align_impl(const float* const* feat, const fod_level_t* levels, i
     rt::Params tp;
     int total = 0;
     for (int l = 0; l < num_levels; ++l) {
-      const int rc = make_nhwc_map_plain(&tp.map[l], feat[l], batch, prm.H[l], prm.W[l], kC, kC, rt::kEdge, rt::kEdge);
+      const int rc = make_nhwc_map(&tp.map[l], feat[l], batch, prm.H[l], prm.W[l], kC, kC, kC, rt::kEdge, rt::kEdge, 1,
+                                   CU_TENSOR_MAP_SWIZZLE_NONE);
       if (rc != FOD_OK) return rc;
       tp.feat[l] = feat[l];
       tp.H[l] = prm.H[l];

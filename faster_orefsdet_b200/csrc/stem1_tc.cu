@@ -20,14 +20,10 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "split_format.cuh"
 #include "tc05.cuh"
 
 namespace fod {
-
-namespace cvt {   // conv_tc.cu
-int make_nhwc_map_strided(CUtensorMap* out, const float* base, int N, int H, int W, int C, long pixel_stride, int bc, int bw,
-                          int bh, int estride);
-}
 
 using namespace tc;
 
@@ -71,21 +67,6 @@ struct Params {
   float mean[3], std[3];
   float xs, xs_inv;      // operand scale 2^e of the normalised pixels and its inverse
 };
-
-// (a, b) -> packed fp16 pair of the rounded values (a in the low half) and of the exact remainders
-// conv_tc.cu's pow2_scale: 2^e with amax * 2^e in [2^13, 2^14); the consumer derives the same scale from the same bound
-__device__ __forceinline__ float pow2_scale_of(float amax) {
-  const int E = (int)((__float_as_uint(amax) >> 23) & 0xFF);
-  return (E < 32 || E > 240) ? 1.f : __uint_as_float((uint32_t)(267 - E) << 23);
-}
-
-__device__ __forceinline__ void split_f16x2(float a, float b, uint32_t& hi, uint32_t& lo) {
-  const __half2 h = __floats2half2_rn(a, b);
-  const float2 hf = __half22float2(h);
-  const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-  hi = *reinterpret_cast<const uint32_t*>(&h);
-  lo = *reinterpret_cast<const uint32_t*>(&l);
-}
 
 // Tile coordinates of a CTA's static schedule t = blockIdx.x, + gridDim.x, ...: carried along with additions and two
 // compares instead of two integer divisions per tile and warp (every role walks the same sequence).
@@ -276,7 +257,8 @@ __global__ void __launch_bounds__(kThreads, 1) stem1_tc_kernel(const __grid_cons
     const uint32_t box0 = sbase + kOffStage + (uint32_t)ew * 2u * kBoxBytes;            // this warp's two staging boxes
     const uint32_t row0 = box0 + (uint32_t)((lane >> 3) * 1024 + (lane & 7) * 128);   // this lane's pixel row
     const float rescale = P.xs_inv * __ldg(P.w_inv);   // undoes the two power-of-two operand scales (exact)
-    const float ysplit = P.y_bound ? pow2_scale_of(__ldg(P.y_bound)) : 0.f;
+    float ysplit = 0.f, unused;   // != 0: the output leaves as fp16 hi / lo of y * ysplit
+    if (P.y_bound) pow2_scale(__ldg(P.y_bound), ysplit, unused);
     float bias[32];
 #pragma unroll
     for (int j = 0; j < 32; ++j) bias[j] = P.bias ? __ldg(P.bias + half * 32 + j) : 0.f;
@@ -314,7 +296,7 @@ __global__ void __launch_bounds__(kThreads, 1) stem1_tc_kernel(const __grid_cons
       const uint32_t row_s = row0 + (uint32_t)(i & 1) * kBoxBytes;
       float lmax = 0.f;
       if (ysplit != 0.f) {
-        // the split hand-off format (conv_tc.cu): per 16 channels 64 bytes = [16 x fp16 hi | 16 x the exact remainders]
+        // the split operand format (split_format.cuh): per 16 channels 64 bytes = [16 x fp16 hi | 16 x the exact remainders]
         // of y * 2^e
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
@@ -410,7 +392,8 @@ static int stem1_u8_tc_impl(const uint8_t* x, int n, int h, int w, const float* 
   const long tiles = (long)n * prm.tiles_per_img;
   FOD_REQUIRE(tiles < (1L << 30), "fod_stem1_u8_tc: too many tiles");
   prm.tiles_total = (int)tiles;
-  int rc = cvt::make_nhwc_map_strided(&prm.out_map, y, n, prm.ho, prm.wo, s1tc::kCout, y_pixel_stride, 32, s1tc::kTileW, 2, 1);
+  int rc = make_nhwc_map(&prm.out_map, y, n, prm.ho, prm.wo, s1tc::kCout, y_pixel_stride, 32, s1tc::kTileW, 2, 1,
+                         CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc != FOD_OK) return rc;
   const __half* whi = reinterpret_cast<const __half*>(packed);
   rc = make_matrix_map_f16(&prm.whi_map, whi, s1tc::kCout, s1tc::kK, s1tc::kK, s1tc::kCout);

@@ -380,11 +380,12 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 PFN_encodeTiled get_encode_tiled();
 
-// fp32 NHWC map [N][H][W][C] -> 4-D tensor map (dims innermost first: C, W, H, N), box (bc, bw, bh, 1),
-// 128-byte swizzle (bc * 4 must be 128), out-of-bounds elements read as zero / are not written.
-int make_nhwc_map(CUtensorMap* out, const float* base, int N, int H, int W, int C, int bc, int bw, int bh);
-// the same without a swizzle: the box lands in shared memory as a dense [bh][bw][bc] array (bc * 4 a multiple of 16)
-int make_nhwc_map_plain(CUtensorMap* out, const float* base, int N, int H, int W, int C, int bc, int bw, int bh);
+// fp32 NHWC map [N][H][W][C] whose pixels lie pixel_stride floats apart (>= C: a channel slice of a wider map) -> 4-D
+// tensor map (dims innermost first: C, W, H, N), box (bc, bw, bh, 1), element strides (1, estride, estride, 1);
+// out-of-bounds elements read as zero / are not written.  CU_TENSOR_MAP_SWIZZLE_128B needs bc * 4 == 128; with
+// CU_TENSOR_MAP_SWIZZLE_NONE the box lands in shared memory as a dense [bh][bw][bc] array (bc * 4 a multiple of 16).
+int make_nhwc_map(CUtensorMap* out, const float* base, int N, int H, int W, int C, long pixel_stride, int bc, int bw, int bh,
+                  int estride, CUtensorMapSwizzle swizzle);
 // fp32 row-major matrix [rows][cols] -> 2-D tensor map, box (box_cols, box_rows), 128-byte swizzle
 // (box_cols * 4 must be 128), rows beyond the matrix read as zero.
 int make_matrix_map(CUtensorMap* out, const float* base, long rows, long cols, int box_cols, int box_rows);

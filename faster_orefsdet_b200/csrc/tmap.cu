@@ -18,35 +18,19 @@ PFN_encodeTiled get_encode_tiled() {
   return fn;
 }
 
-int make_nhwc_map(CUtensorMap* out, const float* base, int N, int H, int W, int C, int bc, int bw, int bh) {
+int make_nhwc_map(CUtensorMap* out, const float* base, int N, int H, int W, int C, long pixel_stride, int bc, int bw, int bh,
+                  int estride, CUtensorMapSwizzle swizzle) {
   PFN_encodeTiled enc = get_encode_tiled();
   if (!enc) return FOD_ERR_CUDA;
   cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 4, (cuuint64_t)W * C * 4, (cuuint64_t)H * W * C * 4};
+  cuuint64_t strides[3] = {(cuuint64_t)pixel_stride * 4, (cuuint64_t)W * pixel_stride * 4, (cuuint64_t)H * W * pixel_stride * 4};
   cuuint32_t box[4] = {(cuuint32_t)bc, (cuuint32_t)bw, (cuuint32_t)bh, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
+  cuuint32_t estr[4] = {1, (cuuint32_t)estride, (cuuint32_t)estride, 1};
   CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed (%d) for map [%d,%d,%d,%d] box [%d,%d,%d]", (int)r, N, H, W, C, bc, bw, bh);
-    return FOD_ERR_CUDA;
-  }
-  return FOD_OK;
-}
-
-int make_nhwc_map_plain(CUtensorMap* out, const float* base, int N, int H, int W, int C, int bc, int bw, int bh) {
-  PFN_encodeTiled enc = get_encode_tiled();
-  if (!enc) return FOD_ERR_CUDA;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 4, (cuuint64_t)W * C * 4, (cuuint64_t)H * W * C * 4};
-  cuuint32_t box[4] = {(cuuint32_t)bc, (cuuint32_t)bw, (cuuint32_t)bh, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed (%d) for plain map [%d,%d,%d,%d] box [%d,%d,%d]", (int)r, N, H, W, C, bc, bw, bh);
+    set_error("cuTensorMapEncodeTiled failed (%d) for map [%d,%d,%d,%d] pixel stride %ld box [%d,%d,%d] element stride %d", (int)r,
+              N, H, W, C, pixel_stride, bc, bw, bh, estride);
     return FOD_ERR_CUDA;
   }
   return FOD_OK;

@@ -166,8 +166,6 @@ class _OSAModule(nn.Module):
             src, off = dst, off + cw
         return buf, amax
 
-    SPLIT_HANDOFF = True      # 3x3 layers write their slices in the operand format of their readers (fod_conv2d_nhwc_split)
-
     def _split_eligible(self) -> bool:
         """Whole 16-channel groups everywhere (the split format packs 16 channels into 64 bytes) and plain 3x3 layers."""
         convs = [layer[0] for layer in self.layers]
@@ -188,9 +186,9 @@ class _OSAModule(nn.Module):
         # the eSE average comes out of the concat convolution's epilogue as per-tile channel sums: no pass over y
         colsum = torch.empty((n, ops.conv2d_tiles_per_image(h, w), cout), dtype=torch.float32, device=buf.device)
         nl = len(self.layers)
-        if in_presplit and not (self.SPLIT_HANDOFF and self._split_eligible()):
+        if in_presplit and not self._split_eligible():
             raise RuntimeError("a pre-split first slice needs the split hand-off of this module")
-        if self.SPLIT_HANDOFF and self._split_eligible():
+        if self._split_eligible():
             # Split hand-off: every 3x3 layer writes its slice in the operand format of its readers (fp16 hi / lo of
             # y * 2^e, e from the bound l1 * max|x| + beta that it publishes into amax[i + 1]); the next 3x3 layer reads it
             # without its conversion pass, the concat convolution rescales each slice to its common scale by a power of
@@ -294,9 +292,6 @@ class VoVNet(Backbone):     # detectron2's build_backbone asserts isinstance(bac
             self._stem1_folded_cache = hit
         return hit[1], hit[2]
 
-    STEM1_TENSOR_CORES = True     # stem_1 of uint8 input: csrc/stem1_tc.cu (False: the FP32 FMA kernel, ops.stem1_u8)
-    STEM1_SPLIT_OUTPUT = True     # ... writing stem_2's operand format (fod_stem1_u8_tc_split) instead of fp32
-
     def _stem1_bound(self, mean, std):
         """One device float >= every output of stem_1 (ReLU of the folded convolution) for ANY uint8 image: the absolute
         row sums of the folded weight times the largest normalised pixel magnitude per colour plane, plus |bias|."""
@@ -324,16 +319,14 @@ class VoVNet(Backbone):     # detectron2's build_backbone asserts isinstance(bac
 
     def stem_u8_writes_split(self) -> bool:
         """tc_stem_u8 leaves its output (the first slice of the stage-2 concat buffer) in the split operand format."""
-        return (self.STEM1_TENSOR_CORES and self.STEM1_SPLIT_OUTPUT and self.STEM3_SPLIT_OUTPUT and "stem" not in self._out_features
-                and self.stem[0].out_channels == 64 and tuple(self.stem[0].weight.shape[1:]) == (3, 3, 3)
-                and self.stem[6].out_channels % 16 == 0 and self._tc_modules()[0].SPLIT_HANDOFF and self._tc_modules()[0]._split_eligible())
-
-    POOL_SPLIT_OUTPUT = True      # the stage poolings write the next stage's first slice in the split format
-    STEM3_SPLIT_OUTPUT = True     # stem_3 writes the operand format of the first OSA layer and of the concat convolution
+        return ("stem" not in self._out_features and self.stem[0].out_channels == 64
+                and tuple(self.stem[0].weight.shape[1:]) == (3, 3, 3) and self.stem[6].out_channels % 16 == 0
+                and self._tc_modules()[0]._split_eligible())
 
     def tc_stem_u8(self, x_u8, mean, std, out, out_amax, out_act=None, scratch=None):
         """Raw uint8 images -> stem_1 (normalisation fused; tensor-core kernel ops.stem1_u8_tc, the im2col gathered into
-        tensor memory) -> stem_2 -> stem_3 into ``out``; same contract as tc_stem."""
+        tensor memory) -> stem_2 -> stem_3 into ``out``; same contract as tc_stem.  With ``out_act`` (when
+        stem_u8_writes_split()) ``out`` is left in the split operand format of the first OSA module."""
         if self.stem[0].out_channels != 64 or tuple(self.stem[0].weight.shape[1:]) != (3, 3, 3):
             return self.tc_stem(ops.stem_patches_u8(x_u8, mean, std), None, out, out_amax)
         n = x_u8.shape[0]
@@ -341,39 +334,29 @@ class VoVNet(Backbone):     # detectron2's build_backbone asserts isinstance(bac
             a1, a2 = scratch[0], scratch[1]
         else:
             a1, a2 = ops.new_amax(x_u8.device, n), ops.new_amax(x_u8.device, n)          # per image
-        if self.STEM1_TENSOR_CORES and self.STEM1_SPLIT_OUTPUT:
-            # stem_1 writes the operand format of stem_2 (fp16 hi / lo of y * 2^e) instead of fp32: its output bound follows
-            # from the weights and the pixel range alone, so the scale is known before the layer runs and stem_2 skips
-            # the conversion pass of every staged tile
-            pk, b = self._stem1_packed()
-            bound = self._stem1_bound(mean, std)
-            if out_act is None:
-                y = ops.stem1_u8_tc(x_u8, mean, std, pk, b, y_bound=bound)
-            if out_act is not None:     # split hand-off all the way: stem_2 -> stem_3 -> the first OSA module
-                y = ops.stem1_u8_tc(x_u8, mean, std, pk, b, y_amax=a1, y_bound=bound)
-                pk2, b2, c2 = tcconv.packed(self.stem[3], self.stem[4])
-                l1, beta = tcconv.bound_consts(self.stem[3], self.stem[4])
-                b2nd = torch.empty((n,), dtype=torch.float32, device=x_u8.device)          # stem_2's published bound, per image (a plain store)
-                y2 = torch.empty((n, y.shape[2], y.shape[3], c2), dtype=torch.float32, device=y.device).permute(0, 3, 1, 2)
-                ops.conv2d_nhwc_split(y, pk2, b2, c2, 3, y2, self._stem1_bound_rows(mean, std, n),
-                                      y_amax=a2, x_presplit=True, x_actual=a1, y_bound=b2nd, y_l1=l1, y_beta=beta)
-                pk3, b3, c3 = tcconv.packed(self.stem[6], self.stem[7])
-                l1, beta = tcconv.bound_consts(self.stem[6], self.stem[7])
-                # out_amax receives stem_3's bound, out_act its max(y)
-                ops.conv2d_nhwc_split(y2, pk3, b3, c3, 3, out, b2nd.view(1, n), y_amax=out_act, x_actual=a2, y_bound=out_amax,
-                                      y_l1=l1, y_beta=beta, x_presplit_from=0, slice_ch=[0], stride=2)
-                return
+        # stem_1 writes the operand format of stem_2 (fp16 hi / lo of y * 2^e) instead of fp32: its output bound follows
+        # from the weights and the pixel range alone, so the scale is known before the layer runs and stem_2 skips
+        # the conversion pass of every staged tile
+        pk, b = self._stem1_packed()
+        bound = self._stem1_bound(mean, std)
+        if out_act is None:
+            y = ops.stem1_u8_tc(x_u8, mean, std, pk, b, y_bound=bound)
             y = tcconv.conv(y, self.stem[3], self.stem[4], relu=True, x_amax=bound, y_amax=a2, x_presplit=True)
             tcconv.conv(y, self.stem[6], self.stem[7], relu=True, out=out, x_amax=a2.view(1, n), y_amax=out_amax)
             return
-        if self.STEM1_TENSOR_CORES:
-            pk, b = self._stem1_packed()
-            y = ops.stem1_u8_tc(x_u8, mean, std, pk, b, y_amax=a1)
-        else:
-            w, b = self._stem1_folded()
-            y = ops.stem1_u8(x_u8, mean, std, w, b, y_amax=a1)
-        y = tcconv.conv(y, self.stem[3], self.stem[4], relu=True, x_amax=a1.view(1, n), y_amax=a2)
-        tcconv.conv(y, self.stem[6], self.stem[7], relu=True, out=out, x_amax=a2.view(1, n), y_amax=out_amax)
+        # split hand-off all the way: stem_2 -> stem_3 -> the first OSA module
+        y = ops.stem1_u8_tc(x_u8, mean, std, pk, b, y_amax=a1, y_bound=bound)
+        pk2, b2, c2 = tcconv.packed(self.stem[3], self.stem[4])
+        l1, beta = tcconv.bound_consts(self.stem[3], self.stem[4])
+        b2nd = torch.empty((n,), dtype=torch.float32, device=x_u8.device)          # stem_2's published bound, per image (a plain store)
+        y2 = torch.empty((n, y.shape[2], y.shape[3], c2), dtype=torch.float32, device=y.device).permute(0, 3, 1, 2)
+        ops.conv2d_nhwc_split(y, pk2, b2, c2, 3, y2, self._stem1_bound_rows(mean, std, n),
+                              y_amax=a2, x_presplit=True, x_actual=a1, y_bound=b2nd, y_l1=l1, y_beta=beta)
+        pk3, b3, c3 = tcconv.packed(self.stem[6], self.stem[7])
+        l1, beta = tcconv.bound_consts(self.stem[6], self.stem[7])
+        # out_amax receives stem_3's bound, out_act its max(y)
+        ops.conv2d_nhwc_split(y2, pk3, b3, c3, 3, out, b2nd.view(1, n), y_amax=out_act, x_actual=a2, y_bound=out_amax,
+                              y_l1=l1, y_beta=beta, x_presplit_from=0, slice_ch=[0], stride=2)
 
     def tc_stem(self, patches, patches_amax, out, out_amax):
         """stem_1 (as a 1x1 convolution over im2col rows) -> stem_2 -> stem_3 into ``out`` (a batch slice of the first
@@ -413,7 +396,7 @@ class VoVNet(Backbone):     # detectron2's build_backbone asserts isinstance(bac
                 buf, first, amax = mods[i + 1].new_buffer(n, h, w, y.device)
                 # the pooling hands the next stage its first slice in the split format when that stage reads it that way:
                 # the bound is the actual maximum of the pooled map's source (the gate is <= 1)
-                in_presplit = self.POOL_SPLIT_OUTPUT and mods[i + 1].SPLIT_HANDOFF and mods[i + 1]._split_eligible() and a_y.numel() == n
+                in_presplit = mods[i + 1]._split_eligible() and a_y.numel() == n
                 ops.maxpool3x3s2_nhwc(y, gate, out=first, y_bound=a_y if in_presplit else None)
                 amax[0].copy_(a_y)
         if fuse_gates:

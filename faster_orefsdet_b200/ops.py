@@ -329,15 +329,6 @@ def roi_align(feats: Sequence[Tensor], strides: Sequence[int], rois: Tensor, roi
 
 
 # --------------------------------------------------------------------------- R2+R3
-def split_tf32(w: Tensor) -> Tensor:
-    """fp32 tensor -> [2, *w.shape]: plane 0 = tf32-rounded value, plane 1 = exact remainder (the B operand planes
-    of the 3xTF32 tensor-core contraction; done once per weight load)."""
-    w = _chk(w, torch.float32, "w").contiguous()
-    out = torch.empty((2,) + tuple(w.shape), dtype=torch.float32, device=w.device)
-    _lib.check(_lib.lib().fod_split_tf32(_ptr(w), _ptr(out), ctypes.c_size_t(w.numel()), _stream()), "fod_split_tf32")
-    return out
-
-
 def relation_pack(w_fold: Tensor) -> Tensor:
     """Folded relation matrix [128, 8192] -> the packed operand of relation_head: scaled fp16 hi / lo planes + the scale
     (fod_conv2d_pack_weights of the matrix seen as a 1x1 convolution weight; once per weight load)."""

@@ -74,28 +74,19 @@ typedef struct {
 int fod_support_taps(const float* proto, int num_classes, int h, int w, float* taps, fod_stream_t stream);
 
 /* ---------------------------------------------------------------------------
- * Q2+Q3  depthwise correlation + 1x1 relation conv on one FPN level, fused.
+ * Q2+Q3  depthwise correlation + 1x1 relation conv, fused, for ALL FPN levels and all (image, class) problems in one
+ * persistent launch (tcgen05 tensor cores, 3xTF32 operand splitting = fp32 accuracy, TMA in/out).
  * Replaces fsod_cen.py:463-470 (p3), :482-491 (p4), :502-509 (p5): four depthwise
  * F.conv2d + ReLUs + adds + torch.cat + self.conv3 + ReLU.
- *   q     : [B][H][W][128]            query map of this level
- *   taps  : [C][7][128]  HOST memory  from fod_support_taps, copied to the host once per episode (see below)
- *   w3    : [128][256]                conv3.weight (out, in) ; in = [attn-sum | q]
- *   b3    : [128]
- *   attn  : [B*C][H][W][128]          problem-major output
- */
-int fod_correlate(const float* q, const float* taps, const float* w3, const float* b3, float* attn, int batch,
-                  int num_classes, int height, int width, fod_stream_t stream);
-
-/* Q2+Q3 for ALL FPN levels and all (image, class) problems in one persistent launch
- * (tcgen05 tensor cores, 3xTF32 operand splitting = fp32 accuracy, TMA in/out).
- * Same arithmetic contract as fod_correlate.  q and attn are HOST arrays of
- * num_levels DEVICE pointers; taps is a HOST array of num_levels HOST pointers:
- *   q[l]    : [B][H_l][W_l][128]
+ * q and attn are HOST arrays of num_levels DEVICE pointers; taps is a HOST array of num_levels HOST pointers:
+ *   q[l]    : [B][H_l][W_l][128]      query map of level l
  *   taps[l] : [C][7][128]  HOST        the output of fod_support_taps on the level-l prototype, read back once per
  *                                      episode.  The taps are warp-uniform operands of the stencil: they are copied
  *                                      into the launch parameters (constant bank 0, 6 sets = 24 KB per launch; classes
  *                                      are processed in groups of 6 / num_levels), so no device state outlives or is
  *                                      shared between calls, and a captured graph bakes in the episode's taps.
+ *   w3      : [128][256]               conv3.weight (out, in) ; in = [attn-sum | q]
+ *   b3      : [128]
  *   attn[l] : [B*C][H_l][W_l][128]     problem-major output
  *   attn_amax : NULL, or per level NULL / B*C DEVICE floats (zeroed by the caller): entry p is raised to max(attn[l] of
  *               problem p) - the per-image operand bound of the convolution that consumes the maps (fod_conv2d_nhwc
@@ -232,7 +223,6 @@ int fod_roi_align_per_roi(const float* const* feat, const fod_level_t* levels, i
  *   logits/deltas (optional, may be NULL): [P][roi_cap][2] / [P][roi_cap][4]
  * At most 2047 problems per call.
  */
-int fod_split_tf32(const float* src, float* hi_lo /* [2][n] */, size_t n, fod_stream_t stream);
 int fod_relation_head(const float* pooled, const float* x_amax, int n_amax, int amax_per_image, const float* w_fold_packed,
                       const float* bias_cls, const float* w_out, const float* b_out, const float* rois,
                       const int32_t* roi_count, int num_problems, int problems_per_image, int roi_cap,

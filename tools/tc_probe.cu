@@ -275,7 +275,8 @@ static int run_tma() {
   CK(cudaMemcpy(dI, in.data(), in.size() * 4, cudaMemcpyHostToDevice));
   CK(cudaMemcpy(dO, out.data(), in.size() * 4, cudaMemcpyHostToDevice));
   CUtensorMap im, om;
-  if (make_nhwc_map(&im, dI, N, H, W, C, 32, 18, 10) || make_nhwc_map(&om, dO, N, H, W, C, 32, 16, 8)) {
+  if (make_nhwc_map(&im, dI, N, H, W, C, C, 32, 18, 10, 1, CU_TENSOR_MAP_SWIZZLE_128B) ||
+      make_nhwc_map(&om, dO, N, H, W, C, C, 32, 16, 8, 1, CU_TENSOR_MAP_SWIZZLE_128B)) {
     char buf[256];
     fod_last_error(buf, sizeof buf);
     printf("tensor map: %s\n", buf);
