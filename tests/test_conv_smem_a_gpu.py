@@ -7,26 +7,11 @@ import pytest
 import torch
 
 from faster_orefsdet_b200 import ops
+from tests.util import amax_per_image, presplit
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 MAGS = [1e-3, 30.0, 0.7]   # per-image magnitudes: every image gets its own scale
-
-
-def _amax(x):
-    return ops.absmax(x.contiguous(memory_format=torch.channels_last), per_image=True).reshape(1, -1)
-
-
-def _presplit(x, amax):
-    """fp32 NHWC view [N,C,H,W] -> the split operand format at the scale of amax ([1, N]), as an fp32 NHWC view."""
-    n, c, h, w = x.shape
-    _, ex = torch.frexp(amax.reshape(-1))                                  # amax = m * 2^ex, m in [0.5, 1)
-    scale = ((141 - ex.to(torch.int32)) << 23).view(torch.float32)      # 2^(14 - ex): max|x| * 2^e in [2^13, 2^14)
-    xs = x.permute(0, 2, 3, 1) * scale.view(n, 1, 1, 1)
-    hi = xs.half()
-    lo = (xs - hi.float()).half()
-    packed = torch.cat([hi.reshape(n, h, w, c // 16, 16), lo.reshape(n, h, w, c // 16, 16)], dim=-1)
-    return packed.contiguous().view(torch.float32).reshape(n, h, w, c).permute(0, 3, 1, 2)
 
 
 def _layer(n, h, w, cin, cout, seed):
@@ -60,10 +45,10 @@ def _in_wide_buffer(x, lead, trail):
 ])
 def test_presplit_3x3_is_bit_identical_to_fp32_input(n, h, w, cin, cout):
     x, pk, b = _layer(n, h, w, cin, cout, 1000 + cin + cout)
-    amax = _amax(x)
+    amax = amax_per_image(x)
     ya_ref, ya = ops.new_amax(DEV, n), ops.new_amax(DEV, n)
     ref = ops.conv2d_nhwc(x, pk, b, cout, 3, True, x_amax=amax, y_amax=ya_ref)
-    xp = _in_wide_buffer(_presplit(x, amax), 16, 48)
+    xp = _in_wide_buffer(presplit(x, amax), 16, 48)
     y = ops.conv2d_nhwc(xp, pk, b, cout, 3, True, x_amax=amax, y_amax=ya, x_presplit=True)
     assert torch.equal(y, ref)
     assert torch.equal(ya, ya_ref)
@@ -73,9 +58,9 @@ def test_presplit_3x3_is_bit_identical_to_fp32_input(n, h, w, cin, cout):
 def test_presplit_3x3_split_output_is_bit_identical():
     n, h, w, cin, cout = 3, 37, 53, 64, 64
     x, pk, b = _layer(n, h, w, cin, cout, 7)
-    amax = _amax(x)
+    amax = amax_per_image(x)
     outs = []
-    for xin, pre in ((x, False), (_presplit(x, amax), True)):
+    for xin, pre in ((x, False), (presplit(x, amax), True)):
         y = torch.empty((n, h, w, cout), device=DEV).permute(0, 3, 1, 2)
         yb, ya = torch.empty((n,), device=DEV), ops.new_amax(DEV, n)
         ops.conv2d_nhwc_split(xin, pk, b, cout, 3, y, amax, y_amax=ya, x_presplit=pre, y_bound=yb, y_l1=2.5, y_beta=0.1)
@@ -89,10 +74,10 @@ def test_presplit_stride2_is_bit_identical_to_fp32_input(n, h, w, cout):
     """stem_3: stride 2 over an input pre-split at a single bound"""
     cin = 64
     x, pk, b = _layer(n, h, w, cin, cout, 300 + h + cout)
-    amax = _amax(x)
+    amax = amax_per_image(x)
     ho, wo = (h - 1) // 2 + 1, (w - 1) // 2 + 1
     outs = []
-    for xin, pre in ((x, -1), (_in_wide_buffer(_presplit(x, amax), 32, 16), 0)):
+    for xin, pre in ((x, -1), (_in_wide_buffer(presplit(x, amax), 32, 16), 0)):
         y = torch.empty((n, ho, wo, cout), device=DEV).permute(0, 3, 1, 2)
         ya = ops.new_amax(DEV, n)
         ops.conv2d_nhwc_split(xin, pk, b, cout, 3, y, amax, y_amax=ya, x_presplit_from=pre,
