@@ -39,8 +39,8 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "pair.cuh"
 #include "split_format.cuh"
-#include "tc05.cuh"
 
 namespace fod {
 
@@ -166,52 +166,16 @@ __device__ __forceinline__ Unit unit_of(const Params& P, int pair, uint32_t rank
 __device__ __forceinline__ bool ends_part(int pc, int lc, int chunks_per_part, int chunks) {
   return pc == chunks_per_part - 1 || lc == chunks - 1;
 }
-// Stage and phase parity of the g-th use of an n-stage ring; the next stage after s
-__device__ __forceinline__ uint32_t ring_stage(uint32_t g, uint32_t n) { return g % n; }
-__device__ __forceinline__ uint32_t ring_phase(uint32_t g, uint32_t n) { return (g / n) & 1u; }
-__device__ __forceinline__ uint32_t ring_next(uint32_t s, uint32_t n) { return s + 1 == n ? 0u : s + 1; }
-// Watcher -> MMA warp: the number of chunks whose operands are in place (an mbarrier wait costs ~200 cycles even on a
-// long-completed phase, so only the watcher waits on barriers).  The MMA warp polls converged; lane 0's load decides.
-__device__ __forceinline__ void flag_publish(uint32_t flag, uint32_t n) {
-  asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(flag), "r"(n) : "memory");
-}
-__device__ __forceinline__ void flag_wait(uint32_t flag, uint32_t& upto, uint32_t g) {
-  while (upto <= g) {
-    uint32_t v;
-    asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"(flag) : "memory");
-    upto = __shfl_sync(0xffffffffu, v, 0);
-  }
-}
-// Bound of max|x| that the input scale of image n comes from (any n in the batch-wide mode)
-__device__ __forceinline__ float image_bound(const Params& P, int n) {
-  float amax = 0.f;
-  const float* col = P.x_amax + (P.x_amax_stride ? n : 0);
-  const int step = P.x_amax_stride ? P.x_amax_stride : 1;
-  for (int i = 0; i < P.n_amax; ++i) amax = fmaxf(amax, __ldg(col + (size_t)i * step));
-  return amax;
-}
-// Both CTAs allocate the pair's tensor memory; barrier initialisation and allocation become visible to both
-__device__ __forceinline__ uint32_t pair_setup(const Params& P, uint8_t* tmem_ptr, int warp, int lane) {
-  if (warp == kWarpAlloc) {
-    tmem_alloc<2>(smem_u32(tmem_ptr), kTmemCols);
-    tmem_relinquish<2>();
-  }
-  if (warp == kWarpTma && lane == 0) {
-    tma_prefetch_desc(&P.in_map);
-    tma_prefetch_desc(&P.out_map);
-    tma_prefetch_desc(&P.whi_map);
-    tma_prefetch_desc(&P.wlo_map);
-  }
-  tc_fence_before();
-  cluster_sync();
-  tc_fence_after();
-  return *reinterpret_cast<volatile uint32_t*>(tmem_ptr);
-}
-__device__ __forceinline__ void pair_teardown(int warp, uint32_t tmem_base) {
-  __syncwarp();
-  tc_fence_before();
-  cluster_sync();
-  if (warp == kWarpAlloc) tmem_dealloc<2>(tmem_base, kTmemCols);
+// Both CTAs allocate the pair's tensor memory while the TMA warp prefetches the tensor maps
+__device__ __forceinline__ uint32_t conv_pair_setup(const Params& P, uint8_t* tmem_ptr, int warp, int lane) {
+  return pair_setup(tmem_ptr, warp, kWarpAlloc, kTmemCols, [&] {
+    if (warp == kWarpTma && lane == 0) {
+      tma_prefetch_desc(&P.in_map);
+      tma_prefetch_desc(&P.out_map);
+      tma_prefetch_desc(&P.whi_map);
+      tma_prefetch_desc(&P.wlo_map);
+    }
+  });
 }
 
 // TMA producer of the weights (lane 0): a B stage holds kTaps taps (one, or a tap row of three) of one 32-channel
@@ -267,7 +231,7 @@ __device__ __forceinline__ void epilogue(const Params& P, uint8_t* smem, uint32_
   uint32_t gp = 0;
   for (int i = 0; has_unit(P, pair, i); ++i) {
     const Unit u = unit_of(P, pair, rank, i);
-    const float x_bound = image_bound(P, u.n);
+    const float x_bound = image_bound(P.x_amax, P.n_amax, P.x_amax_stride, u.n);
     float xs, xs_inv;
     pow2_scale(x_bound, xs, xs_inv);
     const float rescale = xs_inv * w_inv;   // undoes the two power-of-two operand scales (exact)
@@ -294,21 +258,14 @@ __device__ __forceinline__ void epilogue(const Params& P, uint8_t* smem, uint32_
       mbar_wait(acc_full0 + 8u * as_, ring_phase(gp, kAccStages));
       tc_fence_after();
       const uint32_t trow = tmem_acc + ((uint32_t)(qd * 32) << 16) + as_ * 128u;
-      if (sp >= ncol32) {   // a group narrower than the epilogue's slab phases: nothing to read
-        __syncwarp();
-        if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * as_);
-      }
+      if (sp >= ncol32) acc_release(acc_empty_leader + 8u * as_, lane);   // a group narrower than the slab phases: nothing to read
       const bool final = part == parts - 1;
 #pragma unroll 1
       for (int j = sp; j < ncol32; j += sstep) {
         uint32_t v[32];
         tmem_ld32(trow + j * 32, v);
         tmem_wait_ld();
-        if (j + sstep >= ncol32) {  // this warp's columns of the accumulator are read: hand them back to the MMA warp
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * as_);
-        }
+        if (j + sstep >= ncol32) acc_release(acc_empty_leader + 8u * as_, lane);   // this warp's columns are read
         const uint32_t slab = row_s + (uint32_t)j * kSlabBytes;
         float4 xv[8];
 #pragma unroll
@@ -451,7 +408,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel_tmem(const __grid_
     *reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr + 8) = 0;
     fence_barrier_init();
   }
-  const uint32_t tmem_base = pair_setup(P, smem + kOffTmemPtr, warp, lane);
+  const uint32_t tmem_base = conv_pair_setup(P, smem + kOffTmemPtr, warp, lane);
 
   if (warp == kWarpTma) {
     // ------------------------------------------------------------------ TMA producer: input tile + halo, per 32 channels
@@ -628,7 +585,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel_tmem(const __grid_
 
     for (int i = 0; has_unit(P, pair, i); ++i) {
       const Unit u = unit_of(P, pair, rank, i);
-      pow2_scale(image_bound(P, u.n), xs, xs_inv);
+      pow2_scale(image_bound(P.x_amax, P.n_amax, P.x_amax_stride, u.n), xs, xs_inv);
       in_y0 = u.ty * kTileH * P.stride - (ksz >> 1);
       in_x0 = u.tx * kTileW * P.stride - (ksz >> 1);
       for (int cc = 0; cc < P.cin_chunks; ++cc) {
@@ -732,7 +689,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel_tmem(const __grid_
       }
     }
   }
-  pair_teardown(warp, tmem_base);
+  pair_teardown(warp, kWarpAlloc, tmem_base, kTmemCols);
 }
 
 // ---------------------------------------------------------------------------------------------- shared-memory A pipeline
@@ -788,7 +745,7 @@ __global__ void __launch_bounds__(kThreadsS, 1) conv_tc_kernel_smem(const __grid
     *reinterpret_cast<volatile uint32_t*>(smem + off_tmem_ptr + 8) = 0;
     fence_barrier_init();
   }
-  const uint32_t tmem_base = pair_setup(P, smem + off_tmem_ptr, warp, lane);
+  const uint32_t tmem_base = conv_pair_setup(P, smem + off_tmem_ptr, warp, lane);
 
   const bool per_row_a = P.per_tap != 0;
   const uint32_t a_stage_bytes = 3 * L.a_box_bytes;
@@ -898,7 +855,7 @@ __global__ void __launch_bounds__(kThreadsS, 1) conv_tc_kernel_smem(const __grid
   } else {
     epilogue<kEpiWarpsS>(P, smem, L.off_sum, off_bias, acc_full(0), acc_empty(0), tmem_base + kColAcc, warp, lane, pair, rank);
   }
-  pair_teardown(warp, tmem_base);
+  pair_teardown(warp, kWarpAlloc, tmem_base, kTmemCols);
 }
 
 // max |x| of a dense fp32 array into *out (non-negative floats order like their bit patterns); *out must start at 0.
@@ -1173,33 +1130,12 @@ static int conv2d_nhwc_impl(const float* x, int n, int h, int w, int cin, long x
   rc = make_matrix_map_f16(&prm.wlo_map, whi + (size_t)cout * ktot, cout, ktot, cvt::kChunk, prm.nhalf);
   if (rc != FOD_OK) return rc;
   prm.w_inv = packed + (size_t)cout * ktot;   // tail[0] = 1 / weight scale
-  int dev = 0, sms = 0;
-  FOD_CUDA_CALL(cudaGetDevice(&dev));
-  FOD_CUDA_CALL(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const int max_pairs = sms / 2 > 0 ? sms / 2 : 1;
-  prm.num_pairs = prm.pair_units < max_pairs ? prm.pair_units : max_pairs;
+  rc = pair_count(prm.pair_units, &prm.num_pairs);
+  if (rc != FOD_OK) return rc;
   const void* kernel = smem_a ? (const void*)cvt::conv_tc_kernel_smem : (const void*)cvt::conv_tc_kernel_tmem;
   void* args[] = {&prm, smem_a ? (void*)&sm : (void*)&tm};
   const uint32_t smem_bytes = smem_a ? sm.off_sum + cvt::smem_a_tail_bytes(prm.ncol32) + 1024 : cvt::kSmemAlloc;
-  FOD_CUDA_CALL(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * prm.num_pairs);
-  cfg.blockDim = dim3(smem_a ? cvt::kThreadsS : cvt::kThreads);
-  cfg.dynamicSmemBytes = smem_bytes;
-  cfg.stream = as_stream(stream);
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelExC(&cfg, kernel, args);
-  if (e != cudaSuccess) {
-    set_error("fod_conv2d_nhwc: launch failed: %s", cudaGetErrorString(e));
-    return FOD_ERR_CUDA;
-  }
-  return FOD_OK;
+  return launch_pairs(kernel, args, prm.num_pairs, smem_a ? cvt::kThreadsS : cvt::kThreads, smem_bytes, stream, "fod_conv2d_nhwc");
 }
 
 extern "C" int fod_conv2d_nhwc(const float* x, int n, int h, int w, int cin, long x_pixel_stride, const float* x_amax,

@@ -26,8 +26,7 @@
 //   * 4 epilogue warps: tcgen05.ld -> + bias, ReLU -> swizzled staging tile -> TMA store (clipped at the image
 //     border by the tensor map).
 //   HBM traffic = read q once + write attn once = 1024 B per pixel per problem (SURVEY 8d).
-#include "common.cuh"
-#include "tc05.cuh"
+#include "pair.cuh"
 
 namespace fod {
 
@@ -194,10 +193,10 @@ __device__ __forceinline__ void stencil_role(const Params& P, const StencilCtx& 
         for (int sub = 0; sub < kNumSubs; ++sub) {  // uniform counter; this warp takes sub % 4 == myk
           if ((sub & 3) != myk) continue;
           const uint32_t gq = (uint32_t)i * kNumChunks + (sub >> 1);  // q box (32 channels) of this sub-chunk
-          const int qs = gq % kQStages, as_ = sub & 3;                // kNumSubs % kAStages == 0
-          const uint32_t qph = (gq / kQStages) & 1, aph = ((uint32_t)i * 2 + (sub >> 2)) & 1;
-          mbar_wait(bar0 + 8u * qs, qph);                                   // q_full
-          mbar_wait(bar0 + 8u * (2 * kQStages + kAStages + as_), aph ^ 1);  // a_empty
+          const uint32_t ga = (uint32_t)i * kNumSubs + sub;           // A stage use
+          const uint32_t qs = ring_stage(gq, kQStages), as_ = ring_stage(ga, kAStages);
+          mbar_wait(bar0 + 8u * qs, ring_phase(gq, kQStages));                                   // q_full
+          mbar_wait(bar0 + 8u * (2 * kQStages + kAStages + as_), ring_phase(ga, kAStages) ^ 1);  // a_empty
           tc_fence_after();
           const uint32_t qt = cx.sbase + kOffQ + qs * kQStageStride;  // shared-window address: LDS, not generic LD
           const uint32_t tcol = trow + as_ * kAStageCols;
@@ -311,18 +310,14 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
     *reinterpret_cast<volatile uint32_t*>(smem + kOffFlag) = 0;
     fence_barrier_init();
   }
-  if (warp == kWarpAlloc) {
-    tmem_alloc<2>(sbase + kOffTmemPtr, kTmemCols);
-    tmem_relinquish<2>();
-  }
-  if (warp == kWarpTma && lane == 0) {
-    for (int l = 0; l < P.num_levels; ++l) {
-      tma_prefetch_desc(&P.in_map[l]);
-      tma_prefetch_desc(&P.out_map[l]);
+  const uint32_t tmem_base = pair_setup(smem + kOffTmemPtr, warp, kWarpAlloc, kTmemCols, [&] {
+    if (warp == kWarpTma && lane == 0) {
+      for (int l = 0; l < P.num_levels; ++l) {
+        tma_prefetch_desc(&P.in_map[l]);
+        tma_prefetch_desc(&P.out_map[l]);
+      }
     }
-  }
-  // resident weights: this CTA's 64 rows of W3, split into tf32 hi / lo, K-major SW128 chunks
-  {
+    // resident weights: this CTA's 64 rows of W3, split into tf32 hi / lo, K-major SW128 chunks
     const float* wsrc = P.w3 + (size_t)rank * kBHalfRows * 256;
     for (int i = tid; i < (int)kBHalfRows * 64; i += kThreads) {  // float4 index: 64 per row
       int r = i >> 6, c = (i & 63) << 2;
@@ -341,12 +336,8 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
       *reinterpret_cast<uint4*>(smem + kOffBLo + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
     }
     if (tid < kC) reinterpret_cast<float*>(smem + kOffBias)[tid] = P.b3[tid];
-  }
-  fence_proxy_async_smem();
-  tc_fence_before();
-  cluster_sync();
-  tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr);
+    fence_proxy_async_smem();
+  });
 
   // static schedule: iteration i of pair k handles tiles 2*(i*num_pairs + k) + rank
   const int T = P.total_tiles;
@@ -362,9 +353,8 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
         TileCoord tcd = decode_tile(P, t);
         int b = tcd.b;
         for (int ch = 0; ch < kNumChunks; ++ch, ++g) {
-          int s = g % kQStages;
-          uint32_t ph = (g / kQStages) & 1;
-          mbar_wait(q_empty(s), ph ^ 1);
+          const uint32_t s = ring_stage(g, kQStages);
+          mbar_wait(q_empty(s), ring_phase(g, kQStages) ^ 1);
           mbar_arrive_expect_tx(q_full(s), kQStageBytes);
           tma_load_4d(sbase + kOffQ + s * kQStageStride, &P.in_map[tcd.level], q_full(s), ch * kChunk, tcd.x0 - 1,
                       tcd.y0 - 1, b);
@@ -377,25 +367,19 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
       const uint32_t idesc = idesc_tf32(256, 128);
       const uint64_t bhi0 = smem_desc_k_sw128(sbase + kOffBHi);
       const uint64_t blo0 = smem_desc_k_sw128(sbase + kOffBLo);
-      // A watcher thread (warp kWarpAlloc) does all the barrier waiting and publishes the number of sub-chunks whose
-      // operands are in place through one shared-memory word; this warp only polls that word.  The whole warp runs
-      // the loop converged and one elected lane issues, so that every tcgen05.mma operand is a warp-uniform value
-      // in a uniform register (inside an `if (lane == 0)` region ptxas wraps each MMA in a broadcast-and-retry loop
-      // whose latency exceeds the 64 cycles of the MMA itself).
+      // The watcher thread (warp kWarpAlloc) publishes the number of sub-chunks whose operands are in place; this warp
+      // only polls that word.  The whole warp runs the loop converged and one elected lane issues, so that every
+      // tcgen05.mma operand is a warp-uniform value in a uniform register (inside an `if (lane == 0)` region ptxas
+      // wraps each MMA in a broadcast-and-retry loop whose latency exceeds the 64 cycles of the MMA itself).
       int n_iter = 0;
       for (int i = 0; iter_valid(i); ++i) ++n_iter;
       const uint32_t total = (uint32_t)n_iter * kNumSubs;
-      const uint32_t flag = sbase + kOffFlag;
       uint32_t upto = 0;
       for (uint32_t g = 0; g < total; ++g) {
-        while (upto <= g) {
-          uint32_t v;
-          asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"(flag) : "memory");
-          upto = __shfl_sync(0xffffffffu, v, 0);
-        }
+        flag_wait(sbase + kOffFlag, upto, g);
         tc_fence_after();
-        const int sub = g % kNumSubs, s = g % kAStages;
-        const int as_ = (g / kNumSubs) % kAccStages;
+        const int sub = g % kNumSubs;
+        const uint32_t s = ring_stage(g, kAStages), as_ = ring_stage(g / kNumSubs, kAccStages);
         const uint32_t d = tmem_base + kColAcc + as_ * 128;
         const uint32_t a0 = tmem_base + kColA + s * kAStageCols;
         if (elect_one()) {
@@ -424,14 +408,13 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
       int n_iter = 0;
       for (int i = 0; iter_valid(i); ++i) ++n_iter;
       const uint32_t total = (uint32_t)n_iter * kNumSubs;
-      const uint32_t flag = sbase + kOffFlag;
       for (uint32_t g = 0; g < total; ++g) {
         if (g % kNumSubs == 0) {  // first sub-chunk of a tile: its accumulator must have been drained
           const uint32_t it = g / kNumSubs;
-          mbar_wait(acc_empty(it % kAccStages), ((it / kAccStages) & 1) ^ 1);
+          mbar_wait(acc_empty(ring_stage(it, kAccStages)), ring_phase(it, kAccStages) ^ 1);
         }
-        mbar_wait(a_full(g % kAStages), (g / kAStages) & 1);
-        asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(flag), "r"(g + 1) : "memory");
+        mbar_wait(a_full(ring_stage(g, kAStages)), ring_phase(g, kAStages));
+        flag_publish(sbase + kOffFlag, g + 1);
       }
     }
   } else if (warp >= kWarpEpi0 && warp < kWarpEpi0 + 4) {
@@ -445,9 +428,8 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
       bool do_store = t < T;
       TileCoord tcd = decode_tile(P, min(t, T - 1));
       const int pg = tcd.b * P.num_classes + P.class_begin + tcd.cc;
-      int as_ = i % kAccStages;
-      uint32_t aph = (i / kAccStages) & 1;
-      mbar_wait(acc_full(as_), aph);
+      const uint32_t as_ = ring_stage(i, kAccStages);
+      mbar_wait(acc_full(as_), ring_phase(i, kAccStages));
       tc_fence_after();
       const uint32_t trow = tmem_base + ((uint32_t)(qd * 32) << 16) + kColAcc + as_ * 128;
       const bool px_valid = do_store && tcd.y0 + (m >> 4) < P.lv[tcd.level].H && tcd.x0 + (m & 15) < P.lv[tcd.level].W;
@@ -457,11 +439,7 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
         uint32_t v[32];
         tmem_ld32(trow + j * 32, v);
         tmem_wait_ld();
-        if (j == 3) {  // accumulator fully read: hand it back to the MMA warp
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * as_);
-        }
+        if (j == 3) acc_release(acc_empty_leader + 8u * as_, lane);   // accumulator fully read
         if (issuer) tma_store_wait_read<0>();  // staging tile free again
         named_bar_sync(1, 128);
 #pragma unroll
@@ -501,11 +479,7 @@ __global__ void __launch_bounds__(kThreads, 1) correlate_tc_kernel(const __grid_
     cx.rank = (int)rank;
     stencil_role(P, cx, warp);
   }
-  // ---------------------------------------------------------------------- teardown
-  __syncwarp();
-  tc_fence_before();
-  cluster_sync();
-  if (warp == kWarpAlloc) tmem_dealloc<2>(tmem_base, kTmemCols);
+  pair_teardown(warp, kWarpAlloc, tmem_base, kTmemCols);
 }
 
 }  // namespace ctc
@@ -541,12 +515,7 @@ extern "C" int fod_correlate_levels(const float* const* q, const float* const* t
   prm.b3 = b3;
   prm.num_levels = num_levels;
   prm.num_classes = num_classes;
-  int dev = 0, sms = 0;
-  FOD_CUDA_CALL(cudaGetDevice(&dev));
-  FOD_CUDA_CALL(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const int max_pairs = sms / 2 > 0 ? sms / 2 : 1;
-  FOD_CUDA_CALL(cudaFuncSetAttribute(ctc::correlate_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)ctc::kSmemAlloc));
+  void* args[] = {&prm};
   // The taps ride in the launch parameters (ctc::Params::taps, kMaxTapSets sets): classes are processed in groups that
   // fit, one persistent launch per group.  Nothing outside the launch is written: the call is re-entrant.
   const int group = ctc::kMaxTapSets / num_levels;
@@ -573,25 +542,11 @@ extern "C" int fod_correlate_levels(const float* const* q, const float* const* t
     prm.class_begin = c0;
     prm.class_count = cn;
     prm.total_tiles = (int)tiles;
-    const int need_pairs = (int)((tiles + 1) / 2);
-    prm.num_pairs = need_pairs < max_pairs ? need_pairs : max_pairs;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * prm.num_pairs);
-    cfg.blockDim = dim3(ctc::kThreads);
-    cfg.dynamicSmemBytes = ctc::kSmemAlloc;
-    cfg.stream = as_stream(stream);
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, ctc::correlate_tc_kernel, prm);
-    if (e != cudaSuccess) {
-      set_error("fod_correlate_levels: launch failed: %s", cudaGetErrorString(e));
-      return FOD_ERR_CUDA;
-    }
+    int rc = pair_count((tiles + 1) / 2, &prm.num_pairs);
+    if (rc != FOD_OK) return rc;
+    rc = launch_pairs((const void*)ctc::correlate_tc_kernel, args, prm.num_pairs, ctc::kThreads, ctc::kSmemAlloc, stream,
+                      "fod_correlate_levels");
+    if (rc != FOD_OK) return rc;
   }
   return FOD_OK;
 }

@@ -18,18 +18,14 @@
 //     six output dot products, the softmax and the box decoding need no cross-lane traffic.
 #include <cuda_fp16.h>
 
-#include "common.cuh"
+#include "pair.cuh"
 #include "split_format.cuh"
-#include "tc05.cuh"
 
 namespace fod {
 
 using namespace tc;
 
 namespace rtc {
-#ifndef FOD_EXP
-#define FOD_EXP 0
-#endif
 
 constexpr int kK = 64 * kC;          // 8192
 constexpr int kChunk = 32;           // K per pipeline stage
@@ -62,15 +58,12 @@ constexpr uint32_t kOffFlag = kOffTmemPtr + 8;   // chunks released to the MMA t
 constexpr uint32_t kSmemBytes = kOffTmemPtr + 16;
 constexpr uint32_t kSmemAlloc = kSmemBytes + 1024;
 
-constexpr int kConvWarps = 8;        // converter warps per chunk: 4 TMEM quadrants x 2 halves of the 32-wide K chunk
-#ifndef FOD_REL_SETS
-#define FOD_REL_SETS 1
-#endif
-constexpr int kConvSets = FOD_REL_SETS;   // sets of converter warps that take alternate chunks: one chunk costs a warp
-                                          // ~900 cycles (two mbarrier waits of ~250 cycles each, the split, tcgen05.st),
-                                          // the 6 MMAs of a chunk 384
+// Converter warps: 4 TMEM quadrants x 2 halves of the 32-wide K chunk.  One chunk costs a warp ~900 cycles (two mbarrier
+// waits of ~250 cycles each, the split, tcgen05.st), the 6 MMAs of a chunk 384; a second set of 8 warps taking alternate
+// chunks measured neutral (119 vs 120 us)
+constexpr int kConvWarps = 8;
 constexpr int kWarpTma = 0, kWarpMma = 1, kWarpAlloc = 2, kWarpTmaB = 3, kWarpEpi0 = 4, kWarpConv0 = 8;
-constexpr int kThreads = (kWarpConv0 + kConvWarps * kConvSets) * 32;  // 512 (768 with two sets: measured neutral, 119 vs 120 us)
+constexpr int kThreads = (kWarpConv0 + kConvWarps) * 32;  // 512
 
 constexpr uint32_t kTmemCols = 512;
 constexpr uint32_t kAStageCols = 32; // [hi: 16 columns of packed fp16 pairs | lo: 16]
@@ -98,7 +91,7 @@ struct Params {
   const float* w_out;     // [6][128]
   const float* b_out;     // [6]
   float reg_w[4];
-  int num_problems, classes, roi_cap, tiles_per_problem, total_slots, num_pairs;
+  int num_problems, classes, roi_cap, tiles_per_problem, num_pairs;
 };
 
 struct Slot {
@@ -134,13 +127,7 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
   const uint32_t rank = blockIdx.x & 1;  // == %cluster_ctarank for cluster dims (2,1,1)
   const int pair = blockIdx.x >> 1;
   float xs = 1.f, xs_inv = 1.f;   // operand scale 2^e of the pooled rows (converters) and its inverse (epilogue)
-  auto image_scale = [&](int img) {
-    float amax = 0.f;
-    const float* col = P.x_amax + (P.amax_stride ? img : 0);
-    const int step = P.amax_stride ? P.amax_stride : 1;
-    for (int i = 0; i < P.n_amax; ++i) amax = fmaxf(amax, __ldg(col + (size_t)i * step));
-    pow2_scale(amax, xs, xs_inv);
-  };
+  auto image_scale = [&](int img) { pow2_scale(image_bound(P.x_amax, P.n_amax, P.amax_stride, img), xs, xs_inv); };
   image_scale(0);
 
   const uint32_t bar0 = sbase + kOffBars;
@@ -167,42 +154,36 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
     *reinterpret_cast<volatile uint32_t*>(smem + kOffFlag) = 0;
     fence_barrier_init();
   }
-  if (warp == kWarpAlloc) {
-    tmem_alloc<2>(sbase + kOffTmemPtr, kTmemCols);
-    tmem_relinquish<2>();
-  }
-  if (warp == kWarpTma && lane == 0) {
-    tma_prefetch_desc(&P.a_map);
-    tma_prefetch_desc(&P.whi_map);
-    tma_prefetch_desc(&P.wlo_map);
-  }
-  for (int i = tid; i < 6 * kC + 6; i += kThreads)
-    reinterpret_cast<float*>(smem + kOffWout)[i] = i < 6 * kC ? P.w_out[i] : P.b_out[i - 6 * kC];
   int* pref = reinterpret_cast<int*>(smem + kOffPref);
-  if (warp == kWarpTmaB) {  // exclusive prefix sum of the unit counts, one warp, 32 problems per step
-    int carry = 0;
-    for (int base = 0; base < P.num_problems; base += 32) {
-      const int p = base + lane;
-      int v = 0;
-      if (p < P.num_problems) {
-        const int cnt = P.roi_count ? min(__ldg(P.roi_count + p), P.roi_cap) : P.roi_cap;
-        v = (max(cnt, 0) + 127) >> 7;
-      }
-      int inc = v;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += n;
-      }
-      if (p < P.num_problems) pref[p] = carry + inc - v;
-      carry += __shfl_sync(0xffffffffu, inc, 31);
+  const uint32_t tmem_base = pair_setup(smem + kOffTmemPtr, warp, kWarpAlloc, kTmemCols, [&] {
+    if (warp == kWarpTma && lane == 0) {
+      tma_prefetch_desc(&P.a_map);
+      tma_prefetch_desc(&P.whi_map);
+      tma_prefetch_desc(&P.wlo_map);
     }
-    if (lane == 0) pref[P.num_problems] = carry;
-  }
-  tc_fence_before();
-  cluster_sync();
-  tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr);
+    for (int i = tid; i < 6 * kC + 6; i += kThreads)
+      reinterpret_cast<float*>(smem + kOffWout)[i] = i < 6 * kC ? P.w_out[i] : P.b_out[i - 6 * kC];
+    if (warp == kWarpTmaB) {  // exclusive prefix sum of the unit counts, one warp, 32 problems per step
+      int carry = 0;
+      for (int base = 0; base < P.num_problems; base += 32) {
+        const int p = base + lane;
+        int v = 0;
+        if (p < P.num_problems) {
+          const int cnt = P.roi_count ? min(__ldg(P.roi_count + p), P.roi_cap) : P.roi_cap;
+          v = (max(cnt, 0) + 127) >> 7;
+        }
+        int inc = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const int n = __shfl_up_sync(0xffffffffu, inc, o);
+          if (lane >= o) inc += n;
+        }
+        if (p < P.num_problems) pref[p] = carry + inc - v;
+        carry += __shfl_sync(0xffffffffu, inc, 31);
+      }
+      if (lane == 0) pref[P.num_problems] = carry;
+    }
+  });
 
   // Static schedule over the dense unit list: iteration i of pair k owns units 2*(i*num_pairs+k) and +1.
   const int total_units = pref[P.num_problems];
@@ -217,12 +198,8 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
         const Slot me = decode_unit(P, pref, slot_of(i, rank));
         const int tile0 = (me.p * P.tiles_per_problem + (me.r0 >> 7)) * kNumChunks;  // first A tile of this unit
         for (int kc = 0; kc < kNumChunks; ++kc, ++g) {
-          const int s = g % kStages;
-          const uint32_t ph = (g / kStages) & 1;
-          mbar_wait(a_empty(s), ph ^ 1);
-#if FOD_EXP == 1
-          if (g >= (uint32_t)kStages) { mbar_arrive(a_full(s)); continue; }
-#endif
+          const uint32_t s = ring_stage(g, kStages);
+          mbar_wait(a_empty(s), ring_phase(g, kStages) ^ 1);
           mbar_arrive_expect_tx(a_full(s), kABytes);
           tma_load_2d(sbase + kOffA + s * kABytes, &P.a_map, a_full(s), 0, (tile0 + kc) * 128);
         }
@@ -239,13 +216,9 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
       uint32_t g = 0;
       for (int i = 0; in_range(i); ++i) {
         for (int kc = 0; kc < kNumChunks; ++kc, ++g) {
-          const int s = g % kStages;
-          const uint32_t ph = (g / kStages) & 1;
+          const uint32_t s = ring_stage(g, kStages);
           // each CTA loads its 64 rows; both CTAs' bytes complete on the LEADER's barrier
-          mbar_wait(st_free(s), ph ^ 1);
-#if FOD_EXP == 2
-          if (g >= (uint32_t)kStages) { if (rank == 0) mbar_arrive(ready(s)); continue; }
-#endif
+          mbar_wait(st_free(s), ring_phase(g, kStages) ^ 1);
           if (rank == 0) mbar_arrive_expect_tx(ready(s), 2 * kBBytes);
           tma_load_2d_2sm(sbase + kOffB + s * kBBytes, &P.whi_map, b_full_leader + 8u * s, kc * kChunk, rank * kBHalfRows);
           tma_load_2d_2sm(sbase + kOffB + s * kBBytes + kBPlaneBytes, &P.wlo_map, b_full_leader + 8u * s, kc * kChunk,
@@ -256,26 +229,18 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
   } else if (warp == kWarpMma) {
     if (rank == 0) {
       const uint32_t idesc = idesc_f16(256, 128);
-      // A helper thread (warp kWarpAlloc) does all the barrier waiting and publishes the number of chunks whose
-      // operands are in place through one shared-memory word; this warp only polls that word.  The whole warp runs
-      // the loop converged and one elected lane issues, so that every tcgen05.mma operand is a warp-uniform value
-      // in a uniform register (inside an `if (lane == 0)` region ptxas wraps each MMA in a broadcast-and-retry loop
-      // whose latency exceeds the 64 cycles of the MMA itself).
+      // The watcher thread (warp kWarpAlloc) publishes the number of chunks whose operands are in place; this warp only
+      // polls that word.  The whole warp runs the loop converged and one elected lane issues, so that every tcgen05.mma
+      // operand is a warp-uniform value in a uniform register (inside an `if (lane == 0)` region ptxas wraps each MMA in
+      // a broadcast-and-retry loop whose latency exceeds the 64 cycles of the MMA itself).
       int n_iter = 0;
       for (int i = 0; in_range(i); ++i) ++n_iter;
       const uint32_t total = (uint32_t)n_iter * kNumChunks;
-      const uint32_t flag = sbase + kOffFlag;
       uint32_t upto = 0;
       for (uint32_t g = 0; g < total; ++g) {
-        while (upto <= g) {
-          uint32_t v;
-          asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"(flag) : "memory");
-          upto = __shfl_sync(0xffffffffu, v, 0);
-        }
+        flag_wait(sbase + kOffFlag, upto, g);
         tc_fence_after();
-        const int s = g % kStages;
-        const uint32_t gp = g / kChunksPerPart;
-        const int as_ = gp % kAccStages;
+        const uint32_t s = ring_stage(g, kStages), as_ = ring_stage(g / kChunksPerPart, kAccStages);
         const bool first = (g % kChunksPerPart) == 0, last = (g % kChunksPerPart) == kChunksPerPart - 1;
         const uint32_t d = tmem_base + kColAcc + as_ * 128;
         const uint32_t a0 = tmem_base + kColA + s * kAStageCols;
@@ -302,16 +267,14 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
       int n_iter = 0;
       for (int i = 0; in_range(i); ++i) ++n_iter;
       const uint32_t total = (uint32_t)n_iter * kNumChunks;
-      const uint32_t flag = sbase + kOffFlag;
       for (uint32_t g = 0; g < total; ++g) {
-        const int s = g % kStages;
-        const uint32_t ph = (g / kStages) & 1;
-        mbar_wait(ready(s), ph);    // A chunk of both CTAs is in tensor memory and the weight chunks have landed
+        // A chunk of both CTAs is in tensor memory and the weight chunks have landed
+        mbar_wait(ready(ring_stage(g, kStages)), ring_phase(g, kStages));
         if (g % kChunksPerPart == 0) {  // first chunk of a partial sum: its accumulator must have been drained
           const uint32_t gp = g / kChunksPerPart;
-          mbar_wait(acc_empty(gp % kAccStages), ((gp / kAccStages) & 1) ^ 1);
+          mbar_wait(acc_empty(ring_stage(gp, kAccStages)), ring_phase(gp, kAccStages) ^ 1);
         }
-        asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(flag), "r"(g + 1) : "memory");
+        flag_publish(sbase + kOffFlag, g + 1);
       }
     }
   } else if (warp >= kWarpEpi0 && warp < kWarpEpi0 + 4) {
@@ -341,9 +304,8 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
       float out[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
 #pragma unroll 1
       for (int part = 0; part < kParts; ++part, ++gp) {
-        const int as_ = gp % kAccStages;
-        const uint32_t aph = (gp / kAccStages) & 1;
-        mbar_wait(acc_full(as_), aph);
+        const uint32_t as_ = ring_stage(gp, kAccStages);
+        mbar_wait(acc_full(as_), ring_phase(gp, kAccStages));
         tc_fence_after();
         const uint32_t trow = tmem_base + ((uint32_t)(qd * 32) << 16) + kColAcc + as_ * 128;
 #pragma unroll 1
@@ -351,11 +313,7 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
           uint32_t v[32];
           tmem_ld32(trow + j * 32, v);
           tmem_wait_ld();
-          if (j == 3) {  // accumulator fully read: hand it back to the MMA warp
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * as_);
-          }
+          if (j == 3) acc_release(acc_empty_leader + 8u * as_, lane);   // accumulator fully read
 #pragma unroll
           for (int c4 = 0; c4 < 8; ++c4) {
             const uint32_t sa = sum_s + (uint32_t)(j * 8 + c4) * 2048;
@@ -409,7 +367,7 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
     }
   } else if (warp >= kWarpConv0) {
     // ------------------------------------------------------------------ converters: A chunk smem -> tf32 hi/lo in TMEM
-    const int wc = (warp - kWarpConv0) % kConvWarps, set = (warp - kWarpConv0) / kConvWarps;
+    const int wc = warp - kWarpConv0;
     const int qd = wc & 3, half = wc >> 2;
     const int m = qd * 32 + lane;
     const uint32_t ready_leader = map_to_cta(ready(0), 0);
@@ -419,9 +377,7 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
     for (int i = 0; in_range(i); ++i) {
       if (P.amax_stride) image_scale(decode_unit(P, pref, slot_of(i, rank)).p / P.classes);
       for (int kc = 0; kc < kNumChunks; ++kc, ++g) {
-        if ((int)(g % kConvSets) != set) continue;
-        const int s = g % kStages;
-        const uint32_t ph = (g / kStages) & 1;
+        const uint32_t s = ring_stage(g, kStages), ph = ring_phase(g, kStages);
         mbar_wait(a_full(s), ph);
         const uint32_t at = sbase + kOffA + s * kABytes + arow;
         float4 x[4];
@@ -447,10 +403,7 @@ __global__ void __launch_bounds__(kThreads, 1) relation_tc_kernel(const __grid_c
       }
     }
   }
-  __syncwarp();
-  tc_fence_before();
-  cluster_sync();
-  if (warp == kWarpAlloc) tmem_dealloc<2>(tmem_base, kTmemCols);
+  pair_teardown(warp, kWarpAlloc, tmem_base, kTmemCols);
 }
 
 }  // namespace rtc
@@ -504,31 +457,10 @@ extern "C" int fod_relation_head(const float* pooled, const float* x_amax, int n
   prm.classes = problems_per_image;
   prm.roi_cap = roi_cap;
   prm.tiles_per_problem = (roi_cap + 127) / 128;
-  prm.total_slots = num_problems * prm.tiles_per_problem;
-  int dev = 0, sms = 0;
-  FOD_CUDA_CALL(cudaGetDevice(&dev));
-  FOD_CUDA_CALL(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const int max_pairs = sms / 2 > 0 ? sms / 2 : 1;
-  const int need_pairs = (prm.total_slots + 1) / 2;
-  prm.num_pairs = need_pairs < max_pairs ? need_pairs : max_pairs;
-  FOD_CUDA_CALL(cudaFuncSetAttribute(rtc::relation_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)rtc::kSmemAlloc));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * prm.num_pairs);
-  cfg.blockDim = dim3(rtc::kThreads);
-  cfg.dynamicSmemBytes = rtc::kSmemAlloc;
-  cfg.stream = as_stream(stream);
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, rtc::relation_tc_kernel, prm);
-  if (e != cudaSuccess) {
-    set_error("fod_relation_head: launch failed: %s", cudaGetErrorString(e));
-    return FOD_ERR_CUDA;
-  }
-  return FOD_OK;
+  const int total_slots = num_problems * prm.tiles_per_problem;   // the most units the ROI counts can make
+  rc = pair_count((total_slots + 1) / 2, &prm.num_pairs);
+  if (rc != FOD_OK) return rc;
+  void* args[] = {&prm};
+  return launch_pairs((const void*)rtc::relation_tc_kernel, args, prm.num_pairs, rtc::kThreads, rtc::kSmemAlloc, stream,
+                      "fod_relation_head");
 }

@@ -48,12 +48,9 @@ __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarr
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
-// arrive on a barrier of another (or this) CTA of the cluster; `bar` is a shared::cluster address
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// same without the cluster-scope release (no memory barrier): for hand-offs whose payload is not generic memory
-// (tensor memory made visible by tcgen05.wait + tcgen05.fence::before_thread_sync)
+// arrive on a barrier of another (or this) CTA of the cluster; `bar` is a shared::cluster address.  No cluster-scope
+// release (no memory barrier): for hand-offs whose payload is not generic memory (tensor memory made visible by
+// tcgen05.wait + tcgen05.fence::before_thread_sync)
 __device__ __forceinline__ void mbar_arrive_remote(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(bar) : "memory");
 }
@@ -76,24 +73,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
-    if (++spins > (1u << 26)) __trap();
-  }
-}
-// acquire at cluster scope (needed when the arrivals come from the peer CTA)
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cluster(bar, parity)) {
     if (++spins > (1u << 26)) __trap();
   }
 }
@@ -180,15 +159,7 @@ __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
-// 32 lanes x 32-bit, 16 / 32 consecutive columns: thread t of the warp <-> TMEM lane (quadrant base + t)
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr)
-      : "memory");
-}
+// 32 lanes x 32-bit, 32 consecutive columns: thread t of the warp <-> TMEM lane (quadrant base + t)
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
