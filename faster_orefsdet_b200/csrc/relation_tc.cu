@@ -73,7 +73,7 @@ constexpr uint32_t kColAcc = 256;    // 2 stages x 128
 constexpr float kScaleClamp = 4.135166556742356f;  // log(1000/16), d2 box_regression.py:13
 
 struct Params {
-  CUtensorMap a_map;    // pooled, tiled [P*units*256*128][32], box 32 x 128 (one contiguous 16 KB A tile)
+  CUtensorMap a_map;    // pooled, tiled [P*units*256*128][32] (pooled_row in roi.cu), box 32 x 128 (one contiguous 16 KB A tile)
   CUtensorMap whi_map;  // w_fold fp16 hi plane [128][8192], box 32 x 64
   CUtensorMap wlo_map;  // w_fold fp16 lo plane
   const float* x_amax;    // [n_amax] bounds of max|pooled| (= of the feature maps); their maximum fixes the A scale

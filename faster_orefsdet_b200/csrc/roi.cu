@@ -16,7 +16,6 @@ struct RoiParams {
   int num_levels;
   int C;        // problems per image
   int roi_cap;
-  int R;        // output resolution
   int tiled;    // output layout, see roi_align_kernel
   int pix;      // floats per pixel of the maps = channels (a multiple of 128; blockIdx.z selects the 128-channel block)
 };
@@ -99,6 +98,8 @@ struct alignas(16) RoiBlob {
 struct BoxGeom {
   int lvl, H, W, grid_w, grid_h;
   float start_w, start_h, bin_w, bin_h;
+  bool tables;       // the sampling grid fits the tap tables
+  float inv_count;   // 1 / samples per bin
 };
 
 template <int R>
@@ -121,34 +122,46 @@ __device__ __forceinline__ BoxGeom box_geometry(const RoiParams& prm, const floa
   g.grid_w = (int)ceilf(__fdiv_rn(roi_w, (float)R));
   g.bin_w = __fdiv_rn(roi_w, (float)R);
   g.bin_h = __fdiv_rn(roi_h, (float)R);
+  g.tables = g.grid_h <= kMaxGrid && g.grid_w <= kMaxGrid;
+  g.inv_count = 1.0f / fmaxf((float)(g.grid_h * g.grid_w), 1.0f);
   return g;
 }
 
+// Everything of the blob but the tap tables: all that pool_one_roi needs for a ROI beyond the tables.
+template <int R>
+__device__ __forceinline__ void write_blob_header(RoiBlob<R>& B, const BoxGeom& g) {
+  B.gbox[0] = g.start_w; B.gbox[1] = g.start_h; B.gbox[2] = g.bin_w; B.gbox[3] = g.bin_h;
+  B.grid_w = g.grid_w; B.grid_h = g.grid_h; B.W = g.W; B.H = g.H;
+  B.level = g.lvl;
+  B.tables = g.tables ? 1 : 0;
+  B.inv_count = g.inv_count;
+  B.pad = 0;
+}
+
 // The list of DISTINCT map rows (columns) the samples of one bin touch along one axis, with the summed interpolation
-// weight of each (at most grid + 1 <= kMaxTaps entries, ascending).
-__device__ __forceinline__ int build_axis_taps(const BoxGeom& g, bool is_x, int bin, int (&idx)[kMaxTaps], float (&w)[kMaxTaps]) {
+// weight of each, in the order torchvision adds them.  The indices are CONSECUTIVE (the sampling step bin / grid is at
+// most one pixel and the clamped ends repeat the border index), so entry q is index first + q and a sample adds its two
+// weights to the slots lo - first and hi - first: w[] stays in registers.  Returns the number of entries n (at most
+// grid + 1 <= kMaxTaps); w[q] = 0 for q >= n.
+__device__ __forceinline__ int build_axis_taps(const BoxGeom& g, bool is_x, int bin, int& first, float (&w)[kMaxTaps]) {
   int n = 0;
+  first = 0;
+#pragma unroll
+  for (int q = 0; q < kMaxTaps; ++q) w[q] = 0.f;
   const int grid = is_x ? g.grid_w : g.grid_h, size = is_x ? g.W : g.H;
   const float start = is_x ? g.start_w : g.start_h, bsz = is_x ? g.bin_w : g.bin_h;
   for (int i = 0; i < grid; ++i) {
     const AxisSample s = axis_sample(start, bsz, bin, i, grid, size);
     if (s.w_lo == 0.f && s.w_hi == 0.f) continue;
-    if (n > 0 && idx[n - 1] == s.lo) {
-      w[n - 1] += s.w_lo;
-    } else if (n > 1 && idx[n - 2] == s.lo) {
-      w[n - 2] += s.w_lo;
-    } else {
-      idx[n] = s.lo;
-      w[n] = s.w_lo;
-      ++n;
-    }
-    if (idx[n - 1] == s.hi) {
-      w[n - 1] += s.w_hi;
-    } else {
-      idx[n] = s.hi;
-      w[n] = s.w_hi;
-      ++n;
-    }
+    if (n == 0) first = s.lo;
+    const int dlo = s.lo - first, dhi = s.hi - first;
+#pragma unroll
+    for (int q = 0; q < kMaxTaps; ++q)
+      if (q == dlo) w[q] += s.w_lo;
+#pragma unroll
+    for (int q = 0; q < kMaxTaps; ++q)
+      if (q == dhi) w[q] += s.w_hi;
+    n = max(n, dhi + 1);
   }
   return n;
 }
@@ -166,30 +179,23 @@ __global__ void __launch_bounds__(256) roi_tables_kernel(RoiParams prm, const fl
   const float4 box = *reinterpret_cast<const float4*>(rois + ((size_t)p * prm.roi_cap + r) * 4);
   const BoxGeom g = box_geometry<R>(prm, box);
   RoiBlob<R>& B = blobs[(size_t)p * prm.roi_cap + r];
-  const bool tables = g.grid_h <= kMaxGrid && g.grid_w <= kMaxGrid;
   if (k == 0) {
     if (out_level) out_level[(size_t)p * prm.roi_cap + r] = g.lvl;
-    B.gbox[0] = g.start_w; B.gbox[1] = g.start_h; B.gbox[2] = g.bin_w; B.gbox[3] = g.bin_h;
-    B.grid_w = g.grid_w; B.grid_h = g.grid_h; B.W = g.W; B.H = g.H;
-    B.level = g.lvl;
-    B.tables = tables ? 1 : 0;
-    B.inv_count = 1.0f / fmaxf((float)(g.grid_h * g.grid_w), 1.0f);
-    B.pad = 0;
+    write_blob_header(B, g);
   }
-  if (!tables) return;
+  if (!g.tables) return;
   const bool is_x = k < R;
   const int bin = is_x ? k : k - R;
-  // the list of DISTINCT rows / columns the bin's samples touch with their summed weights
-  int idx[kMaxTaps];
+  int first;
   float w[kMaxTaps];
-  const int n = build_axis_taps(g, is_x, bin, idx, w);
+  const int n = build_axis_taps(g, is_x, bin, first, w);
   const int pitch = is_x ? prm.pix : g.W * prm.pix;
   int* po = is_x ? B.xoff[bin] : B.yoff[bin];
   float* pw = is_x ? B.xw[bin] : B.yw[bin];
 #pragma unroll
-  for (int q = 0; q < kMaxTaps; ++q) {
-    po[q] = (q < n ? idx[q] : 0) * pitch;
-    pw[q] = q < n ? w[q] : 0.f;
+  for (int q = 0; q < kMaxTaps; ++q) {      // padding: offset 0, weight 0
+    po[q] = q < n ? (first + q) * pitch : 0;
+    pw[q] = w[q];
   }
   (is_x ? B.xn : B.yn)[bin] = n;
 }
@@ -225,6 +231,22 @@ __device__ __forceinline__ void roi_accumulate(const RoiBlob<R>& B, const float*
       }
     }
   }
+}
+
+// Where a lane stores its 4 channels of bin 0 of a pooled ROI row (problem p, ROI r, 128-channel block cblock), and the
+// stride from one bin to the next.  tiled == 0: [P][roi_cap][bins][pix] (row-major ROI rows).  tiled == 1 (8 x 8 bins,
+// 128 channels, consumed by fod_relation_head): [P][units][256 k-chunks][128 rows][32], units = ceil(roi_cap / 128): the
+// 16 KB A tile of one 32-wide K chunk of 128 ROI rows is contiguous, so one TMA box fetches it as a linear stream.
+// The stride is a function of its own: as a separate select the compiler turns the tile kernel's per-bin multiply
+// into a shift.
+__device__ __forceinline__ float* pooled_row(float* pooled, bool tiled, int roi_cap, int bins, int pix, int p, int r,
+                                             unsigned cblock, int lane) {
+  const int units = (roi_cap + 127) >> 7;
+  return tiled ? pooled + ((((size_t)p * units + (r >> 7)) * 256 + (lane >> 3)) * 128 + (r & 127)) * 32 + (lane & 7) * 4
+               : pooled + ((size_t)p * roi_cap + r) * bins * pix + cblock * kC + lane * 4;
+}
+__device__ __forceinline__ size_t pooled_bin_stride(bool tiled, int pix) {
+  return tiled ? (size_t)4 * 128 * 32 : (size_t)pix;   // tiled: next bin = 4 k-chunks further
 }
 
 // One CTA per ROI (and 128-channel block); warp = (bin row, half of the bin columns), lane = 4 channels: every tap is
@@ -289,19 +311,8 @@ __device__ __forceinline__ void pool_one_roi(const RoiParams& prm, const RoiBlob
     }
   }
   RPROF(2);
-  // Output layout.  tiled == 0: [P][roi_cap][R*R][128] (row-major ROI rows).  tiled == 1 (R == 8, consumed by
-  // fod_relation_head): [P][units][256 k-chunks][128 rows][32], units = ceil(roi_cap / 128): the 16 KB A tile of
-  // one 32-wide K chunk of 128 ROI rows is contiguous, so one TMA box fetches it as a linear stream.
-  float* out;
-  size_t bin_stride;
-  if (prm.tiled) {
-    const int units = (prm.roi_cap + 127) >> 7;
-    out = pooled + ((((size_t)p * units + (r >> 7)) * 256 + (lane >> 3)) * 128 + (r & 127)) * 32 + (lane & 7) * 4;
-    bin_stride = (size_t)4 * 128 * 32;  // next bin = 4 k-chunks further
-  } else {
-    out = pooled + ((size_t)p * prm.roi_cap + r) * R * R * prm.pix + blockIdx.z * kC + lane * 4;
-    bin_stride = prm.pix;
-  }
+  float* out = pooled_row(pooled, prm.tiled, prm.roi_cap, R * R, prm.pix, p, r, blockIdx.z, lane);
+  const size_t bin_stride = pooled_bin_stride(prm.tiled, prm.pix);
   const float inv_count = B.inv_count;
 #pragma unroll
   for (int j = 0; j < R / 2; ++j) {
@@ -386,33 +397,6 @@ struct Params {
 };
 }  // namespace rt
 
-// The same list without indexed local arrays: a bin's distinct rows / columns are CONSECUTIVE (the sampling step
-// bin / grid is at most one pixel and the clamped ends repeat the border index), so entry q is index first + q and a
-// sample adds its two weights to the slots lo - first and hi - first - the same additions in the same order as
-// build_axis_taps (the pooling tests compare the two bit for bit), but w[] stays in registers.
-__device__ __forceinline__ int build_axis_taps_reg(const BoxGeom& g, bool is_x, int bin, int& first, float (&w)[kMaxTaps]) {
-  int n = 0;
-  first = 0;
-#pragma unroll
-  for (int q = 0; q < kMaxTaps; ++q) w[q] = 0.f;
-  const int grid = is_x ? g.grid_w : g.grid_h, size = is_x ? g.W : g.H;
-  const float start = is_x ? g.start_w : g.start_h, bsz = is_x ? g.bin_w : g.bin_h;
-  for (int i = 0; i < grid; ++i) {
-    const AxisSample s = axis_sample(start, bsz, bin, i, grid, size);
-    if (s.w_lo == 0.f && s.w_hi == 0.f) continue;
-    if (n == 0) first = s.lo;
-    const int dlo = s.lo - first, dhi = s.hi - first;
-#pragma unroll
-    for (int q = 0; q < kMaxTaps; ++q)
-      if (q == dlo) w[q] += s.w_lo;
-#pragma unroll
-    for (int q = 0; q < kMaxTaps; ++q)
-      if (q == dhi) w[q] += s.w_hi;
-    n = max(n, dhi + 1);
-  }
-  return n;
-}
-
 // One thread per (ROI, axis, bin), 16 threads per ROI.  Tabled ROIs get a RoiTile; a ROI whose sampling grid is beyond
 // the tables gets the per-ROI kernel's blob header and an entry in the slow list.  Every ROI gets a RoiSum.
 __global__ void __launch_bounds__(256) roi_tile_tables_kernel(RoiParams prm, const float* __restrict__ rois,
@@ -429,13 +413,12 @@ __global__ void __launch_bounds__(256) roi_tile_tables_kernel(RoiParams prm, con
   const size_t row = (size_t)p * prm.roi_cap + (valid ? r : 0);
   const float4 box = *reinterpret_cast<const float4*>(rois + row * 4);
   const BoxGeom g = box_geometry<R>(prm, box);
-  const bool tables = g.grid_h <= kMaxGrid && g.grid_w <= kMaxGrid;
   const bool is_x = k < R;
   const int bin = k & 7;
   int first = 0;
   float w[kMaxTaps];
   int n = 0;
-  if (valid && tables) n = build_axis_taps_reg(g, is_x, bin, first, w);
+  if (valid && g.tables) n = build_axis_taps(g, is_x, bin, first, w);
   int nx = is_x ? n : 0;
   uint32_t yn = is_x ? 0u : ((uint32_t)n << (4 * bin));
 #pragma unroll
@@ -449,23 +432,17 @@ __global__ void __launch_bounds__(256) roi_tile_tables_kernel(RoiParams prm, con
     if (out_level) out_level[row] = g.lvl;
     S.level = (short)g.lvl;
     S.nx = (short)nx;
-    S.tables = tables ? 1 : 0;
+    S.tables = g.tables ? 1 : 0;
     S.pad = 0;
     S.yn = yn;
-    S.inv_count = 1.0f / fmaxf((float)(g.grid_h * g.grid_w), 1.0f);
-    if (!tables) {
-      RoiBlob<R>& B = blobs[row];
-      B.gbox[0] = g.start_w; B.gbox[1] = g.start_h; B.gbox[2] = g.bin_w; B.gbox[3] = g.bin_h;
-      B.grid_w = g.grid_w; B.grid_h = g.grid_h; B.W = g.W; B.H = g.H;
-      B.level = g.lvl;
-      B.tables = 0;
-      B.inv_count = 1.0f / fmaxf((float)(g.grid_h * g.grid_w), 1.0f);
-      B.pad = 0;
+    S.inv_count = g.inv_count;
+    if (!g.tables) {
+      write_blob_header(blobs[row], g);
       slow_list[1 + atomicAdd(slow_list, 1)] = (int32_t)row;
     }
   }
   (is_x ? S.x0 : S.y0)[bin] = (short)first;
-  if (!tables) return;
+  if (!g.tables) return;
   RoiTile& T = tiles[row];
   int4* pi = reinterpret_cast<int4*>(is_x ? T.xi[bin] : T.yi[bin]);
   float4* pw = reinterpret_cast<float4*>(is_x ? T.xw[bin] : T.yw[bin]);
@@ -566,7 +543,6 @@ roi_align_tiles_kernel(const __grid_constant__ rt::Params P, const int32_t* __re
     tc::tma_load_4d(sbase, &P.map[lvl], bar, 0, tx0, ty0, b);
   }
   bool waited = false;
-  const int units = (P.roi_cap + 127) >> 7;
   for (int c = 0; c < P.C; ++c) {
     const int p = b * P.C + c;
     const int cnt = roi_count ? min(roi_count[p], P.roi_cap) : P.roi_cap;
@@ -627,9 +603,8 @@ roi_align_tiles_kernel(const __grid_constant__ rt::Params P, const int32_t* __re
           const uint32_t nz_b = __ballot_sync(0xffffffffu, xb_w != 0.f);
           const int xa_b = xa_r * (kC * 4), xb_b = xb_r * (kC * 4);                    // byte offsets inside the tile
           const int ya_b = ya_r * (kEdge * kC * 4), yb_b = yb_r * (kEdge * kC * 4);
-          float* out_roi = P.tiled ? pooled + ((((size_t)p * units + (r >> 7)) * 256 + (lane >> 3)) * 128 + (r & 127)) * 32 + (lane & 7) * 4
-                                   : pooled + row * 64 * kC + lane * 4;
-          const uint32_t bin_stride = P.tiled ? 4u * 128u * 32u : (uint32_t)kC;
+          float* out_roi = pooled_row(pooled, P.tiled, P.roi_cap, 64, kC, p, r, 0, lane);
+          const size_t bin_stride = pooled_bin_stride(P.tiled, kC);
           for (uint32_t rows = ym; rows; rows &= rows - 1) {
             const int by = __ffs(rows) - 1;
             const bool yhi = by >= 4;
@@ -705,6 +680,32 @@ extern "C" int fod_roi_prof(long long* out8, int reset) {
 
 using namespace fod;
 
+// The workspace of one call of n = problems * roi_cap ROIs: blobs | tile tap lists | scan summaries | slow list (count +
+// entries).  Only resolution 8, where the tile-stationary path can run, has the parts after the blobs.
+struct RoiWorkspace {
+  size_t tiles, sums, slow;   // byte offsets
+  size_t bytes;
+};
+static RoiWorkspace roi_workspace(size_t n, int resolution) {
+  static_assert(sizeof(RoiBlob<8>) % 16 == 0 && sizeof(RoiTile) == 1024 && sizeof(RoiSum) == 48, "workspace layout");
+  RoiWorkspace w;
+  w.tiles = n * (resolution == 4 ? sizeof(RoiBlob<4>) : resolution == 8 ? sizeof(RoiBlob<8>) : sizeof(RoiBlob<14>));
+  w.sums = w.tiles + n * sizeof(RoiTile);
+  w.slow = w.sums + n * sizeof(RoiSum);
+  w.bytes = resolution == 8 ? w.slow + ((n + 1) * sizeof(int32_t) + 15) / 16 * 16 : w.tiles;
+  return w;
+}
+
+// One CTA per ROI and 128-channel block, after the pre-pass has written every ROI's blob.
+template <int R>
+static void launch_per_roi(const RoiParams& prm, unsigned P, const float* rois, const int32_t* roi_count, void* workspace,
+                           float* pooled, int32_t* out_level, cudaStream_t st) {
+  auto* blobs = static_cast<RoiBlob<R>*>(workspace);
+  roi_tables_kernel<R><<<dim3((unsigned)((prm.roi_cap * 2 * R + 255) / 256), P), 256, 0, st>>>(prm, rois, roi_count, blobs,
+                                                                                             out_level);
+  roi_align_kernel<R><<<dim3(prm.roi_cap, P, (unsigned)(prm.pix / kC)), R * 64, 0, st>>>(prm, roi_count, blobs, pooled);
+}
+
 // tile_stationary: 1 = the tile-stationary kernel where it applies (resolution 8, 128 channels), 0 = one CTA per ROI
 static int roi_align_impl(const float* const* feat, const fod_level_t* levels, int num_levels, int batch,
                           int problems_per_image, const float* rois, const int32_t* roi_count, int roi_cap,
@@ -734,20 +735,17 @@ static int roi_align_impl(const float* const* feat, const fod_level_t* levels, i
   prm.num_levels = num_levels;
   prm.C = problems_per_image;
   prm.roi_cap = roi_cap;
-  prm.R = resolution;
   prm.pix = channels;
   FOD_REQUIRE(!tiled || (resolution == 8 && channels == kC), "fod_roi_align: the tiled layout needs resolution 8 and 128 channels");
   prm.tiled = tiled ? 1 : 0;
-  dim3 grid(roi_cap, (unsigned)P, (unsigned)(channels / kC));
-  const dim3 tgrid((unsigned)((roi_cap * 2 * resolution + 255) / 256), (unsigned)P);
   cudaStream_t st = as_stream(stream);
   if (tile_stationary && resolution == 8 && channels == kC) {
-    const size_t n = (size_t)P * roi_cap;
-    auto* blobs = static_cast<RoiBlob<8>*>(workspace);
-    auto* tiles = reinterpret_cast<RoiTile*>(blobs + n);
-    auto* sums = reinterpret_cast<RoiSum*>(tiles + n);
-    auto* slow = reinterpret_cast<int32_t*>(sums + n);
-    static_assert(sizeof(RoiBlob<8>) % 16 == 0 && sizeof(RoiTile) == 1024 && sizeof(RoiSum) == 48, "workspace layout");
+    const RoiWorkspace ws = roi_workspace((size_t)P * roi_cap, resolution);
+    uint8_t* base = static_cast<uint8_t*>(workspace);
+    auto* blobs = reinterpret_cast<RoiBlob<8>*>(base);
+    auto* tiles = reinterpret_cast<RoiTile*>(base + ws.tiles);
+    auto* sums = reinterpret_cast<RoiSum*>(base + ws.sums);
+    auto* slow = reinterpret_cast<int32_t*>(base + ws.slow);
     rt::Params tp;
     int total = 0;
     for (int l = 0; l < num_levels; ++l) {
@@ -780,17 +778,11 @@ static int roi_align_impl(const float* const* feat, const fod_level_t* levels, i
                                                                                                      sums, pooled);
     roi_align_list_kernel<<<74, 512, 0, st>>>(prm, slow, blobs, pooled);
   } else if (resolution == 8) {
-    auto* blobs = static_cast<RoiBlob<8>*>(workspace);
-    roi_tables_kernel<8><<<tgrid, 256, 0, st>>>(prm, rois, roi_count, blobs, out_level);
-    roi_align_kernel<8><<<grid, 512, 0, st>>>(prm, roi_count, blobs, pooled);
+    launch_per_roi<8>(prm, (unsigned)P, rois, roi_count, workspace, pooled, out_level, st);
   } else if (resolution == 4) {
-    auto* blobs = static_cast<RoiBlob<4>*>(workspace);
-    roi_tables_kernel<4><<<tgrid, 256, 0, st>>>(prm, rois, roi_count, blobs, out_level);
-    roi_align_kernel<4><<<grid, 256, 0, st>>>(prm, roi_count, blobs, pooled);
+    launch_per_roi<4>(prm, (unsigned)P, rois, roi_count, workspace, pooled, out_level, st);
   } else {
-    auto* blobs = static_cast<RoiBlob<14>*>(workspace);
-    roi_tables_kernel<14><<<tgrid, 256, 0, st>>>(prm, rois, roi_count, blobs, out_level);
-    roi_align_kernel<14><<<grid, 896, 0, st>>>(prm, roi_count, blobs, pooled);
+    launch_per_roi<14>(prm, (unsigned)P, rois, roi_count, workspace, pooled, out_level, st);
   }
   FOD_CUDA_LAUNCH_CHECK("fod_roi_align");
   return FOD_OK;
@@ -813,10 +805,7 @@ extern "C" int fod_roi_align_per_roi(const float* const* feat, const fod_level_t
 }
 
 extern "C" size_t fod_roi_align_workspace_bytes(int num_problems, int roi_cap, int resolution) {
-  const size_t n = (size_t)num_problems * roi_cap;
-  if (resolution == 8)   // blobs | tile tap lists | scan summaries | slow list (count + entries)
-    return n * (sizeof(RoiBlob<8>) + sizeof(RoiTile) + sizeof(RoiSum)) + ((n + 1) * sizeof(int32_t) + 15) / 16 * 16;
-  return n * (resolution == 4 ? sizeof(RoiBlob<4>) : sizeof(RoiBlob<14>));
+  return roi_workspace((size_t)num_problems * roi_cap, resolution).bytes;
 }
 
 extern "C" int fod_roi_align(const float* const* feat, const fod_level_t* levels, int num_levels, int batch,
