@@ -77,4 +77,82 @@ __device__ __forceinline__ float box_area(const float4 b) { return __fmul_rn(__f
 
 float iou_threshold_as_float(double thr);
 
+// Block primitives of a 1024-thread CTA (32 warps); every thread of the CTA calls them.  Each ends with a barrier, after
+// which `sh` may be used again.
+//
+// op-reduction of one value per thread (op = a + b or fmaxf(a, b)); the result in every thread.  sh: __shared__ T[32]
+template <class T, class Op>
+__device__ inline T block_reduce(T v, T* sh, Op op) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = op(v, __shfl_xor_sync(0xffffffffu, v, o));
+  if (lane == 0) sh[warp] = v;
+  __syncthreads();
+  if (warp == 0) {
+    v = sh[lane];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = op(v, __shfl_xor_sync(0xffffffffu, v, o));
+    if (lane == 0) sh[0] = v;
+  }
+  __syncthreads();
+  const T r = sh[0];
+  __syncthreads();
+  return r;
+}
+
+// Exclusive prefix sum of one int per thread in thread order; `total` gets the sum over the CTA.  sh: __shared__ int[33]
+__device__ inline int block_exclusive_scan(int v, int* sh, int& total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int x = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, x, o);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) sh[warp] = x;
+  __syncthreads();
+  if (warp == 0) {
+    const int w = sh[lane];
+    int xs = w;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, xs, o);
+      if (lane >= o) xs += y;
+    }
+    sh[lane] = xs - w;
+    if (lane == 31) sh[32] = xs;
+  }
+  __syncthreads();
+  const int res = sh[warp] + x - v;
+  total = sh[32];
+  __syncthreads();
+  return res;
+}
+
+// Launches `kernel` on `clusters` clusters of `cluster_size` CTAs of `threads` threads with `smem_bytes` of dynamic
+// shared memory (also set as the kernel's limit).  args[i] points at a local of exactly the type of parameter i; `name`
+// prefixes the error message
+inline int launch_clusters(const void* kernel, void** args, int clusters, int cluster_size, int threads, size_t smem_bytes,
+                           fod_stream_t stream, const char* name) {
+  FOD_CUDA_CALL(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)clusters * (unsigned)cluster_size);
+  cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem_bytes;
+  cfg.stream = as_stream(stream);
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = (unsigned)cluster_size;
+  at[0].val.clusterDim.y = 1;
+  at[0].val.clusterDim.z = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  const cudaError_t e = cudaLaunchKernelExC(&cfg, kernel, args);
+  if (e != cudaSuccess) {
+    set_error("%s: launch failed: %s", name, cudaGetErrorString(e));
+    return FOD_ERR_CUDA;
+  }
+  return FOD_OK;
+}
+
 }  // namespace fod

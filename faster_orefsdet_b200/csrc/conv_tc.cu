@@ -1135,7 +1135,8 @@ static int conv2d_nhwc_impl(const float* x, int n, int h, int w, int cin, long x
   const void* kernel = smem_a ? (const void*)cvt::conv_tc_kernel_smem : (const void*)cvt::conv_tc_kernel_tmem;
   void* args[] = {&prm, smem_a ? (void*)&sm : (void*)&tm};
   const uint32_t smem_bytes = smem_a ? sm.off_sum + cvt::smem_a_tail_bytes(prm.ncol32) + 1024 : cvt::kSmemAlloc;
-  return launch_pairs(kernel, args, prm.num_pairs, smem_a ? cvt::kThreadsS : cvt::kThreads, smem_bytes, stream, "fod_conv2d_nhwc");
+  return launch_clusters(kernel, args, prm.num_pairs, 2, smem_a ? cvt::kThreadsS : cvt::kThreads, smem_bytes, stream,
+                         "fod_conv2d_nhwc");
 }
 
 extern "C" int fod_conv2d_nhwc(const float* x, int n, int h, int w, int cin, long x_pixel_stride, const float* x_amax,

@@ -544,8 +544,8 @@ extern "C" int fod_correlate_levels(const float* const* q, const float* const* t
     prm.total_tiles = (int)tiles;
     int rc = pair_count((tiles + 1) / 2, &prm.num_pairs);
     if (rc != FOD_OK) return rc;
-    rc = launch_pairs((const void*)ctc::correlate_tc_kernel, args, prm.num_pairs, ctc::kThreads, ctc::kSmemAlloc, stream,
-                      "fod_correlate_levels");
+    rc = launch_clusters((const void*)ctc::correlate_tc_kernel, args, prm.num_pairs, 2, ctc::kThreads, ctc::kSmemAlloc,
+                         stream, "fod_correlate_levels");
     if (rc != FOD_OK) return rc;
   }
   return FOD_OK;

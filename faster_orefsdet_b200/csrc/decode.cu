@@ -97,29 +97,13 @@ decode_topk_kernel(DecodeParams prm, float* __restrict__ boxes, float* __restric
   extern __shared__ __align__(16) unsigned char smem_raw[];
   uint32_t* keys = reinterpret_cast<uint32_t*>(smem_raw);
   __shared__ int hist[kDecWarps][256];
-  __shared__ int warp_sums[kDecWarps];
-  __shared__ int sh[8];
+  __shared__ int warp_sums[kDecWarps + 1];
+  __shared__ int sh[2];
   const int roles = min(prm.num_levels, 2);
   const int p = blockIdx.x / roles, role = blockIdx.x - p * roles;
   const int l_begin = role == 0 ? 0 : 1, l_end = (role == 0 && roles == 2) ? 1 : prm.num_levels;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  // block-wide sum of one int per thread (result in every thread)
-  auto block_sum = [&](int local) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) local += __shfl_xor_sync(0xffffffffu, local, o);
-    if (lane == 0) warp_sums[warp] = local;
-    __syncthreads();
-    if (warp == 0) {
-      int v = warp_sums[lane];
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-      if (lane == 0) sh[0] = v;
-    }
-    __syncthreads();
-    const int r = sh[0];
-    __syncthreads();
-    return r;
-  };
+  auto block_sum = [&](int local) { return block_reduce(local, warp_sums, [](int a, int b) { return a + b; }); };
   // key of pixel i of level ll: fp32 bits of the probability if it passes the threshold, else 0
   auto key_of = [&](int ll, int i) -> uint32_t {
     if (prm.taps) return __ldg(prm.keys + (size_t)p * prm.key_stride + prm.key_off[ll] + i);
@@ -201,8 +185,8 @@ decode_topk_kernel(DecodeParams prm, float* __restrict__ boxes, float* __restric
             int acc = above;
             for (int j = 7; j >= 0; --j) {
               if (acc + c[j] >= remaining) {
-                sh[1] = lane * 8 + j;
-                sh[2] = remaining - acc;
+                sh[0] = lane * 8 + j;
+                sh[1] = remaining - acc;
                 break;
               }
               acc += c[j];
@@ -210,9 +194,9 @@ decode_topk_kernel(DecodeParams prm, float* __restrict__ boxes, float* __restric
           }
         }
         __syncthreads();
-        prefix |= (uint32_t)sh[1] << shift;
+        prefix |= (uint32_t)sh[0] << shift;
         mask |= 255u << shift;
-        remaining = sh[2];
+        remaining = sh[1];
         __syncthreads();
       }
       T = prefix;
@@ -229,29 +213,9 @@ decode_topk_kernel(DecodeParams prm, float* __restrict__ boxes, float* __restric
       uint32_t k = (i < n) ? keys[i] : 0u;
       int is_gt = (k > T) ? 1 : 0;
       int is_eq = (T != 0u && k == T) ? 1 : 0;
-      int v = is_gt | (is_eq << 16);
-      // inclusive warp scan, then block offsets
-      int x = v;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        int y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= o) x += y;
-      }
-      if (lane == 31) warp_sums[warp] = x;
-      __syncthreads();
-      if (warp == 0) {
-        int w = warp_sums[lane], xs = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          int y = __shfl_up_sync(0xffffffffu, xs, o);
-          if (lane >= o) xs += y;
-        }
-        warp_sums[lane] = xs - w;
-        if (lane == 31) sh[3] = xs;
-      }
-      __syncthreads();
-      int excl = warp_sums[warp] + x - v;
-      int tot = sh[3];
+      // both counts in one scan: a level has fewer than 2^16 pixels (kMaxLevelPixels)
+      int tot;
+      const int excl = block_exclusive_scan(is_gt | (is_eq << 16), warp_sums, tot);
       int gt_pos = gt_before + (excl & 0xffff);
       int eq_pos = eq_before + (excl >> 16);
       bool sel = is_gt || (is_eq && eq_pos < need);
@@ -298,7 +262,6 @@ decode_topk_kernel(DecodeParams prm, float* __restrict__ boxes, float* __restric
       }
       gt_before += tot & 0xffff;
       eq_before += tot >> 16;
-      __syncthreads();
     }
     if (tid == 0) level_count[p * prm.num_levels + l] = nsel;
     if (tid == 0 && l == prm.num_levels - 1) cand_count[p] = min(out_base + nsel, prm.cand_cap);

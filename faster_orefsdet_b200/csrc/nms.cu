@@ -1,21 +1,22 @@
 // Greedy NMS kernels: one problem per CTA or per thread-block CLUSTER, everything resident in shared memory.
 //
-//   sort   : bitonic sort of 64-bit keys (~ordered(score) << 32 | index) -> stable
-//            score-descending order (lower input index first among equal scores).
+//   sort   : bitonic sort of 64-bit keys (~ordered(score) << 32 | row) -> stable score-descending order (lower input
+//            row first among equal scores); the boxes are then gathered in sorted order (sort_and_gather).
 //   sweep  : blocked greedy suppression, 64 sorted boxes per step:
 //              1. 64x64 IoU bit matrix of the chunk, stored by COLUMN (warp ballots),
 //              2. the chunk is resolved by ONE WARP with a fixed-point iteration on the column masks
 //                 (kept_j = alive_j and no kept_i, i < j, overlaps j: converges to the greedy answer in
 //                 (longest suppression chain + 1) ballot rounds instead of one serial step per survivor),
-//              3. the chunk's survivors suppress every later box (all threads; four lanes share a box).
+//              3. the chunk's survivors suppress every later box (all threads; G = 1..32 lanes share a box, more
+//                 the fewer boxes are alive).
 //            Only survivors ever test later boxes, so the work is kept*n/2 IoU
 //            pairs instead of n^2/2, and no n x n mask goes through HBM.
 //            The sweep stops as soon as the caller's top-k is decided.
 //   cluster: the kernel is instruction bound on one SM (profiles/r1_ncu_v5_summary.md: 59 % issue-active on 64 of
-//            148 SMs), so a problem may be spread over S = 1..8 CTAs of a cluster.  Every CTA holds the sorted boxes
+//            148 SMs), so a problem may be spread over S = 1, 2 or 4 CTAs of a cluster.  Every CTA holds the sorted boxes
 //            and resolves every chunk redundantly (identical results by construction); step 3 is split: CTA r owns
-//            the suppression words w with w % S == r.  After each chunk the owners of the next chunk's two words push
-//            them into every peer's shared memory (st.shared::cluster) and the cluster barriers once.
+//            the suppression words w with w % S == r.  After each pair of chunks the owners of the next pair's four
+//            words push them into every peer's shared memory (st.shared::cluster) and the cluster barriers once.
 //
 // IoU arithmetic is bit-identical to torchvision's CPU kernel (common.cuh).
 #include "common.cuh"
@@ -44,58 +45,87 @@ constexpr int kPreRead = 3;      // list passes a thread may hold in registers (
 constexpr int kMaxCluster = 4;   // measured: 8 CTAs per problem are slower than 4 (cluster barrier + the redundant sort / resolve)
 
 struct NmsSmem {
-  unsigned long long* keys;     // [npad]
-  float4* box;                  // [ncap] sorted boxes (possibly class-offset)
+  unsigned long long* keys;     // [npad] sort keys (sort_key), ~0 padding
+  float4* box;                  // [ncap] sorted boxes (clipped / class-offset as the kernel needs)
   float4* kbox;                 // [128] survivors of the chunk pair being applied
   uint32_t* colmask;            // [2 buffers][lo 64 | hi 64]: bit i of word j: chunk box i (i < j) overlaps chunk box j
   float* karea;                 // [128]
-  uint32_t* suppressed;         // [ncap/32 + 2]; a CTA of a cluster keeps only its own words up to date
+  uint32_t* suppressed;         // [nms_words(ncap)]; a CTA of a cluster keeps only its own words up to date
   uint32_t* chunk_sup;          // [2 parities][4 + 2]: suppression words of the chunk pair being resolved (pushed by their
                                 // owners), then the pair's two cross words (second chunk suppressed by the first one's survivors)
   int* scalars;                 // [8]
-  uint16_t* kept;               // [ncap] sorted ranks of survivors, growing from the front ...
+  uint16_t* kept;               // [ncap + 128] sorted ranks of survivors, growing from the front ...
   uint16_t* alist_top;          // ... and, from the END of the same array downwards (entry e at alist_top[-e]), this CTA's
                                 // boxes that are still alive and not yet resolved (any order).  While a pair of chunks is
                                 // being resolved the list still holds the pair's own <= 128 boxes: survivors + listed
                                 // <= n + 128, which is the size of the array.
 };
 
-__host__ __device__ inline int next_pow2(int n) {
+__host__ __device__ constexpr int next_pow2(int n) {
   int p = 1;
   while (p < n) p <<= 1;
   return p;
 }
 
-__host__ __device__ inline size_t nms_words(int ncap) { return (size_t)(ncap + 31) / 32 + 4; }   // 4 spare (zero) words
+__host__ __device__ constexpr size_t nms_words(int ncap) { return (size_t)(ncap + 31) / 32 + 4; }   // 4 spare (zero) words
 
-__host__ inline size_t nms_smem_bytes(int ncap) {
-  int npad = next_pow2(ncap < 64 ? 64 : ncap);
-  return (size_t)npad * 8 + (size_t)ncap * 16 + 128 * 16 + 2 * 128 * 4 + 128 * 4 + nms_words(ncap) * 4 + 48 + 32 + (size_t)(ncap + 2 * kChunk) * 2 + 64;
+// The layout of NmsSmem for up to ncap rows: where each array starts when the first starts at `base`, and where the
+// last one (with 64 bytes of slack) ends.  Walked with a pointer by carve and with a byte offset by nms_smem_bytes.
+template <class T>
+struct NmsArrays {
+  T keys, box, kbox, colmask, karea, suppressed, chunk_sup, scalars, kept, end;
+};
+template <class T>
+__host__ __device__ constexpr NmsArrays<T> nms_arrays(T base, int ncap) {
+  NmsArrays<T> a{};
+  a.keys = base;
+  base += (size_t)next_pow2(ncap < 64 ? 64 : ncap) * 8;
+  a.box = base;
+  base += (size_t)ncap * 16;
+  a.kbox = base;
+  base += 128 * 16;
+  a.colmask = base;
+  base += 2 * 128 * 4;
+  a.karea = base;
+  base += 128 * 4;
+  a.suppressed = base;
+  base += nms_words(ncap) * 4;
+  a.chunk_sup = base;
+  base += 48;
+  a.scalars = base;
+  base += 32;
+  a.kept = base;
+  base += (size_t)(ncap + 2 * kChunk) * 2 + 64;
+  a.end = base;
+  return a;
 }
 
+__host__ __device__ constexpr size_t nms_smem_bytes(int ncap) { return nms_arrays<size_t>(0, ncap).end; }
+// Every entry point rejects more than FOD_NMS_MAX_BOXES rows, and the size grows with the row count
+static_assert(nms_smem_bytes(FOD_NMS_MAX_BOXES) <= 227 * 1024, "the largest NMS problem must fit in shared memory");
+
 __device__ inline NmsSmem carve(unsigned char* base, int ncap) {
-  int npad = next_pow2(ncap < 64 ? 64 : ncap);
+  const NmsArrays<unsigned char*> a = nms_arrays(base, ncap);
   NmsSmem s;
-  s.keys = reinterpret_cast<unsigned long long*>(base);
-  base += (size_t)npad * 8;
-  s.box = reinterpret_cast<float4*>(base);
-  base += (size_t)ncap * 16;
-  s.kbox = reinterpret_cast<float4*>(base);
-  base += 128 * 16;
-  s.colmask = reinterpret_cast<uint32_t*>(base);
-  base += 2 * 128 * 4;
-  s.karea = reinterpret_cast<float*>(base);
-  base += 128 * 4;
-  s.suppressed = reinterpret_cast<uint32_t*>(base);
-  base += nms_words(ncap) * 4;
-  s.chunk_sup = reinterpret_cast<uint32_t*>(base);
-  base += 48;
-  s.scalars = reinterpret_cast<int*>(base);
-  base += 32;
-  s.kept = reinterpret_cast<uint16_t*>(base);
+  s.keys = reinterpret_cast<unsigned long long*>(a.keys);
+  s.box = reinterpret_cast<float4*>(a.box);
+  s.kbox = reinterpret_cast<float4*>(a.kbox);
+  s.colmask = reinterpret_cast<uint32_t*>(a.colmask);
+  s.karea = reinterpret_cast<float*>(a.karea);
+  s.suppressed = reinterpret_cast<uint32_t*>(a.suppressed);
+  s.chunk_sup = reinterpret_cast<uint32_t*>(a.chunk_sup);
+  s.scalars = reinterpret_cast<int*>(a.scalars);
+  s.kept = reinterpret_cast<uint16_t*>(a.kept);
   s.alist_top = s.kept + (ncap + 2 * kChunk - 1);
   return s;
 }
+
+// Sort key of input row `row`: ascending keys = descending scores, lower row first among equal scores
+__device__ __forceinline__ unsigned long long sort_key(float score, int row) {
+  return ((unsigned long long)(~float_to_ordered(score)) << 32) | (unsigned)row;
+}
+// Input row of sorted rank r
+__device__ __forceinline__ int row_of(const NmsSmem& s, int r) { return (int)(s.keys[r] & 0xffffffffu); }
 
 // One compare-exchange step of the bitonic network on E consecutive keys per thread held in registers (thread t owns
 // the global indices E*t .. E*t+E-1): partner distance j < 32*E, so the partner sits in this thread or in another lane
@@ -129,6 +159,20 @@ __device__ __forceinline__ void bitonic_reg_step(unsigned long long (&v)[E], int
   }
 }
 
+// One compare-exchange step (k, j) of the bitonic network on keys[0..npad) in shared memory, by the whole CTA; ends with
+// a barrier
+__device__ inline void bitonic_smem_step(unsigned long long* keys, int npad, int k, int j) {
+  for (int t = threadIdx.x; t < (npad >> 1); t += blockDim.x) {
+    const int i = 2 * t - (t & (j - 1)), l = i + j;
+    const unsigned long long a = keys[i], b = keys[l];
+    if ((a > b) == ((i & k) == 0)) {
+      keys[i] = b;
+      keys[l] = a;
+    }
+  }
+  __syncthreads();
+}
+
 template <int E>
 __device__ inline void bitonic_sort_reg(unsigned long long* keys, int npad) {
   // npad == E * blockDim.x.  Stages with partner distance >= 32*E go through shared memory, the rest stay in registers.
@@ -144,18 +188,7 @@ __device__ inline void bitonic_sort_reg(unsigned long long* keys, int npad) {
 #pragma unroll
     for (int e = 0; e < E; ++e) keys[g0 + e] = v[e];
     __syncthreads();
-    for (int j = k >> 1; j >= warp_span; j >>= 1) {
-      for (int tt = t; tt < (npad >> 1); tt += blockDim.x) {
-        const int i = 2 * tt - (tt & (j - 1)), l = i + j;
-        const unsigned long long a = keys[i], b = keys[l];
-        const bool up = (i & k) == 0;
-        if ((a > b) == up) {
-          keys[i] = b;
-          keys[l] = a;
-        }
-      }
-      __syncthreads();
-    }
+    for (int j = k >> 1; j >= warp_span; j >>= 1) bitonic_smem_step(keys, npad, k, j);
 #pragma unroll
     for (int e = 0; e < E; ++e) v[e] = keys[g0 + e];
     for (int j = warp_span >> 1; j > 0; j >>= 1) bitonic_reg_step<E>(v, k, j, g0);
@@ -170,21 +203,20 @@ __device__ inline void bitonic_sort(unsigned long long* keys, int npad) {
   if (npad == 2 * kNmsThreads) return bitonic_sort_reg<2>(keys, npad);
   if (npad == 4 * kNmsThreads) return bitonic_sort_reg<4>(keys, npad);
   if (npad == 8 * kNmsThreads) return bitonic_sort_reg<8>(keys, npad);
-  for (int k = 2; k <= npad; k <<= 1) {
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      for (int t = threadIdx.x; t < (npad >> 1); t += blockDim.x) {
-        int i = 2 * t - (t & (j - 1));
-        int l = i + j;
-        unsigned long long a = keys[i], b = keys[l];
-        bool up = (i & k) == 0;
-        if ((a > b) == up) {
-          keys[i] = b;
-          keys[l] = a;
-        }
-      }
-      __syncthreads();
-    }
-  }
+  for (int k = 2; k <= npad; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1) bitonic_smem_step(keys, npad, k, j);
+}
+
+// The prologue of every NMS kernel: keys[0..n) hold sort_key of the rows and are visible to the CTA.  Pads the keys to
+// npad, sorts them and fills s.box[r] = box_of(row_of(s, r)) for every sorted rank r < n.
+template <class BoxFn>
+__device__ inline void sort_and_gather(const NmsSmem& s, int n, BoxFn box_of) {
+  const int npad = next_pow2(max(n, 64));
+  for (int i = n + threadIdx.x; i < npad; i += blockDim.x) s.keys[i] = ~0ull;
+  __syncthreads();
+  bitonic_sort(s.keys, npad);
+  for (int r = threadIdx.x; r < n; r += blockDim.x) s.box[r] = box_of(row_of(s, r));
+  __syncthreads();
 }
 
 // barrier over the CTA (S == 1) or over the whole cluster, with release / acquire of shared-memory writes
@@ -364,9 +396,6 @@ __device__ inline int greedy_sweep(const NmsSmem& s, int n, float thr_f, int lim
     PROF_T(t3);
     if (s.scalars[1] || c + 2 >= nchunks) break;
     const int nk = s.scalars[2];
-#ifdef FOD_NMS_DBG
-    if (tid == 0 && blockIdx.x == 0) printf("pair c=%d base=%d nk=%d nal=%d kept=%d cross=%08x %08x\n", c, base, nk, s.scalars[3], s.scalars[0], csup[4], csup[5]);
-#endif
     // 1'. the next pair's first bit matrix (independent of the suppression state, so it shares this all-warps phase)
     build_colmask(c + 2);
     PROF_ADD(14, t3);
@@ -492,35 +521,22 @@ nms_proposals_kernel(const float* __restrict__ boxes, const float* __restrict__ 
   const int tid = threadIdx.x;
   int n = count ? count[p] : cand_cap;
   n = max(0, min(n, cand_cap));
+  PROF_DECL;
   PROF_T(tk0);
   NmsSmem s = carve(smem_raw, cand_cap);
   const float* pb = boxes + (size_t)p * cand_cap * 4;
   const float* ps = scores + (size_t)p * cand_cap;
-  const int npad = next_pow2(max(n, 64));
-  for (int i = tid; i < npad; i += blockDim.x) {
-    unsigned long long k = ~0ull;
-    if (i < n) k = ((unsigned long long)(~float_to_ordered(ps[i])) << 32) | (unsigned)i;
-    s.keys[i] = k;
-  }
-  __syncthreads();
-  bitonic_sort(s.keys, npad);
-  for (int r = tid; r < n; r += blockDim.x) {
-    int idx = (int)(s.keys[r] & 0xffffffffu);
-    s.box[r] = *reinterpret_cast<const float4*>(pb + (size_t)idx * 4);
-  }
-  __syncthreads();
+  for (int i = tid; i < n; i += blockDim.x) s.keys[i] = sort_key(ps[i], i);
+  sort_and_gather(s, n, [&](int row) { return *reinterpret_cast<const float4*>(pb + (size_t)row * 4); });
+  // row_of written out: through the call this kernel compiles differently (6344 instead of 6328 SASS instructions,
+  // CUDA 12.9), and the one-warp resolve that reads this score was 1 % slower (B200, 1000 W)
   auto score_of_rank = [&](int r) { return ps[(int)(s.keys[r] & 0xffffffffu)]; };
-#ifdef FOD_NMS_PROF
-  if (threadIdx.x == 0 && blockIdx.x == 0) g_nms_prof[6] += clock64() - tk0;
-#endif
+  PROF_ADD(6, tk0);
   PROF_T(tk1);
   int kept = greedy_sweep(s, n, thr_f, post_topk, true, score_of_rank, S, rank);
-#ifdef FOD_NMS_PROF
-  if (threadIdx.x == 0 && blockIdx.x == 0) g_nms_prof[7] += clock64() - tk1;
-#endif
-#ifdef FOD_NMS_PROF
-  if (threadIdx.x == 0 && blockIdx.x == 0) g_nms_prof[8] += kept;
-#endif
+  PROF_ADD(7, tk1);
+  PROF_CNT(8, kept);
+  PROF_FLUSH(6, 9);
   int m = kept;
   if (post_topk > 0 && kept > post_topk) {
     // keep every survivor whose score >= the post_topk-th best (fsod_rpn.py:1198-1206)
@@ -543,7 +559,7 @@ nms_proposals_kernel(const float* __restrict__ boxes, const float* __restrict__ 
   }
   for (int i = tid; i < m; i += blockDim.x) {
     int r = s.kept[i];
-    int idx = (int)(s.keys[r] & 0xffffffffu);
+    int idx = row_of(s, r);
     keep[(size_t)p * roi_cap + i] = idx;
     *reinterpret_cast<float4*>(out_boxes + ((size_t)p * roi_cap + i) * 4) = s.box[r];
     out_scores[(size_t)p * roi_cap + i] = ps[idx];
@@ -554,51 +570,23 @@ nms_proposals_kernel(const float* __restrict__ boxes, const float* __restrict__ 
 // ------------------------------------------------------------------------------------------------
 // R4 / N1 / O1: final class-wise NMS + postprocess, one CTA per image
 // ------------------------------------------------------------------------------------------------
-// Exclusive scan of one int per thread over the CTA (blockDim.x == 1024).  *total gets the sum.
-__device__ inline int block_exclusive_scan(int v, int* warp_sums, int* total) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int x = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    int y = __shfl_up_sync(0xffffffffu, x, o);
-    if (lane >= o) x += y;
-  }
-  if (lane == 31) warp_sums[warp] = x;
-  __syncthreads();
-  if (warp == 0) {
-    int w = warp_sums[lane];
-    int xs = w;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      int y = __shfl_up_sync(0xffffffffu, xs, o);
-      if (lane >= o) xs += y;
-    }
-    warp_sums[lane] = xs - w;
-    if (lane == 31) *total = xs;
-  }
-  __syncthreads();
-  int res = warp_sums[warp] + x - v;
-  __syncthreads();  // warp_sums may be rewritten by the next call; *total stays valid until then
-  return res;
-}
-
-// Shared tail of fod_final_detect / fod_batched_nms.
-//   row ids in the low key bits address `boxes4` / `scores` / `cls_of_row`.
-struct RowSource {
-  const float* boxes;     // [rows][4]
-  const float* scores;    // [rows]
-  const int64_t* idxs;    // per-row class (generic op) or NULL
-  int roi_cap;            // class = row / roi_cap when idxs == NULL and roi_cap > 0
-};
-
 __device__ __forceinline__ float4 clip_box(float4 b, float w, float h) {
   return make_float4(fminf(fmaxf(b.x, 0.f), w), fminf(fmaxf(b.y, 0.f), h), fminf(fmaxf(b.z, 0.f), w),
                      fminf(fmaxf(b.w, 0.f), h));
 }
 
-__device__ inline int class_of(const RowSource& src, int row) {
-  if (src.idxs) return (int)src.idxs[row];
-  return src.roi_cap > 0 ? row / src.roi_cap : 0;
+__device__ __forceinline__ float max_coord(float4 b) { return fmaxf(fmaxf(b.x, b.y), fmaxf(b.z, b.w)); }
+
+// Class offset step of torchvision's coordinate trick (boxes.py batched_nms): boxes.max() + 1 over the CTA, from each
+// thread's maximum over its boxes.  sh: __shared__ float[32]
+__device__ inline float coord_step(float lmax, float* sh) {
+  return __fadd_rn(block_reduce(lmax, sh, [](float a, float b) { return fmaxf(a, b); }), 1.0f);
+}
+
+// box + cls * coord_step on every coordinate, each operation separately rounded like the fp32 tensor ops it restates
+__device__ __forceinline__ float4 offset_box(float4 b, float cls, float coord_step) {
+  const float off = __fmul_rn(cls, coord_step);
+  return make_float4(__fadd_rn(b.x, off), __fadd_rn(b.y, off), __fadd_rn(b.z, off), __fadd_rn(b.w, off));
 }
 
 __global__ void __launch_bounds__(kNmsThreads, 1)
@@ -609,9 +597,8 @@ final_detect_kernel(const float* __restrict__ det_boxes, const float* __restrict
                     int64_t* __restrict__ out_rows, int32_t* __restrict__ out_count, uint32_t* __restrict__ status,
                     const int S) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  __shared__ int warp_sums[32];
-  __shared__ int sh_total;
-  __shared__ float sh_red[32];
+  __shared__ int sh_scan[33];
+  __shared__ float sh_max[32];
   const int b = blockIdx.x / S, rank = blockIdx.x - b * S;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   NmsSmem s = carve(smem_raw, ncap);
@@ -624,7 +611,6 @@ final_detect_kernel(const float* __restrict__ det_boxes, const float* __restrict
   // 1. compaction of valid rows in class-major order (d2 fast_rcnn.py:137-155)
   int n = 0;
   float lmax = -INFINITY;
-  bool overflow = false;
   for (int start = 0; start < total_rows; start += blockDim.x) {
     int row = start + tid;
     bool ok = false;
@@ -637,56 +623,25 @@ final_detect_kernel(const float* __restrict__ det_boxes, const float* __restrict
         float4 bx = *reinterpret_cast<const float4*>(ib + (size_t)row * 4);
         bool fin = isfinite(bx.x) && isfinite(bx.y) && isfinite(bx.z) && isfinite(bx.w) && isfinite(sc);
         ok = fin && (sc > score_thresh);
-        if (ok) {
-          bx = clip_box(bx, fw, fh);
-          lmax = fmaxf(lmax, fmaxf(fmaxf(bx.x, bx.y), fmaxf(bx.z, bx.w)));
-        }
+        if (ok) lmax = fmaxf(lmax, max_coord(clip_box(bx, fw, fh)));
       }
     }
-    int pos = block_exclusive_scan(ok ? 1 : 0, warp_sums, &sh_total);
-    int tot = sh_total;
-    if (ok) {
-      int i = n + pos;
-      if (i < ncap) s.keys[i] = ((unsigned long long)(~float_to_ordered(sc)) << 32) | (unsigned)row;
-    }
+    int tot;
+    const int i = n + block_exclusive_scan(ok ? 1 : 0, sh_scan, tot);
+    if (ok && i < ncap) s.keys[i] = sort_key(sc, row);
     n += tot;
-    __syncthreads();
   }
   if (n > ncap) {
-    overflow = true;
+    if (tid == 0 && rank == 0) atomicOr(status, FOD_STATUS_DET_OVERFLOW);
     n = ncap;
   }
-  if (overflow && tid == 0 && rank == 0) atomicOr(status, FOD_STATUS_DET_OVERFLOW);
-  // 2. max coordinate (torchvision boxes.py batched_nms: boxes.max())
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) lmax = fmaxf(lmax, __shfl_xor_sync(0xffffffffu, lmax, o));
-  if (lane == 0) sh_red[warp] = lmax;
-  __syncthreads();
-  if (warp == 0) {
-    float v = sh_red[lane];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    if (lane == 0) sh_red[0] = v;
-  }
-  __syncthreads();
-  const float coord_step = __fadd_rn(sh_red[0], 1.0f);
-  // 3. sort, gather class-offset boxes
-  const int npad = next_pow2(max(n, 64));
-  for (int i = n + tid; i < npad; i += blockDim.x) s.keys[i] = ~0ull;
-  __syncthreads();
-  bitonic_sort(s.keys, npad);
-  for (int r = tid; r < n; r += blockDim.x) {
-    int row = (int)(s.keys[r] & 0xffffffffu);
-    float4 bx = clip_box(*reinterpret_cast<const float4*>(ib + (size_t)row * 4), fw, fh);
-    float off = __fmul_rn((float)(row / roi_cap), coord_step);
-    bx.x = __fadd_rn(bx.x, off);
-    bx.y = __fadd_rn(bx.y, off);
-    bx.z = __fadd_rn(bx.z, off);
-    bx.w = __fadd_rn(bx.w, off);
-    s.box[r] = bx;
-  }
-  __syncthreads();
-  auto score_of_rank = [&](int r) { return is[(int)(s.keys[r] & 0xffffffffu)]; };
+  // 2. max coordinate (torchvision boxes.py batched_nms: boxes.max()); 3. sort, gather clipped class-offset boxes
+  const float step = coord_step(lmax, sh_max);
+  sort_and_gather(s, n, [&](int row) {
+    const float4 bx = clip_box(*reinterpret_cast<const float4*>(ib + (size_t)row * 4), fw, fh);
+    return offset_box(bx, (float)(row / roi_cap), step);
+  });
+  auto score_of_rank = [&](int r) { return is[row_of(s, r)]; };
   int kept = greedy_sweep(s, n, thr_f, max_det, false, score_of_rank, S, rank);
   if (max_det >= 0) kept = min(kept, max_det);
   // 4. detector_postprocess on the survivors (d2 postprocessing.py:42-59), order preserved.
@@ -700,7 +655,7 @@ final_detect_kernel(const float* __restrict__ det_boxes, const float* __restrict
       float4 bx = make_float4(0, 0, 0, 0);
       int row = 0;
       if (i < kept) {
-        row = (int)(s.keys[s.kept[i]] & 0xffffffffu);
+        row = row_of(s, s.kept[i]);
         bx = clip_box(*reinterpret_cast<const float4*>(ib + (size_t)row * 4), fw, fh);
         bx.x = fminf(fmaxf(__fmul_rn(bx.x, sx), 0.f), (float)ow);
         bx.z = fminf(fmaxf(__fmul_rn(bx.z, sx), 0.f), (float)ow);
@@ -728,62 +683,25 @@ __global__ void __launch_bounds__(kNmsThreads, 1)
 batched_nms_kernel(const float* __restrict__ boxes, const float* __restrict__ scores, const int64_t* __restrict__ idxs,
                    int n, float thr_f, int64_t* __restrict__ keep, int32_t* __restrict__ keep_count, const int S) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  __shared__ float sh_red[32];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  __shared__ float sh_max[32];
+  const int tid = threadIdx.x;
   const int rank = blockIdx.x;   // one problem = one cluster of S CTAs
   NmsSmem s = carve(smem_raw, n);
-  const int npad = next_pow2(max(n, 64));
   float lmax = -INFINITY;
-  for (int i = tid; i < npad; i += blockDim.x) {
-    unsigned long long k = ~0ull;
-    if (i < n) {
-      k = ((unsigned long long)(~float_to_ordered(scores[i])) << 32) | (unsigned)i;
-      float4 bx = *reinterpret_cast<const float4*>(boxes + (size_t)i * 4);
-      lmax = fmaxf(lmax, fmaxf(fmaxf(bx.x, bx.y), fmaxf(bx.z, bx.w)));
-    }
-    s.keys[i] = k;
+  for (int i = tid; i < n; i += blockDim.x) {
+    s.keys[i] = sort_key(scores[i], i);
+    lmax = fmaxf(lmax, max_coord(*reinterpret_cast<const float4*>(boxes + (size_t)i * 4)));
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) lmax = fmaxf(lmax, __shfl_xor_sync(0xffffffffu, lmax, o));
-  if (lane == 0) sh_red[warp] = lmax;
-  __syncthreads();
-  if (warp == 0) {
-    float v = sh_red[lane];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    if (lane == 0) sh_red[0] = v;
-  }
-  __syncthreads();
-  const float coord_step = __fadd_rn(sh_red[0], 1.0f);
-  bitonic_sort(s.keys, npad);
-  for (int r = tid; r < n; r += blockDim.x) {
-    int i = (int)(s.keys[r] & 0xffffffffu);
-    float4 bx = *reinterpret_cast<const float4*>(boxes + (size_t)i * 4);
-    if (idxs) {
-      float off = __fmul_rn((float)idxs[i], coord_step);
-      bx.x = __fadd_rn(bx.x, off);
-      bx.y = __fadd_rn(bx.y, off);
-      bx.z = __fadd_rn(bx.z, off);
-      bx.w = __fadd_rn(bx.w, off);
-    }
-    s.box[r] = bx;
-  }
-  __syncthreads();
-  auto score_of_rank = [&](int r) { return scores[(int)(s.keys[r] & 0xffffffffu)]; };
+  const float step = coord_step(lmax, sh_max);
+  sort_and_gather(s, n, [&](int i) {
+    const float4 bx = *reinterpret_cast<const float4*>(boxes + (size_t)i * 4);
+    return idxs ? offset_box(bx, (float)idxs[i], step) : bx;
+  });
+  auto score_of_rank = [&](int r) { return scores[row_of(s, r)]; };
   int kept = greedy_sweep(s, n, thr_f, 0, false, score_of_rank, S, rank);
   if (rank != 0) return;
-  for (int i = tid; i < kept; i += blockDim.x) keep[i] = (int64_t)(s.keys[s.kept[i]] & 0xffffffffu);
+  for (int i = tid; i < kept; i += blockDim.x) keep[i] = row_of(s, s.kept[i]);
   if (tid == 0) *keep_count = kept;
-}
-
-template <typename K>
-static int set_smem(K kernel, size_t bytes, const char* name) {
-  if (bytes > 227 * 1024) {
-    set_error("%s: needs %zu bytes of shared memory (> 227 KB)", name, bytes);
-    return FOD_ERR_CAPACITY;
-  }
-  FOD_CUDA_CALL(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-  return FOD_OK;
 }
 
 // CTAs per problem: the largest power of two <= kMaxCluster that keeps problems * S within the SM count.
@@ -794,28 +712,6 @@ static int pick_cluster(long problems) {
   if (const char* e = getenv("FOD_NMS_MAX_CLUSTER")) smax = atoi(e) > 0 ? atoi(e) : smax;   // development knob
   while (S * 2 <= smax && problems * (S * 2) <= sms) S *= 2;
   return S;
-}
-
-template <typename K, typename... Args>
-static int launch_clustered(const char* name, K kernel, long problems, int S, size_t smem, cudaStream_t stream, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(problems * S));
-  cfg.blockDim = dim3(kNmsThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = (unsigned)S;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, args...);
-  if (e != cudaSuccess) {
-    set_error("%s: launch failed: %s", name, cudaGetErrorString(e));
-    return FOD_ERR_CUDA;
-  }
-  return FOD_OK;
 }
 
 }  // namespace fod
@@ -845,12 +741,12 @@ extern "C" int fod_nms_proposals(const float* boxes, const float* scores, const 
     return FOD_ERR_CAPACITY;
   }
   if (num_problems == 0) return FOD_OK;
-  size_t smem = nms_smem_bytes(cand_cap);
-  int rc = set_smem(nms_proposals_kernel, smem, "fod_nms_proposals");
-  if (rc != FOD_OK) return rc;
-  return launch_clustered("fod_nms_proposals", nms_proposals_kernel, num_problems, pick_cluster(num_problems), smem,
-                          as_stream(stream), boxes, scores, count, cand_cap, iou_threshold_as_float(iou_thresh), post_topk,
-                          roi_cap, keep, out_boxes, out_scores, out_count, status, pick_cluster(num_problems));
+  float thr_f = iou_threshold_as_float(iou_thresh);
+  int S = pick_cluster(num_problems);
+  void* args[] = {&boxes, &scores, &count, &cand_cap, &thr_f, &post_topk, &roi_cap, &keep, &out_boxes, &out_scores,
+                  &out_count, &status, &S};
+  return launch_clusters((const void*)nms_proposals_kernel, args, num_problems, S, kNmsThreads, nms_smem_bytes(cand_cap),
+                         stream, "fod_nms_proposals");
 }
 
 extern "C" int fod_final_detect(const float* det_boxes, const float* det_scores, const int32_t* roi_count, int batch,
@@ -864,14 +760,13 @@ extern "C" int fod_final_detect(const float* det_boxes, const float* det_scores,
   if (batch == 0) return FOD_OK;
   long rows = (long)problems_per_image * roi_cap;
   int ncap = (int)(rows < FOD_NMS_MAX_BOXES ? rows : FOD_NMS_MAX_BOXES);
-  size_t smem = nms_smem_bytes(ncap);
-  int rc = set_smem(final_detect_kernel, smem, "fod_final_detect");
-  if (rc != FOD_OK) return rc;
+  float thr_f = iou_threshold_as_float(iou_thresh);
   // rows per image decide how far a problem is spread: a few hundred rows are a handful of chunks, not worth a cluster
-  const int S = rows > 1024 ? pick_cluster(batch) : 1;
-  return launch_clustered("fod_final_detect", final_detect_kernel, batch, S, smem, as_stream(stream), det_boxes, det_scores,
-                          roi_count, problems_per_image, roi_cap, ncap, score_thresh, iou_threshold_as_float(iou_thresh),
-                          max_det, image_hw, out_hw, out_boxes, out_scores, out_classes, out_rows, out_count, status, S);
+  int S = rows > 1024 ? pick_cluster(batch) : 1;
+  void* args[] = {&det_boxes, &det_scores, &roi_count, &problems_per_image, &roi_cap, &ncap, &score_thresh, &thr_f,
+                  &max_det, &image_hw, &out_hw, &out_boxes, &out_scores, &out_classes, &out_rows, &out_count, &status, &S};
+  return launch_clusters((const void*)final_detect_kernel, args, batch, S, kNmsThreads, nms_smem_bytes(ncap), stream,
+                         "fod_final_detect");
 }
 
 extern "C" int fod_batched_nms(const float* boxes, const float* scores, const int64_t* idxs, int n, double iou_thresh,
@@ -887,10 +782,9 @@ extern "C" int fod_batched_nms(const float* boxes, const float* scores, const in
     return FOD_OK;
   }
   FOD_REQUIRE(boxes && scores && keep, "fod_batched_nms: null pointer");
-  size_t smem = nms_smem_bytes(n);
-  int rc = set_smem(batched_nms_kernel, smem, "fod_batched_nms");
-  if (rc != FOD_OK) return rc;
-  const int S = n > 512 ? kMaxCluster : 1;
-  return launch_clustered("fod_batched_nms", batched_nms_kernel, 1, S, smem, as_stream(stream), boxes, scores, idxs, n,
-                          iou_threshold_as_float(iou_thresh), keep, keep_count, S);
+  float thr_f = iou_threshold_as_float(iou_thresh);
+  int S = n > 512 ? pick_cluster(1) : 1;
+  void* args[] = {&boxes, &scores, &idxs, &n, &thr_f, &keep, &keep_count, &S};
+  return launch_clusters((const void*)batched_nms_kernel, args, 1, S, kNmsThreads, nms_smem_bytes(n), stream,
+                         "fod_batched_nms");
 }

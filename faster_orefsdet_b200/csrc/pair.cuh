@@ -2,7 +2,8 @@
 // correlate_tc.cu: correlate_tc_kernel, relation_tc.cu: relation_tc_kernel).  Two CTAs form a cluster and share one
 // cta_group::2 MMA issued by the leader (rank 0); the MMA warp walks its rings by a running index, a watcher thread does
 // all the barrier waiting for it, and the epilogue warps of both CTAs hand every accumulator stage back to the leader.
-// A copy of one of these rules that drifts from the others hangs the pair, so each is written once, here.
+// A copy of one of these rules that drifts from the others hangs the pair, so each is written once, here.  The host
+// launches them through launch_clusters (common.cuh) with a cluster size of 2.
 #pragma once
 #include "common.cuh"
 #include "tc05.cuh"
@@ -79,31 +80,6 @@ inline int pair_count(long units, int* pairs) {
   FOD_CUDA_CALL(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const int max_pairs = sms / 2 > 0 ? sms / 2 : 1;
   *pairs = units < max_pairs ? (int)units : max_pairs;
-  return FOD_OK;
-}
-
-// Launches `kernel` on `pairs` clusters of two CTAs of `threads` threads and smem_bytes of dynamic shared memory;
-// `name` prefixes the error message
-inline int launch_pairs(const void* kernel, void** args, int pairs, int threads, uint32_t smem_bytes, fod_stream_t stream,
-                        const char* name) {
-  FOD_CUDA_CALL(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * pairs);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem_bytes;
-  cfg.stream = as_stream(stream);
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  const cudaError_t e = cudaLaunchKernelExC(&cfg, kernel, args);
-  if (e != cudaSuccess) {
-    set_error("%s: launch failed: %s", name, cudaGetErrorString(e));
-    return FOD_ERR_CUDA;
-  }
   return FOD_OK;
 }
 

@@ -461,6 +461,6 @@ extern "C" int fod_relation_head(const float* pooled, const float* x_amax, int n
   rc = pair_count((total_slots + 1) / 2, &prm.num_pairs);
   if (rc != FOD_OK) return rc;
   void* args[] = {&prm};
-  return launch_pairs((const void*)rtc::relation_tc_kernel, args, prm.num_pairs, rtc::kThreads, rtc::kSmemAlloc, stream,
-                      "fod_relation_head");
+  return launch_clusters((const void*)rtc::relation_tc_kernel, args, prm.num_pairs, 2, rtc::kThreads, rtc::kSmemAlloc,
+                         stream, "fod_relation_head");
 }

@@ -63,15 +63,19 @@ def test_batched_nms_all_equal_scores_and_identical_boxes():
 def test_nms_every_cluster_size(max_cluster, monkeypatch):
     """One, two and four CTAs per problem run the same sweep on differently split data (own suppression words, exchanged
     chunk pairs, shared survivor / alive-list array): each must reproduce the oracle on a full sweep without early stop
-    (3000 candidates, almost nothing suppressed at first) and on the duplicated-box list."""
+    (3000 candidates, almost nothing suppressed at first), on the duplicated-box list, with and without classes, and in
+    the class-wise final NMS.  batched_nms uses a cluster above 512 rows, final_detect above 1024 rows per image."""
     monkeypatch.setenv("FOD_NMS_MAX_CLUSTER", str(max_cluster))
-    n = 500
-    boxes = _boxes(n, 77)
-    boxes[250:] = boxes[:250]
-    scores = torch.full((n,), 0.5)
-    ref = O.batched_nms_coordinate_trick(boxes, scores, torch.zeros(n, dtype=torch.long), 0.6)
-    got = ops.batched_nms(boxes.to(DEV), scores.to(DEV), None, 0.6)
-    assert np.array_equal(got.cpu().numpy(), ref.numpy())
+    for n in (500, 1000):
+        boxes = _boxes(n, 77)
+        boxes[n // 2:] = boxes[:n // 2]
+        scores = torch.full((n,), 0.5)
+        classes = [None] if n == 500 else [None, (synth.tensor((n,), 78, 0.0, 1.0) * 3).long()]
+        for idxs in classes:
+            ref = O.batched_nms_coordinate_trick(boxes, scores, torch.zeros(n, dtype=torch.long) if idxs is None else idxs, 0.6)
+            got = ops.batched_nms(boxes.to(DEV), scores.to(DEV), None if idxs is None else idxs.to(DEV), 0.6)
+            assert np.array_equal(got.cpu().numpy(), ref.numpy()), (n, idxs is None)
+    _check_final_detect(10, 320)      # 3 200 rows per image
     cap = 3000
     pb = _boxes(cap, 300, 30.0, 600.0, 20.0, 60.0).unsqueeze(0)
     ps = synth.tensor((cap,), 301, 0.01, 1.0).unsqueeze(0)
@@ -580,8 +584,8 @@ def test_relation_head_ten_classes_per_class_bias():
 
 
 # ----------------------------------------------------------------------------------------- final detect
-@pytest.mark.parametrize("C,cap", [(1, 64), (3, 64), (10, 320)])
-def test_final_detect_bit_exact(C, cap):
+def _check_final_detect(C, cap):
+    """final_detect on three images of C problems of up to `cap` rows each, bit-exact against the oracle."""
     B = 3
     P = B * C
     boxes = _boxes(P * cap, 300, 10.0, 300.0, 10.0, 120.0).reshape(P, cap, 4)      # some stick out of the image
@@ -615,6 +619,11 @@ def test_final_detect_bit_exact(C, cap):
             assert np.array_equal(ob[b, :m].cpu().numpy(), pb.numpy())
             assert np.array_equal(os_[b, :m].cpu().numpy(), ps.numpy())
             assert np.array_equal(ocls[b, :m].cpu().numpy(), pc.numpy())
+
+
+@pytest.mark.parametrize("C,cap", [(1, 64), (3, 64), (10, 320)])
+def test_final_detect_bit_exact(C, cap):
+    _check_final_detect(C, cap)
 
 
 def test_final_detect_golden_reference():
