@@ -45,6 +45,9 @@ _PROTOTYPES = {
                               ctypes.POINTER(_f), _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
     "fod_decode_topk_taps_workspace_bytes": ([ctypes.POINTER(fod_level_t), _i, _i], ctypes.c_size_t),
     "fod_nms_proposals": ([_vp, _vp, _vp, _i, _i, _d, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp], _i),
+    "fod_rpn_proposals_workspace_bytes": ([ctypes.POINTER(fod_level_t), _i, _i, _i, _i], ctypes.c_size_t),
+    "fod_rpn_proposals": ([ctypes.POINTER(_vp), ctypes.POINTER(_i), ctypes.POINTER(_vp), ctypes.POINTER(fod_level_t), _i, _i, _i,
+                           _vp, _i, ctypes.POINTER(_f), _f, _d, _i, _vp, _vp, _vp, _vp, _vp], _i),
     "fod_roi_align_workspace_bytes": ([_i, _i, _i], ctypes.c_size_t),
     "fod_roi_align": ([ctypes.POINTER(_vp), ctypes.POINTER(fod_level_t), _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp],
                       _i),

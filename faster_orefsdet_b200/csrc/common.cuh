@@ -129,6 +129,81 @@ __device__ inline int block_exclusive_scan(int v, int* sh, int& total) {
   return res;
 }
 
+// Radix select of a 1024-thread CTA: the k-th largest of the n keys key_at(0..n-1) (k <= n) as T, and in `need` how many
+// keys equal to T belong to the k largest.  MSB-first, 8 bits per pass; warp-aggregated shared atomics into per-warp
+// histograms hist[32][256]; sh: __shared__ int[2].  Every thread of the CTA calls it and gets the same (T, need).
+template <class KeyAt>
+__device__ inline uint32_t radix_select(KeyAt key_at, int n, int k, int (*hist)[256], int* sh, int& need) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  constexpr int kWarps = 32;
+  uint32_t prefix = 0u, mask = 0u;
+  int remaining = k;
+  for (int shift = 24; shift >= 0; shift -= 8) {
+    for (int i = tid; i < kWarps * 256; i += 1024) (&hist[0][0])[i] = 0;
+    __syncthreads();
+    for (int i0 = 0; i0 < n; i0 += 1024) {
+      int i = i0 + tid;
+      bool act = false;
+      int bin = 0;
+      if (i < n) {
+        uint32_t key = key_at(i);
+        act = (key & mask) == prefix;
+        bin = (key >> shift) & 255;
+      }
+      unsigned am = __ballot_sync(0xffffffffu, act);
+      if (act) {
+        unsigned peers = __match_any_sync(am, bin);
+        if (lane == __ffs(peers) - 1) hist[warp][bin] += __popc(peers);
+      }
+      __syncwarp();
+    }
+    __syncthreads();
+    // column sums over the per-warp histograms, then a top-down scan by warp 0
+    if (tid < 256) {
+      int sum = 0;
+#pragma unroll 8
+      for (int w = 0; w < kWarps; ++w) sum += hist[w][tid];
+      hist[0][tid] = sum;
+    }
+    __syncthreads();
+    if (warp == 0) {
+      // lane handles bins [lane*8, lane*8+8); suffix sums from the top
+      int c[8], tot = 0;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        c[j] = hist[0][lane * 8 + j];
+        tot += c[j];
+      }
+      int x = tot;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        int y = __shfl_down_sync(0xffffffffu, x, o);
+        if (lane + o < 32) x += y;
+      }
+      const int above = x - tot;  // elements in lanes above this one
+      // the digit d is the highest bin with (count of bins >= d) >= remaining
+      if (above < remaining && above + tot >= remaining) {
+        int acc = above;
+        for (int j = 7; j >= 0; --j) {
+          if (acc + c[j] >= remaining) {
+            sh[0] = lane * 8 + j;
+            sh[1] = remaining - acc;
+            break;
+          }
+          acc += c[j];
+        }
+      }
+    }
+    __syncthreads();
+    prefix |= (uint32_t)sh[0] << shift;
+    mask |= 255u << shift;
+    remaining = sh[1];
+    __syncthreads();
+  }
+  need = remaining;
+  return prefix;
+}
+
 // Launches `kernel` on `clusters` clusters of `cluster_size` CTAs of `threads` threads with `smem_bytes` of dynamic
 // shared memory (also set as the kernel's limit).  args[i] points at a local of exactly the type of parameter i; `name`
 // prefixes the error message

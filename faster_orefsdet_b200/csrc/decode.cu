@@ -102,7 +102,7 @@ decode_topk_kernel(DecodeParams prm, float* __restrict__ boxes, float* __restric
   const int roles = min(prm.num_levels, 2);
   const int p = blockIdx.x / roles, role = blockIdx.x - p * roles;
   const int l_begin = role == 0 ? 0 : 1, l_end = (role == 0 && roles == 2) ? 1 : prm.num_levels;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   auto block_sum = [&](int local) { return block_reduce(local, warp_sums, [](int a, int b) { return a + b; }); };
   // key of pixel i of level ll: fp32 bits of the probability if it passes the threshold, else 0
   auto key_of = [&](int ll, int i) -> uint32_t {
@@ -133,75 +133,7 @@ decode_topk_kernel(DecodeParams prm, float* __restrict__ boxes, float* __restric
     const int cnt = block_sum(local);
     uint32_t T = 0u;   // select keys > T plus the first `need` keys == T
     int need = 0;
-    if (cnt > prm.pre_topk) {
-      uint32_t prefix = 0u, mask = 0u;
-      int remaining = prm.pre_topk;
-      for (int shift = 24; shift >= 0; shift -= 8) {
-        for (int i = tid; i < kDecWarps * 256; i += kDecThreads) (&hist[0][0])[i] = 0;
-        __syncthreads();
-        for (int i0 = 0; i0 < n; i0 += kDecThreads) {
-          int i = i0 + tid;
-          bool act = false;
-          int bin = 0;
-          if (i < n) {
-            uint32_t k = keys[i];
-            act = (k & mask) == prefix;
-            bin = (k >> shift) & 255;
-          }
-          unsigned am = __ballot_sync(0xffffffffu, act);
-          if (act) {
-            unsigned peers = __match_any_sync(am, bin);
-            if (lane == __ffs(peers) - 1) hist[warp][bin] += __popc(peers);
-          }
-          __syncwarp();
-        }
-        __syncthreads();
-        // column sums over the per-warp histograms, then a top-down scan by warp 0
-        if (tid < 256) {
-          int sum = 0;
-#pragma unroll 8
-          for (int w = 0; w < kDecWarps; ++w) sum += hist[w][tid];
-          hist[0][tid] = sum;
-        }
-        __syncthreads();
-        if (warp == 0) {
-          // lane handles bins [lane*8, lane*8+8); suffix sums from the top
-          int c[8], tot = 0;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            c[j] = hist[0][lane * 8 + j];
-            tot += c[j];
-          }
-          int above = 0;  // elements in lanes above this one
-          int x = tot;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            int y = __shfl_down_sync(0xffffffffu, x, o);
-            if (lane + o < 32) x += y;
-          }
-          above = x - tot;
-          // the digit d is the highest bin with (count of bins >= d) >= remaining
-          if (above < remaining && above + tot >= remaining) {
-            int acc = above;
-            for (int j = 7; j >= 0; --j) {
-              if (acc + c[j] >= remaining) {
-                sh[0] = lane * 8 + j;
-                sh[1] = remaining - acc;
-                break;
-              }
-              acc += c[j];
-            }
-          }
-        }
-        __syncthreads();
-        prefix |= (uint32_t)sh[0] << shift;
-        mask |= 255u << shift;
-        remaining = sh[1];
-        __syncthreads();
-      }
-      T = prefix;
-      need = remaining;
-    }
+    if (cnt > prm.pre_topk) T = radix_select([&](int i) { return keys[i]; }, n, prm.pre_topk, hist, sh, need);
     // ---- ordered emission
     const int nsel = min(cnt, prm.pre_topk);
     if (out_base + nsel > prm.cand_cap && tid == 0) atomicOr(status, FOD_STATUS_CAND_OVERFLOW);

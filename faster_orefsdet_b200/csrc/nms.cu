@@ -704,6 +704,159 @@ batched_nms_kernel(const float* __restrict__ boxes, const float* __restrict__ sc
   if (tid == 0) *keep_count = kept;
 }
 
+// ------------------------------------------------------------------------------------------------
+// N2: RPN proposals (find_top_rpn_proposals, d2!/modeling/proposal_generator/proposal_utils.py:19-119)
+//   rpn_keys_kernel   : the selection key of every anchor of every level (wide, over all SMs)
+//   rpn_select_kernel : one CTA per (problem, level): radix select of the level's top k, then the k anchors in ascending
+//                       anchor order are decoded, filtered and clipped into the level's k candidate slots
+//   rpn_nms_kernel    : one cluster per problem: the surviving candidates through sort_and_gather + greedy_sweep
+// ------------------------------------------------------------------------------------------------
+struct RpnParams {
+  const float* map[FOD_MAX_LEVELS];       // [P][H][W][ps]: logit of anchor a in channel a, delta j in channel A + 4a + j
+  const float* anchors[FOD_MAX_LEVELS];   // [H*W*A][4]
+  const int32_t* image_hw;                // [P][2]
+  int pixels[FOD_MAX_LEVELS], ps[FOD_MAX_LEVELS];
+  int key_off[FOD_MAX_LEVELS + 1];        // first key of level l in a problem's key row; key_off[L] = anchors per problem
+  int sel_off[FOD_MAX_LEVELS + 1];        // first candidate slot of level l; sel_off[L] = candidate slots per problem
+  int num_levels, A, pre_topk;
+  float inv_w[4];                         // 1 / BBOX_REG_WEIGHTS, rounded to fp32 like ATen's tensor / python-float
+  float scale_clamp;                      // log(1000 / 16) as fp32 (box_regression.py _DEFAULT_SCALE_CLAMP)
+  float min_size;
+};
+
+// Selection key: ascending key = ascending logit in the order of torch.sort, i.e. -0.0 equal to +0.0 and every NaN
+// above +inf
+__device__ __forceinline__ uint32_t rpn_key(float v) {
+  if (isnan(v)) return 0xffffffffu;
+  return float_to_ordered(v == 0.f ? 0.f : v);
+}
+
+// level of entry i of a row laid out by `off` (constant indices only: the parameter array stays in the constant bank)
+__device__ __forceinline__ int rpn_level_of(const int (&off)[FOD_MAX_LEVELS + 1], int L, int i) {
+  int l = 0;
+#pragma unroll
+  for (int j = 1; j < FOD_MAX_LEVELS; ++j) l += (j < L && i >= off[j]) ? 1 : 0;
+  return l;
+}
+
+__global__ void __launch_bounds__(256) rpn_keys_kernel(RpnParams prm, uint32_t* __restrict__ keys) {
+  const int idx = blockIdx.x * 256 + threadIdx.x, p = blockIdx.y;
+  const int total = prm.key_off[prm.num_levels];
+  if (idx >= total) return;
+  const int l = rpn_level_of(prm.key_off, prm.num_levels, idx);
+  const int i = idx - prm.key_off[l], pix = i / prm.A, a = i - pix * prm.A;
+  const float v = __ldg(prm.map[l] + ((size_t)p * prm.pixels[l] + pix) * prm.ps[l] + a);
+  keys[(size_t)p * total + idx] = rpn_key(v);
+}
+
+// Box2BoxTransform.apply_deltas (box_regression.py:77-115) of one anchor, with the roundings of its separate fp32 ATen ops
+__device__ __forceinline__ float4 rpn_decode(float4 an, float d0, float d1, float d2, float d3, const float* inv_w,
+                                             float clamp) {
+  const float w = __fsub_rn(an.z, an.x), h = __fsub_rn(an.w, an.y);
+  const float cx = __fadd_rn(an.x, __fmul_rn(0.5f, w)), cy = __fadd_rn(an.y, __fmul_rn(0.5f, h));
+  const float dx = __fmul_rn(d0, inv_w[0]), dy = __fmul_rn(d1, inv_w[1]);
+  float dw = __fmul_rn(d2, inv_w[2]), dh = __fmul_rn(d3, inv_w[3]);
+  dw = isnan(dw) ? dw : fminf(dw, clamp);      // torch.clamp(max=) lets NaN through
+  dh = isnan(dh) ? dh : fminf(dh, clamp);
+  const float pcx = __fadd_rn(__fmul_rn(dx, w), cx), pcy = __fadd_rn(__fmul_rn(dy, h), cy);
+  const float pw = __fmul_rn(expf(dw), w), ph = __fmul_rn(expf(dh), h);
+  const float hw = __fmul_rn(0.5f, pw), hh = __fmul_rn(0.5f, ph);
+  return make_float4(__fsub_rn(pcx, hw), __fsub_rn(pcy, hh), __fadd_rn(pcx, hw), __fadd_rn(pcy, hh));
+}
+
+// A candidate slot whose logit is NaN holds a dropped row (non-finite box or logit, or empty after the clip)
+__global__ void __launch_bounds__(1024, 1)
+rpn_select_kernel(RpnParams prm, const uint32_t* __restrict__ keys, float4* __restrict__ cand_box,
+                  float* __restrict__ cand_logit) {
+  __shared__ int hist[32][256];
+  __shared__ int scan_sh[33];
+  __shared__ int sh[2];
+  const int L = prm.num_levels;
+  const int p = blockIdx.x / L, l = blockIdx.x - p * L;
+  const int tid = threadIdx.x;
+  const int A = prm.A, n = prm.key_off[l + 1] - prm.key_off[l], k = min(n, prm.pre_topk);
+  const uint32_t* lk = keys + (size_t)p * prm.key_off[L] + prm.key_off[l];
+  // keys > T, plus the first `need` keys == T (a stable descending sort takes the lowest anchor indices first)
+  uint32_t T = 0u;
+  int need = 0;
+  if (n > k) T = radix_select([&](int i) { return __ldg(lk + i); }, n, k, hist, sh, need);
+  const float fh = (float)prm.image_hw[2 * p], fw = (float)prm.image_hw[2 * p + 1];
+  const float* map = prm.map[l] + (size_t)p * prm.pixels[l] * prm.ps[l];
+  const float4* anc = reinterpret_cast<const float4*>(prm.anchors[l]);
+  float4* ob = cand_box + (size_t)p * prm.sel_off[L] + prm.sel_off[l];
+  float* ol = cand_logit + (size_t)p * prm.sel_off[L] + prm.sel_off[l];
+  int gt_before = 0, eq_before = 0;
+  for (int i0 = 0; i0 < n; i0 += 1024) {
+    const int i = i0 + tid;
+    const uint32_t key = i < n ? __ldg(lk + i) : 0u;
+    const int is_gt = i < n && key > T, is_eq = i < n && need > 0 && key == T;
+    int tot;   // both counts of the 1024 keys of this step in one scan (each <= 1024)
+    const int excl = block_exclusive_scan(is_gt | (is_eq << 16), scan_sh, tot);
+    const int gt_pos = gt_before + (excl & 0xffff), eq_pos = eq_before + (excl >> 16);
+    if (is_gt || (is_eq && eq_pos < need)) {
+      const int o = gt_pos + min(eq_pos, need);
+      const int pix = i / A, a = i - pix * A;
+      const float* px = map + (size_t)pix * prm.ps[l];
+      const float logit = __ldg(px + a);
+      const float* d = px + A + 4 * a;
+      const float4 b = rpn_decode(__ldg(anc + i), __ldg(d), __ldg(d + 1), __ldg(d + 2), __ldg(d + 3), prm.inv_w,
+                                     prm.scale_clamp);
+      bool ok = isfinite(b.x) && isfinite(b.y) && isfinite(b.z) && isfinite(b.w) && isfinite(logit);
+      const float4 c = clip_box(b, fw, fh);                                 // Boxes.clip
+      ok = ok && __fsub_rn(c.z, c.x) > prm.min_size && __fsub_rn(c.w, c.y) > prm.min_size;   // Boxes.nonempty
+      ob[o] = c;
+      ol[o] = ok ? logit : __int_as_float(0x7fffffff);
+    }
+    gt_before += tot & 0xffff;
+    eq_before += tot >> 16;
+  }
+}
+
+__global__ void __launch_bounds__(kNmsThreads, 1)
+rpn_nms_kernel(RpnParams prm, const float4* __restrict__ cand_box, const float* __restrict__ cand_logit, float thr_f,
+               int post_topk, float* __restrict__ out_boxes, float* __restrict__ out_logits, int32_t* __restrict__ out_count,
+               const int S) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ float sh_max[32];
+  const int L = prm.num_levels, cap = prm.sel_off[L];
+  const int p = blockIdx.x / S, rank = blockIdx.x - p * S;
+  const int tid = threadIdx.x;
+  NmsSmem s = carve(smem_raw, cap);
+  const float4* pb = cand_box + (size_t)p * cap;
+  const float* pl = cand_logit + (size_t)p * cap;
+  if (tid == 0) s.scalars[0] = 0;
+  __syncthreads();
+  // the surviving candidates as sort keys (any order: the slot index breaks ties), and their largest coordinate
+  float lmax = -INFINITY;
+  for (int i = tid; i < cap; i += blockDim.x) {
+    const float sc = pl[i];
+    if (!isnan(sc)) {
+      s.keys[atomicAdd(&s.scalars[0], 1)] = sort_key(sc, i);
+      lmax = fmaxf(lmax, max_coord(pb[i]));
+    }
+  }
+  __syncthreads();
+  const int n = s.scalars[0];
+  if (n == 0) {   // (the same in every CTA of the cluster)
+    if (rank == 0 && tid == 0) out_count[p] = 0;
+    return;
+  }
+  // batched_nms over the levels: torchvision's coordinate trick, as fod_batched_nms with idxs = level
+  const float step = L > 1 ? coord_step(lmax, sh_max) : 0.f;
+  sort_and_gather(s, n, [&](int i) {
+    return L > 1 ? offset_box(pb[i], (float)rpn_level_of(prm.sel_off, L, i), step) : pb[i];
+  });
+  auto score_of_rank = [&](int r) { return pl[row_of(s, r)]; };
+  const int m = min(greedy_sweep(s, n, thr_f, post_topk, false, score_of_rank, S, rank), post_topk);
+  if (rank != 0) return;
+  for (int i = tid; i < m; i += blockDim.x) {
+    const int row = row_of(s, s.kept[i]);
+    *reinterpret_cast<float4*>(out_boxes + ((size_t)p * post_topk + i) * 4) = pb[row];
+    out_logits[(size_t)p * post_topk + i] = pl[row];
+  }
+  if (tid == 0) out_count[p] = m;
+}
+
 // CTAs per problem: the largest power of two <= kMaxCluster that keeps problems * S within the SM count.
 static int pick_cluster(long problems) {
   int dev = 0, sms = 148;
@@ -787,4 +940,92 @@ extern "C" int fod_batched_nms(const float* boxes, const float* scores, const in
   void* args[] = {&boxes, &scores, &idxs, &n, &thr_f, &keep, &keep_count, &S};
   return launch_clusters((const void*)batched_nms_kernel, args, 1, S, kNmsThreads, nms_smem_bytes(n), stream,
                          "fod_batched_nms");
+}
+
+// Level geometry of fod_rpn_proposals: key and candidate-slot offsets; false if an anchor count overflows int
+static bool rpn_geometry(const fod_level_t* levels, int num_levels, int num_anchors, int pre_topk, int* key_off, int* sel_off) {
+  long keys = 0, sel = 0;
+  for (int l = 0; l < num_levels; ++l) {
+    key_off[l] = (int)keys;
+    sel_off[l] = (int)sel;
+    const long n = (long)levels[l].height * levels[l].width * num_anchors;
+    keys += n;
+    sel += n < pre_topk ? n : pre_topk;
+    if (keys >= (1L << 30)) return false;
+  }
+  key_off[num_levels] = (int)keys;
+  sel_off[num_levels] = (int)sel;
+  return true;
+}
+
+static size_t align16(size_t b) { return (b + 15) & ~(size_t)15; }
+
+// workspace: candidate boxes [P][slots] float4 | candidate logits [P][slots] | keys [P][anchors] uint32
+extern "C" size_t fod_rpn_proposals_workspace_bytes(const fod_level_t* levels, int num_levels, int num_problems,
+                                                   int num_anchors, int pre_topk) {
+  int key_off[FOD_MAX_LEVELS + 1], sel_off[FOD_MAX_LEVELS + 1];
+  if (!levels || num_levels < 1 || num_levels > FOD_MAX_LEVELS || num_problems <= 0 || num_anchors <= 0 || pre_topk <= 0 ||
+      !rpn_geometry(levels, num_levels, num_anchors, pre_topk, key_off, sel_off))
+    return 0;
+  const size_t P = (size_t)num_problems, slots = (size_t)sel_off[num_levels];
+  return P * slots * 16 + align16(P * slots * 4) + P * (size_t)key_off[num_levels] * 4;
+}
+
+extern "C" int fod_rpn_proposals(const float* const* maps, const int* pixel_stride, const float* const* anchors,
+                                 const fod_level_t* levels, int num_levels, int num_problems, int num_anchors,
+                                 const int32_t* image_hw, int pre_topk, const float* box_weights, float min_size,
+                                 double iou_thresh, int post_topk, float* out_boxes, float* out_logits, int32_t* out_count,
+                                 void* workspace, fod_stream_t stream) {
+  FOD_REQUIRE(maps && pixel_stride && anchors && levels && image_hw && box_weights && out_boxes && out_logits && out_count &&
+                  workspace,
+              "fod_rpn_proposals: null pointer");
+  FOD_REQUIRE(num_levels >= 1 && num_levels <= FOD_MAX_LEVELS, "fod_rpn_proposals: num_levels %d out of range", num_levels);
+  FOD_REQUIRE(num_problems >= 0 && num_anchors > 0 && pre_topk > 0 && post_topk > 0, "fod_rpn_proposals: bad sizes");
+  FOD_REQUIRE((reinterpret_cast<uintptr_t>(out_boxes) & 15) == 0 && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
+              "fod_rpn_proposals: out_boxes and workspace must be 16-byte aligned");
+  RpnParams prm = {};
+  for (int l = 0; l < num_levels; ++l) {
+    FOD_REQUIRE(maps[l] && anchors[l] && (reinterpret_cast<uintptr_t>(anchors[l]) & 15) == 0,
+                "fod_rpn_proposals: null or misaligned level pointer");
+    FOD_REQUIRE(levels[l].height > 0 && levels[l].width > 0, "fod_rpn_proposals: bad level %d", l);
+    FOD_REQUIRE(pixel_stride[l] >= 5 * num_anchors, "fod_rpn_proposals: pixel stride %d < 5 * %d channels at level %d",
+                pixel_stride[l], num_anchors, l);
+    prm.map[l] = maps[l];
+    prm.anchors[l] = anchors[l];
+    prm.pixels[l] = levels[l].height * levels[l].width;
+    prm.ps[l] = pixel_stride[l];
+  }
+  if (!rpn_geometry(levels, num_levels, num_anchors, pre_topk, prm.key_off, prm.sel_off)) {
+    set_error("fod_rpn_proposals: more than 2^30 anchors per problem");
+    return FOD_ERR_CAPACITY;
+  }
+  const int slots = prm.sel_off[num_levels];
+  if (slots > FOD_NMS_MAX_BOXES) {
+    set_error("fod_rpn_proposals: %d candidates per problem > %d", slots, FOD_NMS_MAX_BOXES);
+    return FOD_ERR_CAPACITY;
+  }
+  if (num_problems == 0) return FOD_OK;
+  prm.image_hw = image_hw;
+  prm.num_levels = num_levels;
+  prm.A = num_anchors;
+  prm.pre_topk = pre_topk;
+  for (int j = 0; j < 4; ++j) prm.inv_w[j] = 1.0f / (float)box_weights[j];
+  prm.scale_clamp = (float)log(1000.0 / 16);
+  prm.min_size = min_size;
+  const size_t P = (size_t)num_problems;
+  float4* cand_box = static_cast<float4*>(workspace);
+  float* cand_logit = reinterpret_cast<float*>(cand_box + P * slots);
+  uint32_t* keys = reinterpret_cast<uint32_t*>(reinterpret_cast<unsigned char*>(cand_logit) + align16(P * slots * 4));
+  const cudaStream_t st = as_stream(stream);
+  rpn_keys_kernel<<<dim3((unsigned)((prm.key_off[num_levels] + 255) / 256), (unsigned)num_problems), 256, 0, st>>>(prm, keys);
+  FOD_CUDA_LAUNCH_CHECK("fod_rpn_proposals (keys)");
+  rpn_select_kernel<<<num_problems * num_levels, 1024, 0, st>>>(prm, keys, cand_box, cand_logit);
+  FOD_CUDA_LAUNCH_CHECK("fod_rpn_proposals (select)");
+  float thr_f = iou_threshold_as_float(iou_thresh);
+  int S = slots > 512 ? pick_cluster(num_problems) : 1;
+  const float4* cb = cand_box;
+  const float* cl = cand_logit;
+  void* args[] = {&prm, &cb, &cl, &thr_f, &post_topk, &out_boxes, &out_logits, &out_count, &S};
+  return launch_clusters((const void*)rpn_nms_kernel, args, num_problems, S, kNmsThreads, nms_smem_bytes(slots), stream,
+                         "fod_rpn_proposals");
 }

@@ -39,9 +39,10 @@ __all__ = ["CenterNet2Detector"]
 
 
 class PendingBatch:
-    """A query batch that ``CenterNet2Detector.submit`` has put on the device: its host-to-device copies, the stem, the
-    graph replay and the device-to-host copy of the padded detections are all enqueued; ``model(pending)`` (or
-    ``collect``) waits for the one event and builds the ``Instances``.  Equivalent to calling ``model(inputs)``."""
+    """A query batch that ``submit`` (CenterNet2Detector or FsodRCNN) has put on the device: its host-to-device copies,
+    the forward and the device-to-host copy of the padded detections are all enqueued; ``model(pending)`` (or
+    ``collect``) waits for the one event and builds the ``Instances``.  Equivalent to calling ``model(inputs)``.
+    ``x_u8`` holds the device image batch (CenterNet2Detector: raw uint8; FsodRCNN: normalised and padded)."""
 
     __slots__ = ("inputs", "x_u8", "image_sizes", "out_sizes", "block", "host", "status_host", "done")
 

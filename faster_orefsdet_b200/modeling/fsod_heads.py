@@ -24,6 +24,11 @@ from .roi_heads import ROI_HEADS_REGISTRY
 from .rpn import apply_deltas
 
 
+def upload(values, dtype, device) -> torch.Tensor:
+    """A small host list on the device through a pinned, non-blocking copy (a pageable one synchronises the stream)."""
+    return torch.tensor(values, dtype=dtype).pin_memory().to(device, non_blocking=True)
+
+
 def positional_encoding(d_model: int, max_len: int) -> torch.Tensor:
     """PositionalEncoding.pe (fsod_fast_rcnn.py:687-697, fsod_rcnn.py:535-545): [1, max_len, d_model]."""
     pe = torch.zeros(max_len, d_model)
@@ -130,6 +135,16 @@ class FsodRes5ROIHeads(nn.Module):
                           support_embedded: List[Dict[str, torch.Tensor]], class_ids: Sequence[int]):
         """fsod_roi_heads.py:143-191 for a batch: proposals [B*C, cap, 4] (problem = image-major, class-minor), counts
         [B*C]; returns padded detections (boxes [B,K,4], scores [B,K], class ids [B,K] i64, count [B] i32)."""
+        res, raw, status = self.launch_with_support(image_sizes, out_sizes, features, proposals, counts, support_embedded,
+                                                    class_ids)
+        ops.check_status(status)
+        return res, raw
+
+    @torch.no_grad()
+    def launch_with_support(self, image_sizes, out_sizes, features, proposals: torch.Tensor, counts: torch.Tensor,
+                            support_embedded: List[Dict[str, torch.Tensor]], class_ids: Sequence[int]):
+        """eval_with_support without the host: everything is enqueued, the device status word comes back unread
+        (padded detections, per-problem (logits, deltas), status)."""
         C = len(class_ids)
         P, cap = proposals.shape[:2]
         box_features = self._shared_roi_transform(features, proposals, counts, C)                      # [P*cap, 2048, 7, 7]
@@ -144,12 +159,12 @@ class FsodRes5ROIHeads(nn.Module):
             raw.append((logits, deltas))
         bp = self.box_predictor
         if proposals.is_cuda:
-            status = ops.new_status(proposals.device)
-            hw = torch.tensor([list(s) for s in image_sizes], dtype=torch.int32, device=proposals.device)
-            ohw = torch.tensor([list(s) for s in out_sizes], dtype=torch.int32, device=proposals.device)
+            dev = proposals.device
+            status = ops.new_status(dev)
+            hw = upload([list(s) for s in image_sizes], torch.int32, dev)
+            ohw = upload([list(s) for s in out_sizes], torch.int32, dev)
             ob, os_, ocls, _, oc = ops.final_detect(det_boxes, det_scores, counts, C, bp.test_score_thresh, bp.test_nms_thresh,
                                                     bp.test_topk_per_image, hw, ohw, status)
-            ops.check_status(status)
-            ids = torch.tensor(list(class_ids), dtype=torch.int64, device=ocls.device)
-            return (ob, os_, ids[ocls], oc), raw
+            ids = upload(list(class_ids), torch.int64, dev)
+            return (ob, os_, ids[ocls], oc), raw, status
         raise NotImplementedError("FsodRes5ROIHeads: the final class-wise NMS exists only as a CUDA kernel")

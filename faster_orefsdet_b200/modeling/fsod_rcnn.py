@@ -16,6 +16,10 @@ What the reference computes per class c (fsod_rcnn.py:472-513), and where it run
   logits, deltas = FsodFastRCNNOutputLayers(box features, res5_avg_c)
   detections     = class-wise NMS over the union, top-k, rescale                               fod_final_detect
 
+Serving: ``submit(batch)`` enqueues the whole forward without a host synchronisation - the RPN proposals of each class
+are selected on the device (``FsodRPN.propose_device``, fod_rpn_proposals) - and ``model(pending)`` returns exactly what
+``model(batch)`` returns, as for CenterNet2Detector.
+
 Differences to the reference (as for CenterNet2Detector): B >= 1 query images per call, any number of proposals per
 class (the reference slices ``box_features[cnt*100:(cnt+1)*100]``, fsod_roi_heads.py:172), the pickle is read once per
 file version, ``MODEL.DEVICE=cpu`` is refused.
@@ -36,7 +40,8 @@ from .. import _lib, ops
 from ..compat import META_ARCH_REGISTRY, PROPOSAL_GENERATOR_REGISTRY, Boxes, ImageList, Instances, register, resolve
 from .backbone import build_backbone
 from .fsod_heads import positional_encoding
-from .roi_heads import build_roi_heads, pack_instances
+from .fsod_cen import PendingBatch
+from .roi_heads import build_roi_heads, instances_from_block, pack_block, pack_instances
 from . import fsod_heads, rpn  # noqa: F401  (register FsodRes5ROIHeads / FsodRPN)
 
 __all__ = ["FsodRCNN", "ParallelPolarizedSelfAttention"]
@@ -120,8 +125,11 @@ class FsodRCNN(nn.Module):
         return self.pixel_mean.device
 
     def forward(self, batched_inputs):
+        """``batched_inputs``: list[dict] like the reference, or a ``PendingBatch`` from ``submit``."""
         if self.training:
             raise NotImplementedError("FsodRCNN: training (fsod_rcnn.py:141-335) is outside the inference hot path")
+        if isinstance(batched_inputs, PendingBatch):
+            return self.collect(batched_inputs)
         with torch.cuda.device(self.device):
             self.init_model()
             return self.inference(batched_inputs)
@@ -217,8 +225,9 @@ class FsodRCNN(nn.Module):
             pickle.dump(self.build_support_dict(images, boxes), f)
 
     # ------------------------------------------------------------------ inference (query side)
-    def preprocess_image(self, batched_inputs) -> ImageList:
-        images = [(x["image"].to(self.device).float() - self.pixel_mean) / self.pixel_std for x in batched_inputs]
+    def preprocess_image(self, batched_inputs, non_blocking: bool = False) -> ImageList:
+        images = [(x["image"].to(self.device, non_blocking=non_blocking).float() - self.pixel_mean) / self.pixel_std
+                  for x in batched_inputs]
         return ImageList.from_tensors(images, self.backbone.size_divisibility)
 
     @torch.no_grad()
@@ -241,12 +250,8 @@ class FsodRCNN(nn.Module):
     def head(self, features: Dict[str, torch.Tensor], image_sizes, out_sizes):
         """res4 maps [B, 1024, H, W] -> padded detections + a trace of the per-class intermediates."""
         ep = self._episode
-        res4 = features["res4"]
-        if res4.is_cuda:
-            res4 = ops.nhwc(res4, "res4")
+        res4, gates, bounds = self._rpn_gates(features)
         B, C = res4.shape[0], len(ep["class_ids"])
-        gates = self.channel_attention.gates(self.agp(res4), ep["wq"], ep["k"])      # [C, B, 1024]: (:480-488)
-        amax = ops.absmax(res4, per_image=True)                                     # per image: no batch-mate coupling
         trace = {"gate": [], "proposals": []}
         cap = self.proposal_generator.post_nms_topk
         props = torch.zeros((B, C, cap, 4), dtype=torch.float32, device=res4.device)
@@ -254,9 +259,8 @@ class FsodRCNN(nn.Module):
         fake_images = type("Sizes", (), {"image_sizes": image_sizes})()
         for ci in range(C):
             gate = gates[ci]                                                        # channel_att + spatial_att = gate (.) res4
-            bound = (amax * gate.abs().amax(1)).reshape(1, B)
             plist, _ = self.proposal_generator(fake_images, {self.proposal_generator.in_features[0]: res4}, None,
-                                               gates=[gate], bounds=[bound])
+                                               gates=[gate], bounds=[bounds[ci]])
             trace["gate"].append(gate)
             trace["proposals"].append(plist)
             for b, p in enumerate(plist):
@@ -267,3 +271,83 @@ class FsodRCNN(nn.Module):
                                                     counts.reshape(-1), ep["emb"], ep["class_ids"])
         trace["raw"] = raw
         return res, trace
+
+    def _rpn_gates(self, features: Dict[str, torch.Tensor]):
+        """The preamble of ``head``: res4 (NHWC), the correlation gate of every class [C, B, 1024] and, per class, the
+        per-image bound [1, B] of the gated map that the RPN's 3x3 convolution reads."""
+        ep = self._episode
+        res4 = features["res4"]
+        if res4.is_cuda:
+            res4 = ops.nhwc(res4, "res4")
+        B = res4.shape[0]
+        gates = self.channel_attention.gates(self.agp(res4), ep["wq"], ep["k"])      # [C, B, 1024]: (:480-488)
+        amax = ops.absmax(res4, per_image=True)                                     # per image: no batch-mate coupling
+        return res4, gates, [(amax * gate.abs().amax(1)).reshape(1, B) for gate in gates]
+
+    # ------------------------------------------------------------------ serving (submit / collect)
+    def submit(self, batched_inputs: List[dict], do_postprocess: bool = True) -> PendingBatch:
+        """Asynchronous half of ``forward``, as CenterNet2Detector.submit: enqueue everything a batch needs - non-blocking
+        host-to-device copies of the images, the backbone, the RPN of every class with its proposals selected on the
+        device (``FsodRPN.propose_device``), the ROI head, one device-to-host copy of the padded detections and of the
+        status word - and return at once.  A serving loop submits batch k+1 before it collects batch k
+        (``model(pending_k)``), so the host work of one batch runs under the kernels of the other.  ``model(pending)``
+        returns what ``model(batched_inputs)`` returns.
+
+        Contract for the caller: pinned host images are read by the copy engine after this call returns - do not modify
+        or free them until the batch has been collected or abandoned (``abandon``)."""
+        if self.training:
+            raise NotImplementedError("FsodRCNN: training (fsod_rcnn.py:141-335) is outside the inference hot path")
+        with torch.cuda.device(self.device):
+            self.init_model()
+            return self._submit(batched_inputs, do_postprocess)
+
+    @torch.no_grad()
+    def _submit(self, batched_inputs, do_postprocess):
+        ep = self._episode
+        if ep is None:
+            raise _lib.FodError("no support features installed: call init_model() / set_prototypes() first")
+        images = self.preprocess_image(batched_inputs, non_blocking=True)
+        features = self.backbone(images.tensor)
+        sizes = [tuple(s) for s in images.image_sizes]
+        out_sizes = [(int(inp.get("height", s[0])), int(inp.get("width", s[1]))) if do_postprocess else s
+                     for inp, s in zip(batched_inputs, sizes)]
+        res4, gates, bounds = self._rpn_gates(features)
+        B, C = res4.shape[0], len(ep["class_ids"])
+        rpn = self.proposal_generator
+        cap, dev = rpn.post_nms_topk, res4.device
+        # class-major here, so that each class's outputs are contiguous; the ROI head takes them image-major like head's
+        props = torch.zeros((C, B, cap, 4), dtype=torch.float32, device=dev)
+        logits = torch.empty((C, B, cap), dtype=torch.float32, device=dev)
+        counts = torch.zeros((C, B), dtype=torch.int32, device=dev)
+        image_hw = fsod_heads.upload([list(s) for s in sizes], torch.int32, dev)
+        for ci in range(C):
+            rpn.propose_device([res4], image_hw, [gates[ci]], [bounds[ci]], props[ci], logits[ci], counts[ci])
+        (ob, os_, ocls, oc), _, status = self.roi_heads.launch_with_support(
+            sizes, out_sizes, {self.in_features[0]: res4}, props.transpose(0, 1).reshape(B * C, cap, 4),
+            counts.t().reshape(-1), ep["emb"], ep["class_ids"])
+        block = pack_block(ob, os_, ocls, oc)
+        host = torch.empty(block.shape, dtype=torch.float32, pin_memory=True)
+        status_host = torch.empty((1,), dtype=status.dtype, pin_memory=True)
+        host.copy_(block, non_blocking=True)
+        status_host.copy_(status.view(-1)[:1], non_blocking=True)
+        done = torch.cuda.Event()
+        done.record(torch.cuda.current_stream(dev))
+        return PendingBatch(batched_inputs, images.tensor, sizes, out_sizes, block, host, status_host, done)
+
+    def collect(self, pending: PendingBatch, do_postprocess: bool = True):
+        """Wait for a submitted batch and build its results (what ``forward`` returns)."""
+        if pending.done is None:
+            raise _lib.FodError("collect: this PendingBatch was already collected or abandoned")
+        pending.done.synchronize()
+        pending.done = None
+        ops.check_status(pending.status_host)
+        results = instances_from_block(pending.block, pending.host, pending.out_sizes)
+        for r in results:       # the reference emits the support class ids as int8 (fsod_roi_heads.py:176)
+            r.pred_classes = r.pred_classes.to(torch.int8)
+        return [{"instances": r} for r in results] if do_postprocess else results
+
+    def abandon(self, pending: PendingBatch) -> None:
+        """Give up a submitted batch without building its results (its kernels still run to completion)."""
+        if pending.done is not None:
+            pending.done.synchronize()
+            pending.done = None

@@ -4,7 +4,8 @@
 hidden layer, :75-147), ``DefaultAnchorGenerator`` (d2!/modeling/anchor_generator.py) and ``find_top_rpn_proposals``
 (d2!/modeling/proposal_generator/proposal_utils.py:19-119).  B200 path: the 3x3 hidden convolution runs on the
 tensor-core kernel with the support correlation of FsodRCNN fused into its A operand (``a_gate``), objectness and
-anchor deltas are one stacked 1x1 convolution, the NMS is ``fod_batched_nms``.
+anchor deltas are one stacked 1x1 convolution, the NMS is ``fod_batched_nms``.  ``propose_device`` (the serving path of
+FsodRCNN.submit) runs the whole selection of ``predict_proposals`` as one device op, ``fod_rpn_proposals``.
 """
 from __future__ import annotations
 
@@ -130,6 +131,27 @@ class FsodRPN(nn.Module):
         logits = [s.permute(0, 2, 3, 1).flatten(1) for s in logits]                     # (N, Hi*Wi*A)
         deltas = [x.reshape(x.shape[0], -1, 4, x.shape[-2], x.shape[-1]).permute(0, 3, 4, 1, 2).flatten(1, -2) for x in deltas]
         return self.predict_proposals(anchors, logits, deltas, images.image_sizes), {}
+
+    @torch.no_grad()
+    def propose_device(self, feats: List[torch.Tensor], image_hw: torch.Tensor, gates, bounds, out_boxes: torch.Tensor,
+                       out_logits: torch.Tensor, out_count: torch.Tensor) -> None:
+        """``forward`` for one class without the host: the same ``rpn_head`` call, then ``ops.rpn_proposals`` (the
+        selection of ``predict_proposals`` as one device op).  feats: the maps of ``in_features``; image_hw [N, 2] int32
+        on the device; writes the proposals of image n to out_boxes[n] [post_nms_topk, 4], out_logits[n] and
+        out_count[n] (rows at or beyond the count keep their contents)."""
+        logits, deltas = self.rpn_head(feats, gates, bounds)
+        ops.rpn_proposals(logits, deltas, self._anchors(feats), image_hw, self.pre_nms_topk, self.box_weights,
+                          self.min_box_size, self.nms_thresh, self.post_nms_topk, out=(out_boxes, out_logits, out_count))
+
+    def _anchors(self, feats: List[torch.Tensor]) -> List[torch.Tensor]:
+        """anchor_generator(feats), kept per map size and device: building them uploads the cell anchors, which would
+        synchronise with the stream."""
+        key = tuple((tuple(f.shape[-2:]), f.device) for f in feats)
+        hit = self.__dict__.get("_anchor_cache")
+        if hit is None or hit[0] != key:
+            hit = (key, self.anchor_generator(feats))
+            self.__dict__["_anchor_cache"] = hit
+        return hit[1]
 
     @torch.no_grad()
     def predict_proposals(self, anchors, logits, deltas, image_sizes) -> List[Instances]:

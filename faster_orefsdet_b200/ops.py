@@ -281,6 +281,66 @@ def nms_proposals(boxes: Tensor, scores: Tensor, count: Optional[Tensor], iou_th
     return keep, ob, os_, oc
 
 
+# --------------------------------------------------------------------------- N2
+def rpn_proposals(logits: Sequence[Tensor], deltas: Sequence[Tensor], anchors: Sequence[Tensor], image_hw: Tensor,
+                  pre_topk: int, box_weights: Sequence[float], min_size: float, iou_thresh: float, post_topk: int,
+                  out: Optional[Tuple[Tensor, Tensor, Tensor]] = None):
+    """find_top_rpn_proposals (proposal_utils.py:19-119) of P problems, problem p = image p of every level ->
+    (boxes [P,post_topk,4], objectness logits [P,post_topk], count [P] i32), proposals in NMS visit order.  Rows at or
+    beyond count are not written: zeros in fresh outputs, untouched in ``out`` (preallocated, written in place).
+    logits[l] [P,A,H,W] / deltas[l] [P,4A,H,W]: the channels of the stacked StandardRPNHead output; read in place when
+    deltas[l] directly follows logits[l] in one NHWC buffer (StandardRPNHead.forward's views), stacked into one first
+    otherwise.  anchors[l] [H*W*A,4] (DefaultAnchorGenerator); image_hw [P,2] int32 (height, width) on the device."""
+    L = len(logits)
+    if L < 1 or L > 3 or len(deltas) != L or len(anchors) != L:
+        raise _lib.FodError("rpn_proposals: 1..3 levels with logits, deltas and anchors each")
+    P, A = logits[0].shape[0], logits[0].shape[1]
+    dev = logits[0].device
+    maps, ps, ancs, slots = [], [], [], 0
+    for lg, dl, an in zip(logits, deltas, anchors):
+        _chk(lg, torch.float32, "logits"), _chk(dl, torch.float32, "deltas"), _chk(an, torch.float32, "anchors")
+        n, a, h, w = lg.shape
+        if (n, a) != (P, A) or tuple(dl.shape) != (P, 4 * A, h, w) or tuple(an.shape) != (h * w * A, 4):
+            raise _lib.FodError("rpn_proposals: logits [P,A,H,W], deltas [P,4A,H,W] and anchors [H*W*A,4] per level")
+        try:
+            s = _pixel_stride(lg, "logits")
+            in_place = dl.data_ptr() == lg.data_ptr() + 4 * A and _pixel_stride(dl, "deltas") == s
+        except _lib.FodError:
+            in_place = False
+        if not in_place:
+            lg = nhwc(torch.cat((lg, dl), 1))
+            s = 5 * A
+        if not an.is_contiguous() or an.data_ptr() % 16:
+            an = an.clone()
+        maps.append(lg)
+        ps.append(int(s))
+        ancs.append(an)
+        slots += min(h * w * A, int(pre_topk))
+    if slots > _lib.FOD_NMS_MAX_BOXES:
+        raise _lib.FodError(f"rpn_proposals: {slots} candidates per problem > FOD_NMS_MAX_BOXES ({_lib.FOD_NMS_MAX_BOXES})")
+    image_hw = _chk(image_hw, torch.int32, "image_hw")
+    if tuple(image_hw.shape) != (P, 2) or not image_hw.is_contiguous():
+        raise _lib.FodError("rpn_proposals: image_hw must be a contiguous [P, 2] int32 tensor")
+    if out is None:
+        out = (torch.zeros((P, post_topk, 4), dtype=torch.float32, device=dev),
+               torch.zeros((P, post_topk), dtype=torch.float32, device=dev),
+               torch.zeros((P,), dtype=torch.int32, device=dev))
+    ob, ol, oc = out
+    for t_, dt, shape, name in ((ob, torch.float32, (P, post_topk, 4), "boxes"), (ol, torch.float32, (P, post_topk), "logits"),
+                                (oc, torch.int32, (P,), "count")):
+        if tuple(_chk(t_, dt, name).shape) != shape or not t_.is_contiguous():
+            raise _lib.FodError(f"rpn_proposals: out {name} must be a contiguous {shape} tensor")
+    lv = _levels(maps, [0] * L)
+    L_ = _lib.lib()
+    ws = torch.empty((max(int(L_.fod_rpn_proposals_workspace_bytes(lv, L, P, A, int(pre_topk))), 16),), dtype=torch.uint8,
+                     device=dev)
+    bw = (ctypes.c_float * 4)(*[float(v) for v in box_weights])
+    _lib.check(L_.fod_rpn_proposals(_ptr_array(maps), (ctypes.c_int * L)(*ps), _ptr_array(ancs), lv, L, P, A, _ptr(image_hw),
+                                    int(pre_topk), bw, float(min_size), float(iou_thresh), int(post_topk), _ptr(ob), _ptr(ol),
+                                    _ptr(oc), _ptr(ws), _stream()), "fod_rpn_proposals")
+    return ob, ol, oc
+
+
 # --------------------------------------------------------------------------- R1 / P1
 def tile_pooled(x: Tensor) -> Tensor:
     """[P,cap,64,128] ROI rows -> the tiled operand layout [P,U,256,128,32] of relation_head (U = ceil(cap/128);

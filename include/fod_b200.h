@@ -157,6 +157,38 @@ int fod_nms_proposals(const float* boxes, const float* scores, const int32_t* co
                       float* out_scores, int32_t* out_count, uint32_t* status, fod_stream_t stream);
 
 /* ---------------------------------------------------------------------------
+ * N2  RPN proposal selection of the Attention-RPN (FsodRPN.predict_proposals).  Replaces find_top_rpn_proposals,
+ * d2!/modeling/proposal_generator/proposal_utils.py:19-119, with the decode of Box2BoxTransform.apply_deltas,
+ * d2!/modeling/box_regression.py:77-115.  A problem is one image of one class's RPN output: problem p reads image p of
+ * every level's map.  Per problem and level:
+ *   1. select the top k = min(H*W*A, pre_topk) objectness logits: score descending, ties by ascending anchor index,
+ *      NaN above +inf (torch.sort(descending=True) made stable);
+ *   2. decode them against their anchors with the separate fp32 roundings of ATen (deltas / weights as a product with
+ *      the fp32 reciprocal, dw / dh clamped at log(1000/16) before the exp);
+ *   3. drop rows with a non-finite box or logit, clip to the problem's image (x to [0, w], y to [0, h]), keep width and
+ *      height > min_size;
+ * then over the levels: the NMS of fod_batched_nms (stable score-descending visit order, torchvision's IoU arithmetic,
+ * boxes offset by level * (max coordinate + 1) when num_levels > 1), and the first post_topk survivors in visit order
+ * (a strict cut: no tie extension, no status bit).
+ *   maps[l]    : [P][H_l][W_l][pixel_stride[l] >= 5 * num_anchors] fp32, the stacked 1x1 output of StandardRPNHead read in
+ *                place: logit of anchor a in channel a, delta j (dx, dy, dw, dh) in channel num_anchors + 4a + j
+ *   anchors[l] : [H_l * W_l * num_anchors][4] xyxy fp32, 16-byte aligned (DefaultAnchorGenerator, (y, x, anchor) order)
+ *   levels     : only height / width are read
+ *   image_hw   : [P][2] int32 (height, width) DEVICE
+ *   box_weights: HOST, 4 floats (RPN.BBOX_REG_WEIGHTS)
+ *   out_boxes  : [P][post_topk][4] (16-byte aligned), out_logits [P][post_topk], out_count [P] int32; rows at or beyond
+ *                out_count[p] are not written
+ *   workspace  : fod_rpn_proposals_workspace_bytes(...) bytes of device memory, 16-byte aligned
+ * The selected candidates of a problem, sum over l of min(H_l * W_l * num_anchors, pre_topk), must not exceed
+ * FOD_NMS_MAX_BOXES (FOD_ERR_CAPACITY otherwise; the caller can check it from the shapes). */
+size_t fod_rpn_proposals_workspace_bytes(const fod_level_t* levels, int num_levels, int num_problems, int num_anchors,
+                                         int pre_topk);
+int fod_rpn_proposals(const float* const* maps, const int* pixel_stride, const float* const* anchors,
+                      const fod_level_t* levels, int num_levels, int num_problems, int num_anchors, const int32_t* image_hw,
+                      int pre_topk, const float* box_weights, float min_size, double iou_thresh, int post_topk,
+                      float* out_boxes, float* out_logits, int32_t* out_count, void* workspace, fod_stream_t stream);
+
+/* ---------------------------------------------------------------------------
  * R1 / P1  multi-level ROIAlign (aligned=True, sampling_ratio=0) with FPN level
  * assignment.  Replaces ROIPooler.forward + assign_boxes_to_levels +
  * torchvision.ops.roi_align, d2!/modeling/poolers.py:22-58,190-250,
